@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - fake-quant fwd+bwd throughput on the ResNet-50 W4A4 QAT quantizer set.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one synthetic ImageNet-shaped batch: for each of the 54
 quantised layers of torchvision ResNet-50 the activation fake-quant forward (A4 unsigned, per-tensor,
@@ -247,6 +247,8 @@ def run_ours(args, rank, world, device):
     t1.record()
     fence()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl, args.dump_outputs)
     if os.environ.get("DLMCQ_BENCH_PER_RANK"):
         print(f"rank {rank}: {t0.elapsed_time(t1) / args.steps:.4f} ms/step", file=sys.stderr, flush=True)
     ms = torch.tensor([t0.elapsed_time(t1)], device=device)
@@ -305,6 +307,36 @@ def run_ours(args, rank, world, device):
     if rank == 0:
         out["cpu_baseline"] = cpu_reference(sample_batch=1, passes=3) if world == 1 else None
         print(json.dumps(out), flush=True)
+
+
+DUMP_SAMPLE = 1 << 16       # elements kept per array: 4 arrays x 54 layers x 64 Ki float32 stays under 64 MB
+
+
+def dump_outputs(wl, out_dir):
+    """What the timed path handed back in its last step, as float32 .npy files under out_dir: per layer the
+    activation's and the weight's fake-quant forward (`<layer>.act_y`, `<layer>.wt_y`) and input gradient
+    (`<layer>.act_dx`, `<layer>.wt_dx`), and `dscale`, the flat scale-gradient buffer (one entry per layer's
+    activation, then the weights' per-channel entries in layer order).  An array longer than DUMP_SAMPLE is stored
+    as DUMP_SAMPLE elements at sorted indices drawn from one fixed-seed generator in this fixed order, so two builds
+    run with the same arguments are compared element for element.  Called on rank 0 only: with N > 1 ranks the y / dx
+    arrays are rank 0's (inputs seeded 2333 + 0) and `dscale` holds the SUM over the N ranks, so a dump depends on N."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    gen = torch.Generator().manual_seed(2333)
+
+    def save(name, t):
+        flat = t.reshape(-1)
+        if flat.numel() > DUMP_SAMPLE:
+            idx = torch.randint(flat.numel(), (DUMP_SAMPLE,), generator=gen).sort().values
+            flat = flat[idx.to(flat.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), flat.float().cpu().numpy())
+
+    for (name, _, _), a, w in zip(wl.layers, wl.acts, wl.wts):
+        save(name + ".act_y", a["y"])
+        save(name + ".act_dx", a["dx"])
+        save(name + ".wt_y", w["y"])
+        save(name + ".wt_dx", w["dx"])
+    np.save(os.path.join(out_dir, "dscale.npy"), wl.dscale.cpu().numpy())
 
 
 def run_e2e(args, wl, rank, world, device):
@@ -853,7 +885,16 @@ def main():
     ap.add_argument("--qat-only", action="store_true", help="skip the kernel metric; print only the QAT arms (diagnostic)")
     ap.add_argument("--qat-batch", type=int, default=128, help="per-GPU batch of the QAT arms")
     ap.add_argument("--qat-small-batch", type=int, default=32, help="per-GPU batch of the host-bound / CUDA-graph arms")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's outputs to DIR/<name>.npy (float32, sampled "
+                         "to at most 64 MB in all) for comparing two builds on identical seeded inputs; under torchrun "
+                         "only rank 0 writes (its own y/dx, and the scale gradients summed over ranks), so compare "
+                         "dumps taken with the same number of GPUs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.qat_only):
+        ap.error("--dump-outputs writes the outputs of the timed kernel path: it needs --impl ours without --qat-only")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,12 +1,16 @@
 """The reference's OWN trainers, unmodified, driving this package's modules (north star: "drop-in").
 
-Runs wherever /root/reference exists (the authoring container; the GPU box has no reference checkout - there
-tests/test_gpu_trainer_sequence.py replays the same call sequences).  No compute happens here (no GPU): what is checked
-is the wiring the trainers rely on - class identity through `compat.install()`, `reset_qparams` discovery and period,
-fnmatch name filters, `change_quant_state`, `generate_optimizer`'s parameter groups, target selection of the block
-reconstruction."""
+What the trainers contribute - the QAT trainer's reset period and epoch length, the FSPTQ trainer's target selection,
+model-state switch and per-name learning rates - is stored in tests/golden/reference_trainers.json, so both tests run
+without an upstream checkout and check this package against those values.  When DLMCQ_REFERENCE_ROOT names an upstream
+checkout, the fixture imports the real trainer classes, every stored value is re-derived from them and must match,
+and the FSPTQ trainer's change_model_state is run on this package's modules (that one check needs the upstream code).
+No compute happens here (no GPU): what is checked is the wiring the trainers rely on - class identity through
+`compat.install()`, `reset_qparams` discovery and period, fnmatch name filters, `change_quant_state`,
+`generate_optimizer`'s parameter groups, target selection of the block reconstruction."""
 import copy
 import importlib
+import json
 import logging
 import os
 import sys
@@ -17,8 +21,10 @@ import pytest
 import torch
 from torch import nn
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
+REF = os.environ.get("DLMCQ_REFERENCE_ROOT", "")
+HAVE_REF = bool(REF) and os.path.isdir(os.path.join(REF, "trainer"))
+with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_trainers.json")) as _f:
+    GOLDEN = json.load(_f)
 
 CFG = {"weight": {"enable": True, "type": "minmax_channel", "args": {"n_bits": 8, "signed": True, "ch_axis": 0}},
        "input": {"enable": True, "type": "minmax_tensor", "args": {"n_bits": 8, "signed": False}},
@@ -28,16 +34,36 @@ CFG = {"weight": {"enable": True, "type": "minmax_channel", "args": {"n_bits": 8
 @pytest.fixture()
 def reference_trainers():
     """Import trainer/{quantization_aware_training,fsptq}_trainer.py from the reference tree with `dlmc.*` resolved
-    to this package and the reference's heavyweight side modules (tensorboard writer, yaml utils) stubbed."""
+    to this package and the reference's heavyweight side modules (tensorboard writer, yaml utils) stubbed.
+    (None, None) without an upstream checkout: the tests then use the stored values."""
     import dlmc_quant_b200.compat as compat
     saved_modules = dict(sys.modules)
     saved_path = list(sys.path)
     compat.install(force=True)
+    try:
+        yield _import_reference_trainers() if HAVE_REF else (None, None)
+    finally:
+        sys.path[:] = saved_path
+        mine = ("dlmc.", "trainer", "utils", "logger", "base", "matplotlib", "ruamel")
+        for k in list(sys.modules):
+            if k not in saved_modules and (k == "dlmc" or k.startswith(mine)):
+                del sys.modules[k]
+        for k in ("utils", "logger", "base"):
+            if k in saved_modules:
+                sys.modules[k] = saved_modules[k]
+            else:
+                sys.modules.pop(k, None)
+        for k, v in saved_modules.items():
+            if k == "trainer" or k.startswith("trainer."):
+                sys.modules[k] = v
+
+
+def _import_reference_trainers():
     sys.path.insert(0, REF)
     for name in ("matplotlib", "matplotlib.pyplot"):
         sys.modules.setdefault(name, types.ModuleType(name))
     # utils.MetricTracker / logger.TensorboardWriter: stand-ins with the surface the trainers use (the reference's own
-    # MetricTracker writes into read-only pandas views and fails on the pandas in this image)
+    # MetricTracker writes into read-only pandas views and fails on current pandas)
     util = types.ModuleType("utils")
 
     class MetricTracker:
@@ -64,24 +90,9 @@ def reference_trainers():
     tr = types.ModuleType("trainer")
     tr.__path__ = [os.path.join(REF, "trainer")]          # bypass trainer/__init__.py (imports a missing file)
     sys.modules["trainer"] = tr
-    try:
-        qat = importlib.import_module("trainer.quantization_aware_training_trainer")
-        fsp = importlib.import_module("trainer.fsptq_trainer")
-        yield qat, fsp
-    finally:
-        sys.path[:] = saved_path
-        mine = ("dlmc.", "trainer", "utils", "logger", "base", "matplotlib", "ruamel")
-        for k in list(sys.modules):
-            if k not in saved_modules and (k == "dlmc" or k.startswith(mine)):
-                del sys.modules[k]
-        for k in ("utils", "logger", "base"):
-            if k in saved_modules:
-                sys.modules[k] = saved_modules[k]
-            else:
-                sys.modules.pop(k, None)
-        for k, v in saved_modules.items():
-            if k == "trainer" or k.startswith("trainer."):
-                sys.modules[k] = v
+    qat = importlib.import_module("trainer.quantization_aware_training_trainer")
+    fsp = importlib.import_module("trainer.fsptq_trainer")
+    return qat, fsp
 
 
 class _Config(dict):
@@ -114,16 +125,22 @@ def _loader():
 
 def test_qat_trainer_finds_and_drives_our_modules(reference_trainers, tmp_path, monkeypatch):
     qat, _ = reference_trainers
+    gold = GOLDEN["qat"]
     from dlmc.utils.quantize import quantize_model           # resolves to dlmc_quant_b200.quantize
     from dlmc_quant_b200.scalar.modules.base import QBase
     net = Net()
     quantize_model(net, copy.deepcopy(CFG), None)
     assert all(isinstance(m, QBase) for m in (net.conv1, net.block[0], net.linear))
-    monkeypatch.setattr(qat.QATTrainer, "_save_checkpoint", lambda self, epoch: None, raising=False)
     opt = torch.optim.SGD(net.parameters(), lr=0.1)
-    t = qat.QATTrainer(net, nn.CrossEntropyLoss(), [], opt, _Config(str(tmp_path), update_qparams_period=2), _loader(),
-                       train_log_density=1, valid_log_density=1, rank=-1, world_size=-1)
-    assert t.update_qparams_period == 2 and t.len_epoch == 4
+    loader = _loader()
+    assert len(loader) == gold["loader_batches"]
+    period, len_epoch, model = gold["update_qparams_period"], gold["len_epoch"], net
+    if qat is not None:
+        monkeypatch.setattr(qat.QATTrainer, "_save_checkpoint", lambda self, epoch: None, raising=False)
+        t = qat.QATTrainer(net, nn.CrossEntropyLoss(), [], opt, _Config(str(tmp_path), **gold["trainer_config"]),
+                           loader, train_log_density=1, valid_log_density=1, rank=-1, world_size=-1)
+        assert (t.update_qparams_period, t.len_epoch) == (period, len_epoch)
+        model = t.model
     # the trainer's reset hook: `if hasattr(m, 'reset_qparams'): m.reset_qparams()` (qat_trainer.py:44-48)
     for m in net.modules():
         if isinstance(m, QBase):
@@ -133,11 +150,11 @@ def test_qat_trainer_finds_and_drives_our_modules(reference_trainers, tmp_path, 
     def _reset(m):
         if hasattr(m, "reset_qparams"):
             m.reset_qparams()
-    t.model.apply(_reset)
+    model.apply(_reset)
     assert all(m._host_init == {"in": False, "wt": False} and float(m.in_init_state) == 0
                for m in net.modules() if isinstance(m, QBase))
     # steps at which the trainer resets: (epoch*len + batch) % period == 1
-    assert [b for b in range(4) if (1 * t.len_epoch + b) % t.update_qparams_period == 1] == [1, 3]
+    assert [b for b in range(4) if (1 * len_epoch + b) % period == 1] == [1, 3]
     # the parameter-name filters it logs by (qat_trainer.py:92,139) find our parameters
     names = [n for n, _ in net.named_parameters()]
     assert sum(fnmatch(n, "*in_scale*") for n in names) == 4 and all(p.requires_grad for p in net.parameters())
@@ -149,31 +166,41 @@ def test_qat_trainer_finds_and_drives_our_modules(reference_trainers, tmp_path, 
 
 def test_fsptq_trainer_sees_our_blocks_and_param_groups(reference_trainers, tmp_path, monkeypatch):
     _, fsp = reference_trainers
+    gold = GOLDEN["fsptq"]
     from dlmc.utils.quantize import quantize_model
+    from dlmc_quant_b200.recon import FSPTQReconstructor
     from dlmc_quant_b200.scalar.FSPTQuant.base import FSPTQBase
-    assert fsp.FSPTQBase is FSPTQBase                         # one class object on both sides of the import alias
+    # the class fsptq_trainer.py:9 imports by its full upstream path: one class object on both sides of the alias
+    assert importlib.import_module("dlmc.quantization.scalar.FSPTQuant.base").FSPTQBase is FSPTQBase
     net, fp = Net(), Net()
     quantize_model(net, copy.deepcopy(CFG), None, quantization_type="FSPTQ")
-    monkeypatch.setattr(fsp.FSPTQTrainer, "_save_checkpoint", lambda self, epoch: None, raising=False)
-    t = fsp.FSPTQTrainer(net, fp, None, [], None, _Config(str(tmp_path), epochs=10), _loader(),
-                         block_dict={nn.Sequential: True}, train_log_density=1, valid_log_density=1, rank=-1, world_size=-1)
-    # target selection of train() (fsptq_trainer.py:44-59): FSPTQ layers named conv1 / linear, and block types
-    picked = [n for (n, m), _ in zip(net.named_modules(), fp.modules())
-              if (isinstance(m, fsp.FSPTQBase) and n in ["conv1", "linear"]) or type(m) in t.block_dict]
-    assert picked == ["conv1", "block", "linear"]
-    from dlmc_quant_b200.recon import FSPTQReconstructor
-    assert [n for n, _, _ in FSPTQReconstructor(net, fp, block_types=(nn.Sequential,)).targets()] == picked
-    # change_model_state (fsptq_trainer.py:155-161): conv1 keeps its input un-quantised
-    t.change_model_state(net, True, True)
-    assert net.conv1.wt_quant and not net.conv1.act_quant and net.block[0].act_quant and net.linear.wt_quant
+    block_types = tuple(getattr(nn, n) for n in gold["block_dict"])
+    assert [n for n, _, _ in FSPTQReconstructor(net, fp, block_types=block_types).targets()] == gold["targets"]
     # generate_optimizer (fsptq_trainer.py:136-152): our parameter names fall into the groups the reference's own
     # modules fall into - `.endswith("scales")` matches neither `in_scale` nor `wt_scale` there either, so scales train
     # at 1e-5 like weights; recon.py reproduces exactly that by default (scale_lr=None)
-    opt, sched = t.generate_optimizer(net.block)
-    lrs = {n: g["lr"] for (n, _), g in zip(net.block.named_parameters(), opt.param_groups)}
-    assert lrs["0.weight"] == 1e-5 and lrs["0.in_scale"] == 1e-5 and lrs["0.wt_scale"] == 1e-5 and lrs["0.bias"] == 1e-5
     ours, _ = FSPTQReconstructor(net, fp, epochs=10).generate_optimizer(net.block)
-    assert [g["lr"] for g in ours.param_groups] == [g["lr"] for g in opt.param_groups]
+    ours_lrs = [[n, g["lr"]] for (n, _), g in zip(net.block.named_parameters(), ours.param_groups)]
+    assert len(ours.param_groups) == len(gold["block_optimizer_lrs"]) and ours_lrs == gold["block_optimizer_lrs"]
     tuned, _ = FSPTQReconstructor(net, fp, epochs=10, scale_lr=1e-3).generate_optimizer(net.block)
     got = {n: g["lr"] for (n, _), g in zip(net.block.named_parameters(), tuned.param_groups)}
     assert got["0.in_scale"] == 1e-3 and got["0.wt_scale"] == 1e-3 and got["0.weight"] == 1e-5
+    if fsp is None:
+        return
+    # the live upstream trainer: every stored value above is re-derived from it
+    assert fsp.FSPTQBase is FSPTQBase
+    monkeypatch.setattr(fsp.FSPTQTrainer, "_save_checkpoint", lambda self, epoch: None, raising=False)
+    t = fsp.FSPTQTrainer(net, fp, None, [], None, _Config(str(tmp_path), epochs=10), _loader(),
+                         block_dict={b: True for b in block_types}, train_log_density=1, valid_log_density=1, rank=-1,
+                         world_size=-1)
+    # target selection of train() (fsptq_trainer.py:44-59): FSPTQ layers named conv1 / linear, and block types
+    picked = [n for (n, m), _ in zip(net.named_modules(), fp.modules())
+              if (isinstance(m, fsp.FSPTQBase) and n in ["conv1", "linear"]) or type(m) in t.block_dict]
+    assert picked == gold["targets"]
+    # change_model_state (fsptq_trainer.py:155-161): conv1 keeps its input un-quantised
+    t.change_model_state(net, True, True)
+    for name, state in gold["change_model_state_wt_act_true"].items():
+        assert {k: bool(getattr(net.get_submodule(name), k)) for k in state} == state, name
+    opt, _ = t.generate_optimizer(net.block)
+    ref_lrs = [[n, g["lr"]] for (n, _), g in zip(net.block.named_parameters(), opt.param_groups)]
+    assert len(opt.param_groups) == len(gold["block_optimizer_lrs"]) and ref_lrs == gold["block_optimizer_lrs"]
