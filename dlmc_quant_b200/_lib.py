@@ -97,6 +97,7 @@ SIGNATURES = {
     "dlmcq_fq_partials_floats": (_Z, []),
     "dlmcq_fq_backward_partials": (_I, [_P, _P, _P, _LP, _QP, _P, _P]),
     "dlmcq_fq_finalize_many": (_I, [_P, _I, _P]),
+    "dlmcq_capture_overlap_count": (_I, []),
     "dlmcq_dequantize": (_I, [_P, _P, _LP, _P, _P, _P]),
     "dlmcq_ste_value": (_I, [_P, _P, _L, _I, _I, _P]),
     "dlmcq_grad_scale_value": (_I, [_P, _P, _L, _F, _P]),

@@ -299,7 +299,13 @@ inline SlabGeom make_slab(int64_t outer, int64_t channels, int64_t inner) {
 // Programmatic dependent launch: consecutive kernels of one stream (the per-layer quantizer launches of a
 // training step) hide their launch latency behind the predecessor's tail.  Every kernel launched this way
 // executes pdl_wait() before its first global-memory access - it then sees all of the predecessor's
-// writes - and pdl_trigger() right away so that its own successor can be staged early.
+// writes - and pdl_trigger() right away so that its own successor can be staged early.  The exceptions load
+// data that the host or the call sequence proves the predecessor does not write (bnq_apply_kernel, and the flat
+// fake-quant kernels when capture_check reports an independent launch) before pdl_wait().
+// Invariant: every CTA of every kernel launched through launch_pdl executes pdl_wait() before it triggers, stores
+// or exits.  So launch N+2 cannot start before every CTA of launch N+1 has passed its wait, i.e. before launch N
+// has completed and flushed: loads hoisted above the wait of N+2 can only race with N+1, and checking N+2's reads
+// against N+1's writes alone is enough.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;"); }
 bool pdl_enabled();

@@ -10,6 +10,8 @@
 //            owns one row segment (<= kRowSeg elements), so the channel's qparams are loaded
 //            once per warp and the per-channel scale gradient is a warp-shuffle reduction.
 // Roofline: HBM.  Algorithmic bytes: forward 2*sizeof(T), backward 3*sizeof(T) per element.
+#include <mutex>
+
 #include "fq_rows.cuh"
 
 namespace dlmcq {
@@ -19,19 +21,35 @@ constexpr int kUnroll = 4;
 // ---------------------------------------------------------------------------------------
 // flat forward
 // ---------------------------------------------------------------------------------------
+// independent (TILED only): the host proved that the preceding launch writes nothing this one reads
+// (capture_check), so the qparams and the first tile are loaded before pdl_wait() and overlap its tail.
 template <int FORM, typename T, int U = kUnroll, int MINB = 4, bool TILED = false>
 __global__ void __launch_bounds__(kThreads, MINB)
 fq_fwd_flat(const T* __restrict__ x, T* __restrict__ y, T* __restrict__ codes, int64_t n,
-            const float* __restrict__ scale, const float* __restrict__ offset, float g, float lo, float hi) {
+            const float* __restrict__ scale, const float* __restrict__ offset, float g, float lo, float hi,
+            int independent) {
   using V = Vec<T>;
   using raw = typename V::raw;
+  const int64_t nvec = n / V::N;
+  const raw* xv = reinterpret_cast<const raw*>(x);
+  const int64_t tile_vecs = static_cast<int64_t>(U) * blockDim.x;
+  const int64_t ntiles = nvec / tile_vecs;
+  ChanParams p;
+  raw r0[U];
+  const bool hoist = TILED && independent && blockIdx.x < ntiles;
+  if (TILED && independent) {
+    p = make_params<FORM>(scale, offset, 0, g, lo, hi);
+    if (hoist) {
+      const int64_t b = static_cast<int64_t>(blockIdx.x) * tile_vecs + threadIdx.x;
+#pragma unroll
+      for (int k = 0; k < U; ++k) r0[k] = ld_stream(xv + b + k * blockDim.x);
+    }
+  }
   pdl_wait();
   pdl_trigger();
-  const ChanParams p = make_params<FORM>(scale, offset, 0, g, lo, hi);
-  const int64_t nvec = n / V::N;
+  if (!(TILED && independent)) p = make_params<FORM>(scale, offset, 0, g, lo, hi);
   const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
   int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-  const raw* xv = reinterpret_cast<const raw*>(x);
   raw* yv = reinterpret_cast<raw*>(y);
   raw* cv = reinterpret_cast<raw*>(codes);
 
@@ -44,9 +62,14 @@ fq_fwd_flat(const T* __restrict__ x, T* __restrict__ y, T* __restrict__ codes, i
   };
   if (TILED) {
     // each CTA iteration covers one contiguous tile of U*256 vectors (16 KB for fp32, U=4)
-    const int64_t tile_vecs = static_cast<int64_t>(U) * blockDim.x;
-    const int64_t ntiles = nvec / tile_vecs;
-    for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+    int64_t t = blockIdx.x;
+    if (hoist) {
+      const int64_t b = t * tile_vecs + threadIdx.x;
+#pragma unroll
+      for (int k = 0; k < U; ++k) body(r0[k], b + k * blockDim.x);
+      t += gridDim.x;
+    }
+    for (; t < ntiles; t += gridDim.x) {
       const int64_t b = t * tile_vecs + threadIdx.x;
       raw r[U];
 #pragma unroll
@@ -125,24 +148,42 @@ __device__ __forceinline__ void finalize_flat(float* partials, int nblocks, floa
 // DEFER: leave the per-CTA partials in `ws` ([0]=#CTAs, [1]=chain factor, then (ds, doff) pairs) for
 // dlmcq_fq_finalize_many instead of finalising in the last CTA - the ticket + serial finalisation costs
 // ~3.4 us per launch (measured, profiles/README.md), a once-per-step batched finalisation ~4 us in total.
+// independent (VECTOR only): as for fq_fwd_flat, the qparams and the first tile of x and dy are loaded before
+// pdl_wait(); the partials, the ticket and every store stay behind it.
 template <int FORM, typename T, bool VECTOR, bool WANT_OFF, bool DEFER>
 __global__ void __launch_bounds__(kThreads, 4)
 fq_bwd_flat(const T* __restrict__ x, const T* __restrict__ dy, T* __restrict__ dx, int64_t n,
             const float* __restrict__ scale, const float* __restrict__ offset, float g, float lo, float hi,
-            float* __restrict__ dscale, float* __restrict__ doffset, void* ws) {
+            float* __restrict__ dscale, float* __restrict__ doffset, void* ws, int independent) {
   using V = Vec<T>;
   using raw = typename V::raw;
   __shared__ __align__(16) float smem[128];
+  const int64_t nvec = n / V::N;
+  const raw* xv = reinterpret_cast<const raw*>(x);
+  const raw* gv = reinterpret_cast<const raw*>(dy);
+  const int64_t tile_vecs = static_cast<int64_t>(kUnroll) * blockDim.x;
+  const int64_t ntiles = nvec / tile_vecs;
+  ChanParams p;
+  raw rx0[kUnroll], rg0[kUnroll];
+  const bool hoist = VECTOR && independent && blockIdx.x < ntiles;
+  if (VECTOR && independent) {
+    p = make_params<FORM>(scale, offset, 0, g, lo, hi);
+    if (hoist) {
+      const int64_t b = static_cast<int64_t>(blockIdx.x) * tile_vecs + threadIdx.x;
+#pragma unroll
+      for (int k = 0; k < kUnroll; ++k) {
+        rx0[k] = ld_stream(xv + b + k * blockDim.x);
+        rg0[k] = ld_stream(gv + b + k * blockDim.x);
+      }
+    }
+  }
   pdl_wait();
   pdl_trigger();
-  const ChanParams p = make_params<FORM>(scale, offset, 0, g, lo, hi);
+  if (!(VECTOR && independent)) p = make_params<FORM>(scale, offset, 0, g, lo, hi);
   float acc[2] = {0.f, 0.f};
   const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
   int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (VECTOR) {
-    const int64_t nvec = n / V::N;
-    const raw* xv = reinterpret_cast<const raw*>(x);
-    const raw* gv = reinterpret_cast<const raw*>(dy);
     raw* ov = reinterpret_cast<raw*>(dx);
     auto body = [&](const raw& rx, const raw& rg, int64_t idx) {
       float fx[V::N], fg[V::N], fo[V::N];
@@ -152,9 +193,14 @@ fq_bwd_flat(const T* __restrict__ x, const T* __restrict__ dy, T* __restrict__ d
       st_stream(ov + idx, V::pack(fo));
     };
     // each CTA iteration covers one contiguous tile of kUnroll*256 vectors of x and of dy
-    const int64_t tile_vecs = static_cast<int64_t>(kUnroll) * blockDim.x;
-    const int64_t ntiles = nvec / tile_vecs;
-    for (int64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+    int64_t t = blockIdx.x;
+    if (hoist) {
+      const int64_t b = t * tile_vecs + threadIdx.x;
+#pragma unroll
+      for (int k = 0; k < kUnroll; ++k) body(rx0[k], rg0[k], b + k * blockDim.x);
+      t += gridDim.x;
+    }
+    for (; t < ntiles; t += gridDim.x) {
       const int64_t b = t * tile_vecs + threadIdx.x;
       raw rx[kUnroll], rg[kUnroll];
 #pragma unroll
@@ -601,6 +647,84 @@ static inline bool elem_aligned(const void* p, int dtype) {
 }
 static inline RowGeom make_geom(const dlmcq_layout* l) { return make_geom(l->outer, l->channels, l->inner); }
 
+// ---------------------------------------------------------------------------------------
+// capture-time independence of consecutive flat launches.  Eagerly the host cannot know what the kernel
+// before a launch writes, so every kernel waits before its first load.  During a stream capture it can: the
+// capture reports the node(s) the next launch will depend on.  When that is exactly one node and it is this
+// library's previous flat launch in the same capture sequence, both launches' pointers and lengths are known
+// here, and if the new launch reads nothing the previous one writes, its CTAs load their qparams and first tile
+// before pdl_wait() (the invariant next to pdl_wait in common.cuh makes the pairwise check sufficient).
+// ---------------------------------------------------------------------------------------
+struct ByteRange {
+  uintptr_t beg, end;   // [beg, end)
+};
+struct FlatAccess {
+  ByteRange rd[5], wr[6];
+  int nrd = 0, nwr = 0;
+  void read(const void* p, size_t bytes) {
+    if (p && bytes) rd[nrd++] = {reinterpret_cast<uintptr_t>(p), reinterpret_cast<uintptr_t>(p) + bytes};
+  }
+  void write(const void* p, size_t bytes) {
+    if (p && bytes) wr[nwr++] = {reinterpret_cast<uintptr_t>(p), reinterpret_cast<uintptr_t>(p) + bytes};
+  }
+};
+struct CaptureLast {          // the last flat launch of one capture sequence
+  unsigned long long id;
+  cudaGraphNode_t node;       // nullptr: free slot
+  FlatAccess acc;
+};
+constexpr int kCaptureSlots = 16;   // concurrent capture sequences tracked; an evicted one only loses the overlap
+static std::mutex g_capture_mu;
+static CaptureLast g_capture[kCaptureSlots];
+static int g_capture_next = 0;
+static thread_local int g_overlap_count = 0;
+
+// the stream's capture id and its single pending dependency; false when not capturing or not exactly one
+static bool capture_tip(cudaStream_t st, unsigned long long* id, cudaGraphNode_t* node) {
+  cudaStreamCaptureStatus status = cudaStreamCaptureStatusNone;
+  const cudaGraphNode_t* deps = nullptr;
+  size_t ndeps = 0;
+  if (cudaStreamGetCaptureInfo(st, &status, id, nullptr, &deps, &ndeps) != cudaSuccess) {
+    (void)cudaGetLastError();   // the launch that follows reports any real problem with the stream
+    return false;
+  }
+  if (status != cudaStreamCaptureStatusActive || ndeps != 1 || deps[0] == nullptr) return false;
+  *node = deps[0];
+  return true;
+}
+
+// before the launch: 1 when it may load ahead of pdl_wait(), 0 (wait first) otherwise
+static int capture_check(cudaStream_t st, const FlatAccess& a) {
+  unsigned long long id = 0;
+  cudaGraphNode_t node = nullptr;
+  if (!pdl_enabled() || !capture_tip(st, &id, &node)) return 0;
+  std::lock_guard<std::mutex> lock(g_capture_mu);
+  for (const CaptureLast& c : g_capture) {
+    if (c.node != node || c.id != id) continue;
+    for (int r = 0; r < a.nrd; ++r)
+      for (int w = 0; w < c.acc.nwr; ++w)
+        if (a.rd[r].beg < c.acc.wr[w].end && c.acc.wr[w].beg < a.rd[r].end) return 0;
+    return 1;
+  }
+  return 0;
+}
+
+// after a successful launch: it is now the capture's single dependency
+static void capture_record(cudaStream_t st, const FlatAccess& a, int independent) {
+  unsigned long long id = 0;
+  cudaGraphNode_t node = nullptr;
+  if (!pdl_enabled() || !capture_tip(st, &id, &node)) return;
+  if (independent) ++g_overlap_count;
+  std::lock_guard<std::mutex> lock(g_capture_mu);
+  CaptureLast* slot = nullptr;
+  for (CaptureLast& c : g_capture)
+    if (c.node != nullptr && c.id == id) slot = &c;
+  if (!slot) slot = &g_capture[g_capture_next++ % kCaptureSlots];
+  slot->id = id;
+  slot->node = node;
+  slot->acc = a;
+}
+
 template <int FORM, typename T>
 static int launch_fwd(const void* x, void* y, void* codes, const dlmcq_layout* l, const dlmcq_qparams* qp,
                       cudaStream_t st) {
@@ -614,10 +738,19 @@ static int launch_fwd(const void* x, void* y, void* codes, const dlmcq_layout* l
       // 2^26..2^28 elements vs 5.9-6.0 for a persistent grid-stride grid (profiles/README.md).
       auto kern = fq_fwd_flat<FORM, T, kUnroll, 4, true>;
       const int bps = 1024;
+      const size_t bytes = static_cast<size_t>(n) * sizeof(T);
+      FlatAccess acc;
+      acc.read(x, bytes);
+      acc.read(qp->scale, sizeof(float));
+      acc.read(qp->offset, sizeof(float));
+      acc.write(y, bytes);
+      acc.write(codes, bytes);
+      const int independent = capture_check(st, acc);
       cudaError_t e = launch_pdl(kern, dim3(stream_grid(tiles, bps)), dim3(kThreads), 0, st,
                                  static_cast<const T*>(x), static_cast<T*>(y), static_cast<T*>(codes), n, qp->scale,
-                                 qp->offset, qp->g, lo, hi);
+                                 qp->offset, qp->g, lo, hi, independent);
       if (e != cudaSuccess) return set_cuda_error(e);
+      capture_record(st, acc, independent);
     } else {
       const int64_t tiles = (n + kThreads - 1) / kThreads;
       fq_fwd_flat_unaligned<FORM, T><<<stream_grid(tiles, 8), kThreads, 0, st>>>(
@@ -673,10 +806,25 @@ static int launch_bwd(const void* x, const void* dy, void* dx, float* dscale, fl
     auto k = vec ? (doffset ? fq_bwd_flat<FORM, T, true, true, false> : fq_bwd_flat<FORM, T, true, false, false>)
                  : (doffset ? fq_bwd_flat<FORM, T, false, true, false> : fq_bwd_flat<FORM, T, false, false, false>);
     if (defer) k = vec ? fq_bwd_flat<FORM, T, true, false, true> : fq_bwd_flat<FORM, T, false, false, true>;
+    FlatAccess acc;
+    if (vec) {
+      const size_t bytes = static_cast<size_t>(n) * sizeof(T);
+      acc.read(x, bytes);
+      acc.read(dy, bytes);
+      acc.read(qp->scale, sizeof(float));
+      acc.read(qp->offset, sizeof(float));
+      if (!defer) acc.read(ws, ws_bytes);        // ticket counter and partials
+      acc.write(dx, bytes);
+      acc.write(dscale, sizeof(float));
+      acc.write(doffset, sizeof(float));
+      acc.write(ws, defer ? (2 + 2 * static_cast<size_t>(grid)) * sizeof(float) : ws_bytes);
+    }
+    const int independent = vec ? capture_check(st, acc) : 0;
     cudaError_t e = launch_pdl(k, dim3(grid), dim3(kThreads), 0, st, static_cast<const T*>(x),
                                static_cast<const T*>(dy), static_cast<T*>(dx), n, qp->scale, qp->offset, qp->g, lo, hi,
-                               dscale, doffset, ws);
+                               dscale, doffset, ws, independent);
     if (e != cudaSuccess) return set_cuda_error(e);
+    if (vec) capture_record(st, acc, independent);
   } else if (doffset == nullptr && n > 0 && tiled_ok<T>(l, x, dy, dx)) {
     const TileGeom tg = make_tile_geom<T>(l);
     const int64_t tiles = (tg.nvec + kTileVecs - 1) / kTileVecs;
@@ -751,6 +899,8 @@ static int dispatch_bwd(const void* x, const void* dy, void* dx, float* ds, floa
 __global__ void __launch_bounds__(kThreads)
 finalize_many_kernel(const dlmcq_finalize_item* __restrict__ items, int n_items) {
   __shared__ double sm[2][kThreads / 32];
+  pdl_wait();          // the partials come from the backward launches before it
+  pdl_trigger();
   const dlmcq_finalize_item it = items[blockIdx.x];
   const float* p = it.partials;
   const int nblocks = __float_as_int(p[0]);
@@ -852,10 +1002,17 @@ extern "C" int dlmcq_fq_backward_partials(const void* x, const void* dy, void* d
              : dispatch_bwd<__nv_bfloat16>(x, dy, dx, nullptr, nullptr, layout, qp, partials, 0, st, true);
 }
 
+extern "C" int dlmcq_capture_overlap_count(void) {
+  const int n = g_overlap_count;
+  g_overlap_count = 0;
+  return n;
+}
+
 extern "C" int dlmcq_fq_finalize_many(const dlmcq_finalize_item* items, int n_items, void* stream) {
   if (!items || n_items < 0) return DLMCQ_EINVAL;
   if (n_items == 0) return DLMCQ_OK;
-  finalize_many_kernel<<<n_items, kThreads, 0, static_cast<cudaStream_t>(stream)>>>(items, n_items);
-  DLMCQ_LAUNCH_CHECK();
+  cudaError_t e = launch_pdl(finalize_many_kernel, dim3(n_items), dim3(kThreads), 0, static_cast<cudaStream_t>(stream),
+                             items, n_items);
+  if (e != cudaSuccess) return set_cuda_error(e);
   return DLMCQ_OK;
 }

@@ -28,6 +28,8 @@ template <typename T>
 __global__ void __launch_bounds__(kRowWarps * 32)
 grouped_fwd_kernel(const dlmcq_group_item* __restrict__ items, const int64_t* __restrict__ prefix, int n_items,
                    int64_t total_units) {
+  pdl_wait();          // the inputs and the device table: written by earlier work the host cannot see
+  pdl_trigger();
   const int lane = threadIdx.x & 31;
   const int64_t unit = static_cast<int64_t>(blockIdx.x) * kRowWarps + (threadIdx.x >> 5);
   if (unit >= total_units) return;
@@ -53,6 +55,8 @@ template <typename T>
 __global__ void __launch_bounds__(kRowWarps * 32)
 grouped_bwd_kernel(const dlmcq_group_item* __restrict__ items, const int64_t* __restrict__ prefix, int n_items,
                    int64_t total_units, float* __restrict__ partials) {
+  pdl_wait();
+  pdl_trigger();
   const int lane = threadIdx.x & 31;
   const int64_t unit = static_cast<int64_t>(blockIdx.x) * kRowWarps + (threadIdx.x >> 5);
   if (unit >= total_units) return;
@@ -83,6 +87,8 @@ __global__ void __launch_bounds__(kRowWarps * 32)
 grouped_finalize_kernel(const dlmcq_group_item* __restrict__ items, const int64_t* __restrict__ prefix,
                         const int64_t* __restrict__ chan_prefix, int n_items, int64_t total_channels,
                         const float* __restrict__ partials) {
+  pdl_wait();          // the partials come from grouped_bwd_kernel launched just before
+  pdl_trigger();
   const int lane = threadIdx.x & 31;
   const int64_t gch = static_cast<int64_t>(blockIdx.x) * kRowWarps + (threadIdx.x >> 5);
   if (gch >= total_channels) return;
@@ -112,13 +118,11 @@ extern "C" int dlmcq_fq_forward_grouped(const dlmcq_group_item* items, const int
   const int64_t blocks = (total_units + kRowWarps - 1) / kRowWarps;
   if (blocks > 0x7fffffffLL) return DLMCQ_EUNSUPPORTED;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (dtype == DLMCQ_F32)
-    grouped_fwd_kernel<float><<<static_cast<unsigned>(blocks), kRowWarps * 32, 0, st>>>(items, unit_prefix, n_items, total_units);
-  else if (dtype == DLMCQ_BF16)
-    grouped_fwd_kernel<__nv_bfloat16><<<static_cast<unsigned>(blocks), kRowWarps * 32, 0, st>>>(items, unit_prefix, n_items, total_units);
-  else
-    return DLMCQ_EINVAL;
-  DLMCQ_LAUNCH_CHECK();
+  if (dtype != DLMCQ_F32 && dtype != DLMCQ_BF16) return DLMCQ_EINVAL;
+  cudaError_t e = launch_pdl(dtype == DLMCQ_F32 ? grouped_fwd_kernel<float> : grouped_fwd_kernel<__nv_bfloat16>,
+                             dim3(static_cast<unsigned>(blocks)), dim3(kRowWarps * 32), 0, st, items, unit_prefix,
+                             n_items, total_units);
+  if (e != cudaSuccess) return set_cuda_error(e);
   return DLMCQ_OK;
 }
 
@@ -131,14 +135,13 @@ extern "C" int dlmcq_fq_backward_grouped(const dlmcq_group_item* items, const in
   const int64_t fblocks = (total_channels + kRowWarps - 1) / kRowWarps;
   if (blocks > 0x7fffffffLL || fblocks > 0x7fffffffLL) return DLMCQ_EUNSUPPORTED;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (dtype == DLMCQ_F32)
-    grouped_bwd_kernel<float><<<static_cast<unsigned>(blocks), kRowWarps * 32, 0, st>>>(items, unit_prefix, n_items, total_units, partials);
-  else if (dtype == DLMCQ_BF16)
-    grouped_bwd_kernel<__nv_bfloat16><<<static_cast<unsigned>(blocks), kRowWarps * 32, 0, st>>>(items, unit_prefix, n_items, total_units, partials);
-  else
-    return DLMCQ_EINVAL;
-  DLMCQ_LAUNCH_CHECK();
-  grouped_finalize_kernel<<<static_cast<unsigned>(fblocks), kRowWarps * 32, 0, st>>>(items, unit_prefix, chan_prefix, n_items, total_channels, partials);
-  DLMCQ_LAUNCH_CHECK();
+  if (dtype != DLMCQ_F32 && dtype != DLMCQ_BF16) return DLMCQ_EINVAL;
+  cudaError_t e = launch_pdl(dtype == DLMCQ_F32 ? grouped_bwd_kernel<float> : grouped_bwd_kernel<__nv_bfloat16>,
+                             dim3(static_cast<unsigned>(blocks)), dim3(kRowWarps * 32), 0, st, items, unit_prefix,
+                             n_items, total_units, partials);
+  if (e != cudaSuccess) return set_cuda_error(e);
+  e = launch_pdl(grouped_finalize_kernel, dim3(static_cast<unsigned>(fblocks)), dim3(kRowWarps * 32), 0, st, items,
+                 unit_prefix, chan_prefix, n_items, total_channels, partials);
+  if (e != cudaSuccess) return set_cuda_error(e);
   return DLMCQ_OK;
 }

@@ -128,6 +128,13 @@ int dlmcq_fq_backward_partials(const void* x, const void* dy, void* dx, const dl
                                const dlmcq_qparams* qp, float* partials, void* stream);
 int dlmcq_fq_finalize_many(const dlmcq_finalize_item* items, int n_items, void* stream);
 
+/* Diagnostic: the number of per-tensor (channels == 1, 16-byte aligned) forward / backward launches that this
+ * thread captured into a CUDA graph as independent of their predecessor since the previous call, then resets it.
+ * Such a launch directly follows another of these launches in the same capture sequence, and it reads nothing
+ * that launch writes; its CTAs then load their first tile while the predecessor is still running.  Eager
+ * launches never count. */
+int dlmcq_capture_overlap_count(void);
+
 /* utils.py:29-37 round_pass / floor_pass values and RootQ/function.py:5-8 sgn:
  * mode 0: (round(x)-x)+x   mode 1: (floor(x)-x)+x   mode 2: sign(x) (sign(NaN)=0) */
 int dlmcq_ste_value(const void* x, void* y, int64_t numel, int dtype, int mode, void* stream);
