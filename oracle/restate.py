@@ -120,6 +120,29 @@ def bn_act_fq_chain(x, gamma, beta, running_mean, running_var, training, momentu
     return a, fq_affine(a, scale, offset, lo, hi, g)
 
 
+def fma_f32(a, b, c):
+    """fp32 fma(a, b, c) rounded ONCE to nearest-even, as the fused kernels' __fmaf_rn / __ffma2_rn compute it
+    (the fused BatchNorm's z = fma(x - mean, gamma * invstd, beta)), from float32 tensors of one shape.
+    a * b is exact in float64 (24 + 24 significant bits); the float64 sum s = RN64(a*b + c) can differ from the exact
+    sum, and rounding s to fp32 then gives a different result from rounding the exact sum in exactly one case: s lands
+    on the midpoint of two fp32 neighbours while the exact sum does not.  TwoSum recovers the exact error e of s, and
+    the sign of e says on which side of that midpoint the exact sum lies.  Non-finite sums are rounded as they are.
+    One case is not corrected: a float64 sum exactly on the fp32 overflow threshold 2^128 - 2^103 with the exact sum
+    below it returns inf where fmaf returns FLT_MAX (the midpoint there is computed as inf).  Callers stay far below."""
+    p = a.double() * b.double()
+    cd = c.double()
+    s = p + cd
+    bb = s - p
+    e = (p - (s - bb)) + (cd - bb)                 # TwoSum: p + c == s + e exactly (finite s)
+    r = s.float()
+    rd = r.double()
+    up = s > rd
+    toward = torch.nextafter(r, torch.where(up, torch.full_like(r, math.inf), torch.full_like(r, -math.inf)))
+    mid = (rd + toward.double()) * 0.5              # exact in float64
+    fix = (s == mid) & ((e > 0) | (e < 0)) & ((e > 0) == up)     # e is NaN for a non-finite s
+    return torch.where(fix, toward, r)
+
+
 def lsq_init_scale(x, qmax):
     """modules/base.py:84,119 - LSQ initial scale 2*mean|x|/sqrt(qmax)."""
     return 2 * x.detach().abs().mean() / math.sqrt(qmax)
