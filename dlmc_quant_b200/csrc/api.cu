@@ -27,23 +27,6 @@ int num_sms() {
   return cached[dev];
 }
 
-int64_t cmaj_max_inner() {
-  static const int64_t v = [] {
-    const char* e = getenv("DLMCQ_CMAJ_MAX_INNER");
-    const long long t = e ? atoll(e) : 0;
-    return static_cast<int64_t>(t > 0 ? t : kCmajMaxInner);
-  }();
-  return v;
-}
-
-bool slab_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("DLMCQ_NO_SLAB");
-    return !(e && e[0] == '1');
-  }();
-  return on;
-}
-
 bool pdl_enabled() {
   static const bool on = [] {
     const char* e = getenv("DLMCQ_NO_PDL");

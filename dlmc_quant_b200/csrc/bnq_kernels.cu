@@ -24,8 +24,6 @@
 // same `fq_vec<FORM_AFFINE>` code as the stand-alone kernels: given the BatchNorm output `a` (which the kernel
 // can also write), a_q is BIT-IDENTICAL to dlmcq_fq_forward(a) - that is how parity with the reference's
 // quantizer chain is carried over (tests: fused a_q == fq_forward(fused a)).
-#include <stdlib.h>
-
 #include "fq_math.cuh"
 
 namespace dlmcq {
@@ -639,8 +637,9 @@ __device__ __forceinline__ float2 dz_pair(float2 act, float2 dq, float2 da_in, b
   return make_float2(up0 ? da.x : 0.f, up1 ? da.y : 0.f);
 }
 
-// U / MINB: rows in flight per thread and resident CTAs per SM.  The recomputing quantizer variants carry ~100 live
-// registers with four rows in flight: <4, 2> keeps them all, <2, 3> trades rows in flight for a third resident CTA.
+// U / MINB: rows in flight per thread and resident CTAs per SM.  The recomputing quantizer variant carries ~100 live
+// registers with four rows in flight and runs <4, 2>, which keeps them all; the residual variants run <2, 3> and the
+// plain BatchNorm variant <4, 3>.
 template <typename T, bool RESID, bool QUANT, int U, int MINB>
 __global__ void __launch_bounds__(kBnqThreads, MINB)
 bnq_bwd_reduce_kernel(const T* __restrict__ x, const T* __restrict__ a_saved, const T* __restrict__ d_a,
@@ -649,7 +648,7 @@ bnq_bwd_reduce_kernel(const T* __restrict__ x, const T* __restrict__ a_saved, co
                       BnqGeom gm, int relu, const float* __restrict__ scale, const float* __restrict__ offset, float g,
                       float lo, float hi, float* __restrict__ part, float* __restrict__ part_s,
                       uint32_t* __restrict__ keep_mask) {
-  // keep_mask (plain quantizer chain, U == kBnqU): bit (u * VN + e) of word [(tile * gy + blockIdx.y) * 256 + thread]
+  // keep_mask (plain quantizer chain): bit (u * VN + e) of word [(tile * gy + blockIdx.y) * 256 + thread]
   // says "dz == d_q" for that element (inside the clamp range and above the ReLU floor), so that the dx pass needs
   // neither the quantizer arithmetic nor its ~60 extra registers - 1/8 byte per element written here, read there.
   using V = Vec<T>;
@@ -839,23 +838,25 @@ bnq_bwd_finalize_kernel(const float* __restrict__ part, const float* __restrict_
 }
 
 // pass 2: dx = gamma*invstd * (dz - mean(dz) - xhat * mean(dz*xhat))     (eval mode: gamma*invstd * dz)
-template <typename T, bool RESID, bool QUANT, int U, int MINB>
+// Generic form: dz is recomputed from x and the upstream gradients (the light kernel below covers the residual form
+// and the plain quantizer chain without d_a).  MINB: resident CTAs per SM, 2 with the quantizer, 3 without.
+template <typename T, bool QUANT, int MINB>
 __global__ void __launch_bounds__(kBnqThreads, MINB)
-bnq_bwd_dx_kernel(const T* __restrict__ x, const T* __restrict__ dz_in, const T* __restrict__ d_a,
-                  const T* __restrict__ d_q, const float* __restrict__ gamma, const float* __restrict__ beta,
-                  const float* __restrict__ mean, const float* __restrict__ invstd, const float* __restrict__ coef,
-                  T* __restrict__ dx, BnqGeom gm, int relu, const float* __restrict__ scale,
-                  const float* __restrict__ offset, float g, float lo, float hi) {
+bnq_bwd_dx_kernel(const T* __restrict__ x, const T* __restrict__ d_a, const T* __restrict__ d_q,
+                  const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ mean,
+                  const float* __restrict__ invstd, const float* __restrict__ coef, T* __restrict__ dx, BnqGeom gm,
+                  int relu, const float* __restrict__ scale, const float* __restrict__ offset, float g, float lo,
+                  float hi) {
   using V = Vec<T>;
   using raw = typename V::raw;
   constexpr int VN = V::N;
+  constexpr int U = kBnqU;
   const int tx = static_cast<int>(threadIdx.x) % gm.txw;
   const int ty = static_cast<int>(threadIdx.x) / gm.txw;
   const int col = static_cast<int>(blockIdx.y) * gm.txw + tx;
   const bool active = (col < gm.cv) && (ty < gm.ty);
   const bool has_da = d_a != nullptr;
   const raw* xv = reinterpret_cast<const raw*>(x);
-  const raw* zv = reinterpret_cast<const raw*>(dz_in);
   const raw* dav = reinterpret_cast<const raw*>(d_a);
   const raw* dqv = reinterpret_cast<const raw*>(d_q);
   raw* ov = reinterpret_cast<raw*>(dx);
@@ -867,12 +868,8 @@ bnq_bwd_dx_kernel(const T* __restrict__ x, const T* __restrict__ dz_in, const T*
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       rx[u] = ld_stream(xv + o + u * tl.du);
-      if (RESID) {
-        r1[u] = ld_stream(zv + o + u * tl.du);
-      } else {
-        if (has_da) r1[u] = ld_stream(dav + o + u * tl.du);
-        if (QUANT) r2[u] = ld_stream(dqv + o + u * tl.du);
-      }
+      if (has_da) r1[u] = ld_stream(dav + o + u * tl.du);
+      if (QUANT) r2[u] = ld_stream(dqv + o + u * tl.du);
     }
   };
   // everything except coef is older than the finalisation kernel this launch depends on: fetch it before the wait
@@ -899,7 +896,7 @@ bnq_bwd_dx_kernel(const T* __restrict__ x, const T* __restrict__ dz_in, const T*
   // dz of one vector (packed when `fast`), then the BatchNorm input gradient
   auto finish_vec = [&](const float (&fx)[VN], const float (&f1)[VN], const float (&f2)[VN], bool fast, int64_t idx) {
     float dzs[VN], o[VN];
-    if (!RESID && !fast) {
+    if (!fast) {
       float dummy = 0.f;
       bnq_dz_vec<T, VN, false, QUANT>(fx, fx, has_da ? f1 : nullptr, f2, unpack_bnch<VN>(c2), relu != 0, k.p, lo, hi, dummy,
                                       dzs);
@@ -908,9 +905,7 @@ bnq_bwd_dx_kernel(const T* __restrict__ x, const T* __restrict__ dz_in, const T*
     for (int e = 0; e < VN; e += 2) {
       const float2 tt = __fadd2_rn(make_float2(fx[e], fx[e + 1]), c2.nmean[e / 2]);
       float2 d2;
-      if (RESID) {
-        d2 = make_float2(f1[e], f1[e + 1]);
-      } else if (fast) {
+      if (fast) {
         float2 dummy2 = make_float2(0.f, 0.f);
         bool k0, k1;
         const float2 act = round_to_storage<T>(act_pair(__ffma2_rn(tt, c2.a[e / 2], c2.b[e / 2]), floor));
@@ -935,9 +930,9 @@ bnq_bwd_dx_kernel(const T* __restrict__ x, const T* __restrict__ dz_in, const T*
     for (int u = 0; u < U; ++u) {
       float fx[VN], f1[VN], f2[VN];
       V::unpack(rx[u], fx);
-      if (RESID || has_da) V::unpack(r1[u], f1);
-      if (!RESID && QUANT) V::unpack(r2[u], f2);
-      const bool fast = RESID || (fast_ok && absmax_vec<VN>(fx, 0.f) <= kBnqSafe);
+      if (has_da) V::unpack(r1[u], f1);
+      if (QUANT) V::unpack(r2[u], f2);
+      const bool fast = fast_ok && absmax_vec<VN>(fx, 0.f) <= kBnqSafe;
       finish_vec(fx, f1, f2, fast, off + u * tl.du);
     }
     t += gridDim.x;
@@ -952,10 +947,9 @@ bnq_bwd_dx_kernel(const T* __restrict__ x, const T* __restrict__ dz_in, const T*
       const int64_t idx = row * gm.cv + col;
       float fx[VN], f1[VN], f2[VN];
       V::unpack(ld_stream(xv + idx), fx);
-      if (RESID) V::unpack(ld_stream(zv + idx), f1);
-      else if (has_da) V::unpack(ld_stream(dav + idx), f1);
-      if (!RESID && QUANT) V::unpack(ld_stream(dqv + idx), f2);
-      finish_vec(fx, f1, f2, RESID, idx);
+      if (has_da) V::unpack(ld_stream(dav + idx), f1);
+      if (QUANT) V::unpack(ld_stream(dqv + idx), f2);
+      finish_vec(fx, f1, f2, false, idx);
     }
   }
 }
@@ -1053,77 +1047,9 @@ bnq_bwd_dx_light_kernel(const T* __restrict__ x, const T* __restrict__ src /* dz
   }
 }
 
-// A/B aid (DLMCQ_BNQ_DXV=1): the first, scalar version of the dz -> dx pass
-template <typename T>
-__global__ void __launch_bounds__(kBnqThreads, 3)
-bnq_bwd_dx_scalar_kernel(const T* __restrict__ x, const T* __restrict__ dz_in, const float* __restrict__ gamma,
-                         const float* __restrict__ beta, const float* __restrict__ mean, const float* __restrict__ invstd,
-                         const float* __restrict__ coef, T* __restrict__ dx, BnqGeom gm) {
-  using V = Vec<T>;
-  using raw = typename V::raw;
-  constexpr int VN = V::N;
-  BNQ_THREAD_COORDS();
-  if (!active) return;
-  BnCh<VN> c;
-  load_bnch<VN>(c, gamma, beta, mean, invstd, col * VN);
-  float c1[VN], c2[VN];
-#pragma unroll
-  for (int e = 0; e < VN; ++e) {
-    c1[e] = __ldg(coef + col * VN + e);
-    c2[e] = __ldg(coef + gm.C + col * VN + e);
-  }
-  const raw* xv = reinterpret_cast<const raw*>(x);
-  const raw* zv = reinterpret_cast<const raw*>(dz_in);
-  raw* ov = reinterpret_cast<raw*>(dx);
-  for (int64_t r0 = static_cast<int64_t>(blockIdx.x) * rpp; r0 < gm.rows; r0 += static_cast<int64_t>(gridDim.x) * rpp) {
-    raw rx[kBnqU], r1[kBnqU];
-    bool ok[kBnqU];
-#pragma unroll
-    for (int u = 0; u < kBnqU; ++u) {
-      const int64_t row = r0 + ty + static_cast<int64_t>(u) * gm.ty;
-      ok[u] = row < gm.rows;
-      if (ok[u]) {
-        const int64_t idx = row * gm.cv + col;
-        rx[u] = ld_stream(xv + idx);
-        r1[u] = ld_stream(zv + idx);
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < kBnqU; ++u) {
-      if (!ok[u]) continue;
-      const int64_t idx = (r0 + ty + static_cast<int64_t>(u) * gm.ty) * gm.cv + col;
-      float fx[VN], dz[VN], o[VN];
-      V::unpack(rx[u], fx);
-      V::unpack(r1[u], dz);
-#pragma unroll
-      for (int e = 0; e < VN; ++e) {
-        const float xh = (fx[e] - c.mean[e]) * c.istd[e];
-        const float t = __fmaf_rn(-xh, c2[e], dz[e] - c1[e]);
-        o[e] = c.a[e] * t;
-      }
-      st_stream(ov + idx, V::pack(o));
-    }
-  }
-}
-
 // ---------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------
-// tuning aids (environment): DLMCQ_BNQ_TILES tiles per CTA of the streaming kernels (default 8), DLMCQ_BNQ_U rows in
-// flight per thread of the recomputing quantizer kernels (2 -> <2 rows, 3 CTAs/SM>, default 4 -> <4 rows, 2 CTAs/SM>)
-static inline int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return (e && e[0]) ? atoi(e) : dflt;
-}
-static inline int tiles_per_cta() {
-  static const int v = env_int("DLMCQ_BNQ_TILES", 8);
-  return v;
-}
-static inline int recompute_rows() {
-  static const int v = env_int("DLMCQ_BNQ_U", 4);
-  return v;
-}
-
 static inline int bnq_check(const dlmcq_bnq_desc* d) {
   if (!d || d->rows < 0 || d->channels < 1) return DLMCQ_EINVAL;
   if (d->dtype != DLMCQ_F32 && d->dtype != DLMCQ_BF16) return DLMCQ_EINVAL;
@@ -1131,13 +1057,13 @@ static inline int bnq_check(const dlmcq_bnq_desc* d) {
   if (d->channels % vn != 0 || d->channels > (int64_t(1) << 20)) return DLMCQ_EUNSUPPORTED;
   return DLMCQ_OK;
 }
-// CTAs along the rows for the non-reducing kernels: about four tiles per CTA (amortises the per-thread set-up) but
+// CTAs along the rows for the non-reducing kernels: about `tiles` tiles per CTA (amortises the per-thread set-up) but
 // never fewer CTAs than 8 per SM while the tensor has that many tiles
-static inline int apply_grid(const BnqGeom& g, int u = kBnqU, int tiles = 0) {
-  const int64_t rpp = static_cast<int64_t>(g.ty) * u;
+static inline int apply_grid(const BnqGeom& g, int tiles) {
+  const int64_t rpp = static_cast<int64_t>(g.ty) * kBnqU;
   const int64_t passes = (g.rows + rpp - 1) / rpp;
   const int64_t floor_ctas = static_cast<int64_t>(num_sms()) * 8 / g.gy;
-  int64_t n = passes / (tiles > 0 ? tiles : tiles_per_cta());
+  int64_t n = passes / tiles;
   if (n < floor_ctas) n = floor_ctas;
   if (n > passes) n = passes;
   return n < 1 ? 1 : static_cast<int>(n);
@@ -1175,7 +1101,7 @@ static int bnq_forward_t(const void* x, const void* idn, const float* gamma, con
   const float* sc = quant ? qp->scale : nullptr;
   const float* of = quant ? qp->offset : nullptr;
   const float gq = quant ? qp->g : 0.f;
-  const dim3 grid(apply_grid(g), g.gy);
+  const dim3 grid(apply_grid(g, 8), g.gy);
   auto k = idn ? (quant ? bnq_apply_kernel<T, true, true> : bnq_apply_kernel<T, true, false>)
                : (quant ? bnq_apply_kernel<T, false, true> : bnq_apply_kernel<T, false, false>);
   cudaError_t e = launch_pdl(k, grid, dim3(kBnqThreads), 0, st, xt, static_cast<const T*>(idn), gamma, beta,
@@ -1206,14 +1132,11 @@ static int bnq_backward_t(const void* x, const void* a_saved, const void* d_a, c
   const T* at = static_cast<const T*>(a_saved);
   const T* dat = static_cast<const T*>(d_a);
   const T* dqt = static_cast<const T*>(d_q);
-  static const int light = env_int("DLMCQ_BNQ_LIGHT", 1);
   // plain quantizer chain without a plain-output gradient: the reduce pass leaves a keep mask for a light dx pass
-  const bool masked = light == 1 && !resid && quant && d_a == nullptr && dx != nullptr && recompute_rows() != 2;
+  const bool masked = !resid && quant && d_a == nullptr && dx != nullptr;
   {
-    const bool u2 = recompute_rows() == 2;
     auto k = resid ? (quant ? bnq_bwd_reduce_kernel<T, true, true, 2, 3> : bnq_bwd_reduce_kernel<T, true, false, 2, 3>)
-                   : (quant ? (u2 ? bnq_bwd_reduce_kernel<T, false, true, 2, 3> : bnq_bwd_reduce_kernel<T, false, true, 4, 2>)
-                            : bnq_bwd_reduce_kernel<T, false, false, 4, 3>);
+                   : (quant ? bnq_bwd_reduce_kernel<T, false, true, 4, 2> : bnq_bwd_reduce_kernel<T, false, false, 4, 3>);
     cudaError_t e = launch_pdl(k, dim3(g.nbx, g.gy), dim3(kBnqThreads), bnq_smem<VN>(g), st, xt, at, dat, dqt, gamma, beta,
                                smean, sinv, static_cast<T*>(dz_out), g, relu, sc, of, gq, lo, hi, w.part, w.part_s,
                                masked ? w.mask : static_cast<uint32_t*>(nullptr));
@@ -1226,31 +1149,20 @@ static int bnq_backward_t(const void* x, const void* a_saved, const void* d_a, c
                                quant ? dscale : static_cast<float*>(nullptr));
     if (e != cudaSuccess) return set_cuda_error(e);
   }
-  static const int dxv = env_int("DLMCQ_BNQ_DXV", 0);
-  if (dx && resid && dxv == 1) {
-    const int64_t rpp = static_cast<int64_t>(g.ty) * kBnqU;
-    const int64_t passes = (g.rows + rpp - 1) / rpp;
-    bnq_bwd_dx_scalar_kernel<T><<<dim3(static_cast<unsigned>(passes), g.gy), kBnqThreads, 0, st>>>(
-        xt, static_cast<const T*>(dz_out), gamma, beta, smean, sinv, w.coef, static_cast<T*>(dx), g);
-    DLMCQ_LAUNCH_CHECK();
-  } else if (dx && light == 1 && (resid || masked)) {
-    static const int light_tiles = env_int("DLMCQ_BNQ_TILES_LIGHT", 8);
+  if (!dx) return DLMCQ_OK;
+  const dim3 grid(apply_grid(g, 8), g.gy);
+  cudaError_t e;
+  if (resid || masked) {
     auto k = resid ? bnq_bwd_dx_light_kernel<T, false> : bnq_bwd_dx_light_kernel<T, true>;
-    cudaError_t e = launch_pdl(k, dim3(apply_grid(g, kBnqU, light_tiles), g.gy), dim3(kBnqThreads), 0, st, xt,
-                               resid ? static_cast<const T*>(dz_out) : dqt, static_cast<const uint32_t*>(w.mask), gamma,
-                               beta, smean, sinv, static_cast<const float*>(w.coef), static_cast<T*>(dx), g);
-    if (e != cudaSuccess) return set_cuda_error(e);
-  } else if (dx) {
-    const bool u2 = !resid && quant && recompute_rows() == 2;
-    const dim3 grid(apply_grid(g, u2 ? 2 : kBnqU), g.gy);
-    auto k = resid ? bnq_bwd_dx_kernel<T, true, false, 4, 3>
-                   : (quant ? (u2 ? bnq_bwd_dx_kernel<T, false, true, 2, 3> : bnq_bwd_dx_kernel<T, false, true, 4, 2>)
-                            : bnq_bwd_dx_kernel<T, false, false, 4, 3>);
-    cudaError_t e = launch_pdl(k, grid, dim3(kBnqThreads), 0, st, xt, static_cast<const T*>(dz_out), dat, dqt, gamma, beta,
-                               smean, sinv, static_cast<const float*>(w.coef), static_cast<T*>(dx), g, relu, sc, of, gq,
-                               lo, hi);
-    if (e != cudaSuccess) return set_cuda_error(e);
+    e = launch_pdl(k, grid, dim3(kBnqThreads), 0, st, xt, resid ? static_cast<const T*>(dz_out) : dqt,
+                   static_cast<const uint32_t*>(w.mask), gamma, beta, smean, sinv, static_cast<const float*>(w.coef),
+                   static_cast<T*>(dx), g);
+  } else {
+    auto k = quant ? bnq_bwd_dx_kernel<T, true, 2> : bnq_bwd_dx_kernel<T, false, 3>;
+    e = launch_pdl(k, grid, dim3(kBnqThreads), 0, st, xt, dat, dqt, gamma, beta, smean, sinv,
+                   static_cast<const float*>(w.coef), static_cast<T*>(dx), g, relu, sc, of, gq, lo, hi);
   }
+  if (e != cudaSuccess) return set_cuda_error(e);
   return DLMCQ_OK;
 }
 

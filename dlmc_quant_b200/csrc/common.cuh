@@ -220,9 +220,8 @@ constexpr int kCmajUnroll = 8;
 constexpr int64_t kCmajMaxInner = 256;
 
 // short rows, more than one batch index, and 32-bit element offsets inside one work item
-int64_t cmaj_max_inner();   // kCmajMaxInner unless overridden by DLMCQ_CMAJ_MAX_INNER (tuning aid)
 inline bool cmaj_ok(int64_t outer, int64_t channels, int64_t inner) {
-  return outer > 1 && inner >= 1 && inner < cmaj_max_inner() && channels * 8192 < (int64_t(1) << 31);
+  return outer > 1 && inner >= 1 && inner < kCmajMaxInner && channels * 8192 < (int64_t(1) << 31);
 }
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
@@ -260,12 +259,11 @@ struct SlabGeom {
   int32_t groups;       // C / G
 };
 constexpr int kSlabUnroll = 4;
-bool slab_enabled();    // DLMCQ_NO_SLAB=1 falls back to the scalar channel-major kernels (A/B aid)
 template <typename T>
 inline bool slab_ok(int64_t outer, int64_t channels, int64_t inner, const void* a, const void* b, const void* c,
                     const void* d) {
   constexpr int VEC = Vec<T>::N;
-  if (!slab_enabled() || !cmaj_ok(outer, channels, inner) || inner % VEC == 0) return false;
+  if (!cmaj_ok(outer, channels, inner) || inner % VEC == 0) return false;
   int g = 1;
   while ((inner * g) % VEC != 0) g <<= 1;                  // VEC / gcd(inner, VEC): a power of two <= VEC
   return channels % g == 0 && aligned16(a) && aligned16(b) && aligned16(c) && aligned16(d) &&

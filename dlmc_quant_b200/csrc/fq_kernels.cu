@@ -21,10 +21,10 @@ constexpr int kUnroll = 4;
 // ---------------------------------------------------------------------------------------
 // flat forward
 // ---------------------------------------------------------------------------------------
-// independent (TILED only): the host proved that the preceding launch writes nothing this one reads
-// (capture_check), so the qparams and the first tile are loaded before pdl_wait() and overlap its tail.
-template <int FORM, typename T, int U = kUnroll, int MINB = 4, bool TILED = false>
-__global__ void __launch_bounds__(kThreads, MINB)
+// independent: the host proved that the preceding launch writes nothing this one reads (capture_check), so the
+// qparams and the first tile are loaded before pdl_wait() and overlap its tail.
+template <int FORM, typename T>
+__global__ void __launch_bounds__(kThreads, 4)
 fq_fwd_flat(const T* __restrict__ x, T* __restrict__ y, T* __restrict__ codes, int64_t n,
             const float* __restrict__ scale, const float* __restrict__ offset, float g, float lo, float hi,
             int independent) {
@@ -32,24 +32,24 @@ fq_fwd_flat(const T* __restrict__ x, T* __restrict__ y, T* __restrict__ codes, i
   using raw = typename V::raw;
   const int64_t nvec = n / V::N;
   const raw* xv = reinterpret_cast<const raw*>(x);
-  const int64_t tile_vecs = static_cast<int64_t>(U) * blockDim.x;
+  const int64_t tile_vecs = static_cast<int64_t>(kUnroll) * blockDim.x;
   const int64_t ntiles = nvec / tile_vecs;
   ChanParams p;
-  raw r0[U];
-  const bool hoist = TILED && independent && blockIdx.x < ntiles;
-  if (TILED && independent) {
+  raw r0[kUnroll];
+  const bool hoist = independent && blockIdx.x < ntiles;
+  if (independent) {
     p = make_params<FORM>(scale, offset, 0, g, lo, hi);
     if (hoist) {
       const int64_t b = static_cast<int64_t>(blockIdx.x) * tile_vecs + threadIdx.x;
 #pragma unroll
-      for (int k = 0; k < U; ++k) r0[k] = ld_stream(xv + b + k * blockDim.x);
+      for (int k = 0; k < kUnroll; ++k) r0[k] = ld_stream(xv + b + k * blockDim.x);
     }
   }
   pdl_wait();
   pdl_trigger();
-  if (!(TILED && independent)) p = make_params<FORM>(scale, offset, 0, g, lo, hi);
+  if (!independent) p = make_params<FORM>(scale, offset, 0, g, lo, hi);
   const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
-  int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   raw* yv = reinterpret_cast<raw*>(y);
   raw* cv = reinterpret_cast<raw*>(codes);
 
@@ -60,34 +60,23 @@ fq_fwd_flat(const T* __restrict__ x, T* __restrict__ y, T* __restrict__ codes, i
     if (y) st_stream(yv + idx, V::pack(fy));
     if (codes) st_stream(cv + idx, V::pack(fc));
   };
-  if (TILED) {
-    // each CTA iteration covers one contiguous tile of U*256 vectors (16 KB for fp32, U=4)
-    int64_t t = blockIdx.x;
-    if (hoist) {
-      const int64_t b = t * tile_vecs + threadIdx.x;
+  // each CTA iteration covers one contiguous tile of kUnroll*256 vectors (16 KB for fp32)
+  int64_t t = blockIdx.x;
+  if (hoist) {
+    const int64_t b = t * tile_vecs + threadIdx.x;
 #pragma unroll
-      for (int k = 0; k < U; ++k) body(r0[k], b + k * blockDim.x);
-      t += gridDim.x;
-    }
-    for (; t < ntiles; t += gridDim.x) {
-      const int64_t b = t * tile_vecs + threadIdx.x;
-      raw r[U];
-#pragma unroll
-      for (int k = 0; k < U; ++k) r[k] = ld_stream(xv + b + k * blockDim.x);
-#pragma unroll
-      for (int k = 0; k < U; ++k) body(r[k], b + k * blockDim.x);
-    }
-    for (int64_t j = ntiles * tile_vecs + i; j < nvec; j += stride) body(ld_stream(xv + j), j);
-  } else {
-    for (; i + (U - 1) * stride < nvec; i += U * stride) {
-      raw r[U];
-#pragma unroll
-      for (int k = 0; k < U; ++k) r[k] = ld_stream(xv + i + k * stride);
-#pragma unroll
-      for (int k = 0; k < U; ++k) body(r[k], i + k * stride);
-    }
-    for (; i < nvec; i += stride) body(ld_stream(xv + i), i);
+    for (int k = 0; k < kUnroll; ++k) body(r0[k], b + k * blockDim.x);
+    t += gridDim.x;
   }
+  for (; t < ntiles; t += gridDim.x) {
+    const int64_t b = t * tile_vecs + threadIdx.x;
+    raw r[kUnroll];
+#pragma unroll
+    for (int k = 0; k < kUnroll; ++k) r[k] = ld_stream(xv + b + k * blockDim.x);
+#pragma unroll
+    for (int k = 0; k < kUnroll; ++k) body(r[k], b + k * blockDim.x);
+  }
+  for (int64_t j = ntiles * tile_vecs + i; j < nvec; j += stride) body(ld_stream(xv + j), j);
   // ragged tail (< one vector)
   if (blockIdx.x == 0) {
     const int64_t t = nvec * V::N + threadIdx.x;
@@ -736,7 +725,7 @@ static int launch_fwd(const void* x, void* y, void* codes, const dlmcq_layout* l
       const int64_t tiles = (n / Vec<T>::N + kThreads * kUnroll - 1) / (kThreads * kUnroll);
       // One contiguous 16 KB tile per CTA (grid-stride only beyond 148*1024 CTAs): measured 6.6-6.7 TB/s on
       // 2^26..2^28 elements vs 5.9-6.0 for a persistent grid-stride grid (profiles/README.md).
-      auto kern = fq_fwd_flat<FORM, T, kUnroll, 4, true>;
+      auto kern = fq_fwd_flat<FORM, T>;
       const int bps = 1024;
       const size_t bytes = static_cast<size_t>(n) * sizeof(T);
       FlatAccess acc;

@@ -13,8 +13,6 @@
 //
 // Rooflines: stats / l2norm are HBM-bound (4 B/elem fp32).  The sweeps are fp32-issue-bound once
 // staged (80 x ~20 instructions per element against 4 B of traffic).
-#include <cstdlib>
-
 #include "fq_math.cuh"
 
 namespace dlmcq {
@@ -1241,10 +1239,6 @@ extern "C" int dlmcq_obs_sweep_channel_plan(dlmcq_sweep_item* item, int64_t geom
   // warps-per-row choice fixes the summation order, so a row gets the same qparams whoever sweeps it
   const int64_t min_per_warp = geom_channels <= num_sms() ? 256 : 512;   // measured: profiles/README.md
   while (wpr < kSweepWarps && geom_channels * wpr < want_warps && inner >= min_per_warp * wpr) wpr *= 2;
-  if (const char* ov = getenv("DLMCQ_SWEEP_WPR")) {           // tuning aid (profiles/sweep_wpr_table.py)
-    const int v = atoi(ov);
-    if (v == 1 || v == 2 || v == 4 || v == 8) wpr = v;
-  }
   const int64_t row_floats = ((inner + 8 + 3) / 4) * 4;
   while (wpr < kSweepWarps && (kSweepWarps / wpr) * row_floats > kSweepSmemFloats) wpr *= 2;
   const int staged = (kSweepWarps / wpr) * row_floats <= kSweepSmemFloats ? 1 : 0;

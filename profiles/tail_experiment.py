@@ -1,7 +1,7 @@
 """Scratch experiment kept for the record: back-to-back launches on ROTATING buffers (so that no input is L2-resident)
 for the flat forward / backward kernels at several sizes - the source of the "rotating buffers" figures quoted in the
 round-1 kernel history.   python profiles/tail_experiment.py"""
-import ctypes as C, math, os, sys, torch
+import ctypes as C, math, sys, torch
 sys.path.insert(0, "/root/repo")
 from dlmc_quant_b200 import _lib, functional as F
 h=_lib.lib()
@@ -30,4 +30,4 @@ def run(n, nbuf=24, iters=240):
     return out
 for n in [int(a) for a in sys.argv[1:]] or (1605632, 3211264, 6422528, 12845056):
     f,b=run(n)
-    print(f"tune={os.environ.get('DLMCQ_FWD_TUNE','0')} n={n}: fwd {f:.2f} us ({8*n/f/1e3:.0f} GB/s)  bwd {b:.2f} us ({12*n/b/1e3:.0f} GB/s)")
+    print(f"n={n}: fwd {f:.2f} us ({8*n/f/1e3:.0f} GB/s)  bwd {b:.2f} us ({12*n/b/1e3:.0f} GB/s)")

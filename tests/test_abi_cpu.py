@@ -54,6 +54,20 @@ def test_workspace_query_needs_no_gpu(libpath):
     assert h.dlmcq_host_ctx_synchronize(None) == -1 and h.dlmcq_host_ctx_destroy(None) == 0
 
 
+def test_sweep_channel_plan_needs_no_gpu(libpath):
+    """The channel sweep's warps per row for the shapes the GPU tests use to reach 1, 2, 4 and 8 warps per row
+    (tests/test_gpu_rootq_obs.py), and the CTA count and shared memory that follow from it.  Without a device the SM
+    count is 148, a B200's."""
+    from dlmc_quant_b200 import _lib
+    h = _lib.lib()
+    for ch, inner, wpr in ((96, 100, 1), (96, 300, 2), (96, 700, 4), (96, 2304, 8),
+                           (6, 100, 1), (6, 300, 2), (6, 700, 4), (6, 1100, 8)):
+        it = _lib.SweepItem(channels=ch, inner=inner)
+        assert h.dlmcq_obs_sweep_channel_plan(ctypes.byref(it), ch) == 0
+        assert (it.wpr, it.staged) == (wpr, 1), (ch, inner)
+        assert it.ctas == (ch * wpr + 7) // 8 and it.smem_bytes == (8 // wpr) * it.row_floats * 4, (ch, inner)
+
+
 def test_argument_validation_without_gpu(libpath):
     """Bad arguments are rejected before any CUDA call is made."""
     from dlmc_quant_b200 import _lib

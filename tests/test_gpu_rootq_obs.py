@@ -721,30 +721,54 @@ def test_bf16_rootq_and_observers():
     assert doneb == donef and torch.allclose(sb, sf, rtol=1e-5)
 
 
+def _sweep_plan(rows2d):
+    """dlmcq_obs_sweep_channel_plan for a [channels, inner] matrix: the launch geometry sweep_channel gives it."""
+    import ctypes as C
+    from dlmc_quant_b200 import _lib
+    ch, inner = rows2d.shape
+    it = _lib.SweepItem(channels=ch, inner=inner)
+    _lib.check(_lib.lib().dlmcq_obs_sweep_channel_plan(C.byref(it), ch))
+    return it
+
+
+def _sweep_channel_with_wpr(rows2d, n_bits, signed, wpr):
+    """sweep_channel of one fp32 matrix through dlmcq_obs_sweep_channel_grouped, with `wpr` warps per row set by hand
+    instead of the plan's choice (8 warps per CTA: 8 / wpr rows per CTA, each staged in row_floats floats)."""
+    import ctypes as C
+    from dlmc_quant_b200 import _lib
+    ch = rows2d.shape[0]
+    out = torch.empty(2, ch, dtype=torch.float32, device=rows2d.device)
+    it = _sweep_plan(rows2d)
+    assert it.staged == 1
+    it.x, it.scale, it.offset = rows2d.data_ptr(), out[0].data_ptr(), out[1].data_ptr()
+    it.n_bits, it.is_signed, it.wpr = n_bits, int(signed), wpr
+    it.ctas = (ch * wpr + 7) // 8
+    it.smem_bytes = (8 // wpr) * it.row_floats * 4
+    tab = torch.frombuffer(bytearray(bytes(it)), dtype=torch.uint8).to(rows2d.device)
+    pre = torch.zeros(1, dtype=torch.int64, device=rows2d.device)
+    _lib.check(_lib.lib().dlmcq_obs_sweep_channel_grouped(C.c_void_p(tab.data_ptr()), C.c_void_p(pre.data_ptr()), 1,
+                                                          it.ctas, _lib.F32, it.smem_bytes, None))
+    torch.cuda.synchronize()
+    return out[0], out[1]
+
+
 def test_reductions_are_deterministic_run_to_run():
     """Every reduction on the path is fixed-order (no floating-point atomics): repeated launches on the same input
     return the same bits - also a race detector for the multi-warp channel sweep (shared-memory exchange + named
     barriers) under every warps-per-row setting."""
-    import os
     from dlmc_quant_b200 import functional as Fn
     gen = torch.Generator().manual_seed(71)
-    w = dev(torch.randn(96, 2304, generator=gen) * 0.02)
+    for inner, wpr in ((100, 1), (300, 2), (700, 4), (2304, 8)):     # the plan's warps per row for 96 rows of `inner`
+        w = dev(torch.randn(96, inner, generator=gen) * 0.02)
+        assert _sweep_plan(w).wpr == wpr, inner
+        first = Fn.sweep_channel(w, 4, True)
+        for _ in range(10):
+            again = Fn.sweep_channel(w, 4, True)
+            assert torch.equal(first[0], again[0]) and torch.equal(first[1], again[1]), wpr
     x = dev(torch.relu(torch.randn(1 << 22, generator=gen)) * 2)
     dy = dev(torch.randn(1 << 22, generator=gen))
     xa = dev(torch.relu(torch.randn(64, 48, 14, 14, generator=gen)))
     dya = dev(torch.randn(64, 48, 14, 14, generator=gen))
-    try:
-        for wpr in ("1", "2", "4", "8", None):
-            if wpr is None:
-                os.environ.pop("DLMCQ_SWEEP_WPR", None)
-            else:
-                os.environ["DLMCQ_SWEEP_WPR"] = wpr
-            first = Fn.sweep_channel(w, 4, True)
-            for _ in range(10):
-                again = Fn.sweep_channel(w, 4, True)
-                assert torch.equal(first[0], again[0]) and torch.equal(first[1], again[1]), wpr
-    finally:
-        os.environ.pop("DLMCQ_SWEEP_WPR", None)
     st = Fn.obs_stats(x)
     scale, off = Fn.minmax_from_stats(st, 4, False)
     ref = (Fn.fq_backward(x, dy, scale, off, 0, 15, 1, g=1e-3)[1], Fn.sweep_tensor_sse(x, st, 8), Fn.obs_stats(x),
@@ -761,34 +785,34 @@ def test_reductions_are_deterministic_run_to_run():
 def test_sweep_channel_edge_rows_under_every_geometry():
     """NaN rows, constant rows (zero scale: literal chain), all-zero rows, single-element rows and rows shorter than
     the number of lanes, with 1..8 warps per row (warps without elements must still take part in the exchange)."""
-    import os
     from dlmc_quant_b200 import functional as Fn
     gen = torch.Generator().manual_seed(81)
     cases = []
-    t = torch.rand(6, 700, generator=gen) * 3 + 0.5
-    t[1, 13] = float("nan")
-    t[2] = 1.75
-    t[3] = 0.0
-    t[4, ::2] = 0.0
-    cases.append(t)
-    cases.append(torch.rand(5, 1, generator=gen) + 0.1)
-    cases.append(torch.rand(3, 5, generator=gen) * 2)
-    cases.append((torch.randn(4, 33, generator=gen) * 0.02))
-    try:
-        for wpr in ("1", "2", "4", "8"):
-            os.environ["DLMCQ_SWEEP_WPR"] = wpr
-            for t in cases:
-                for signed in (False, True):
-                    s, o = Fn.sweep_channel(dev(t), 4, signed)
-                    rs, ro = R.obs_l2loss_channel(t.clone(), 4, signed)
-                    rs, ro = rs.reshape(-1), ro.reshape(-1).float()
-                    s, o = s.cpu(), o.cpu()
-                    nan_rows = torch.isnan(rs)
-                    assert torch.equal(torch.isnan(s), nan_rows) and torch.equal(torch.isnan(o), torch.isnan(ro)), (wpr, t.shape)
-                    ok = ~nan_rows
-                    _sweep_rows_equivalent(t[ok], s[ok], o[ok], rs[ok], ro[ok], 4)
-    finally:
-        os.environ.pop("DLMCQ_SWEEP_WPR", None)
+    for inner, wpr in ((100, 1), (300, 2), (700, 4), (1100, 8)):     # the plan's warps per row for 6 rows of `inner`
+        t = torch.rand(6, inner, generator=gen) * 3 + 0.5
+        t[1, 13] = float("nan")
+        t[2] = 1.75
+        t[3] = 0.0
+        t[4, ::2] = 0.0
+        assert _sweep_plan(t).wpr == wpr, inner
+        cases.append(t)
+    short = [torch.rand(5, 1, generator=gen) + 0.1, torch.rand(3, 5, generator=gen) * 2,
+             torch.randn(4, 33, generator=gen) * 0.02]
+    # the plan gives these short rows one warp each; more warps per row only through a hand-set geometry
+    runs = [(t, None) for t in cases + short] + [(t, wpr) for t in short for wpr in (2, 4, 8)]
+    for t, wpr in runs:
+        for signed in (False, True):
+            if wpr is None:
+                s, o = Fn.sweep_channel(dev(t), 4, signed)
+            else:
+                s, o = _sweep_channel_with_wpr(dev(t), 4, signed, wpr)
+            rs, ro = R.obs_l2loss_channel(t.clone(), 4, signed)
+            rs, ro = rs.reshape(-1), ro.reshape(-1).float()
+            s, o = s.cpu(), o.cpu()
+            nan_rows = torch.isnan(rs)
+            assert torch.equal(torch.isnan(s), nan_rows) and torch.equal(torch.isnan(o), torch.isnan(ro)), (wpr, t.shape)
+            ok = ~nan_rows
+            _sweep_rows_equivalent(t[ok], s[ok], o[ok], rs[ok], ro[ok], 4)
 
 
 def test_grouped_channel_sweep_is_bit_identical_to_per_tensor_sweeps():
