@@ -76,6 +76,12 @@ class BnqDesc(C.Structure):
 BNQ_TRAINING, BNQ_RELU, BNQ_RESIDUAL = 1, 2, 4
 
 
+class ConvGeom(C.Structure):
+    _fields_ = ([(n, C.c_int64) for n in ("batch", "h", "w", "cin", "n")] +
+                [(n, C.c_int32) for n in ("kh", "kw", "stride_h", "stride_w", "pad_h", "pad_w", "dil_h", "dil_w",
+                                          "groups")])
+
+
 class DlmcqError(RuntimeError):
     pass
 
@@ -152,6 +158,8 @@ SIGNATURES = {
     "dlmcq_codes_forward": (_I, [_P, _P, _LP, _QP, _I, _P]),
     "dlmcq_qgemm_prepare": (_I, [_P, _L, _L, _I, _QP, _QP, _L, _P, _P, _P, _P]),
     "dlmcq_qgemm": (_I, [_P, _P, _P, _P, _P, _L, _L, _L, _I, _I, _I, _I, _P]),
+    "dlmcq_qconv_prepare": (_I, [_P, C.POINTER(ConvGeom), _I, _QP, _QP, _L, _P, _P, _P, _P]),
+    "dlmcq_qconv": (_I, [_P, _P, _P, _P, _P, C.POINTER(ConvGeom), _I, _I, _I, _I, _P]),
 }
 
 

@@ -78,6 +78,18 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map
       ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1)
       : "memory");
 }
+// im2col mode: 128 consecutive output pixels (N*Ho*Wo order, wrapping rows and images inside the map's bounding box)
+// of one filter tap: {c0, w, h, img} is the window corner of the first pixel, {off_w, off_h} the tap's offset in input
+// pixels (s*dil_w, r*dil_h).  Pixels outside the image arrive as zero bytes.
+__device__ __forceinline__ void tma_load_im2col(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int w, int h,
+                                                int img, uint16_t off_w, uint16_t off_h) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.shared::cluster.global.im2col.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], "
+      "[%2], {%7, %8};"
+      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(w), "r"(h), "r"(img), "h"(off_w),
+        "h"(off_h)
+      : "memory");
+}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 // tcgen05.commit: the mbarrier receives one arrival when every tcgen05.mma this thread issued so far has completed
@@ -92,6 +104,11 @@ __device__ __forceinline__ void tc_commit(uint32_t bar) {
 __device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr) {
   return static_cast<uint64_t>((smem_addr & 0x3FFFFu) >> 4) | (1ull << 16) | (static_cast<uint64_t>(1024 >> 4) << 32) |
          (1ull << 46) | (2ull << 61);
+}
+// The same for 64-byte rows (SWIZZLE_64B, layout type 4): 8-row groups 512 bytes apart.
+__device__ __forceinline__ uint64_t umma_desc_sw64(uint32_t smem_addr) {
+  return static_cast<uint64_t>((smem_addr & 0x3FFFFu) >> 4) | (1ull << 16) | (static_cast<uint64_t>(512 >> 4) << 32) |
+         (1ull << 46) | (4ull << 61);
 }
 template <int KIND>
 __device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
@@ -141,9 +158,34 @@ __device__ __forceinline__ float acc_value(uint32_t v) {
   return IS_INT ? static_cast<float>(static_cast<int>(v)) : __uint_as_float(v);
 }
 
+// Implicit-GEMM geometry of a convolution (qconv_kernel): output row m of the [B*Ho*Wo, n] product is pixel
+// (m / HoWo, oh, ow) of a channels-last output; the A operand is the im2col view of the [B, H, W, Cin] codes.
+struct ConvArgs {
+  int H, W, Ho, Wo, HoWo, kh, kw, sh, sw, ph, pw, dh, dw, cchunks;   // cchunks = Cin / CHUNK
+};
+
+// Taps t in [0, k) with 0 <= top + t*d < size form one contiguous range [lo, hi1) (empty when lo >= hi1); both ends
+// lie in [0, k], so (lo, hi1) indexes a (k+1) x (k+1) table.
+__device__ __forceinline__ void tap_range(int top, int size, int d, int k, int& lo, int& hi1) {
+  lo = top >= 0 ? 0 : min(k, (d - 1 - top) / d);
+  const int last = size - 1 - top;
+  hi1 = last < 0 ? 0 : min(k, last / d + 1);
+}
+
+// Offset of output row m's beta vector in the border-class table [(kh+1)^2 (kw+1)^2][N] (dlmcq_qconv_prepare).
+__device__ __forceinline__ int conv_beta_offset(const ConvArgs& c, int m, int N) {
+  const int img = m / c.HoWo, pix = m - img * c.HoWo;
+  const int oh = pix / c.Wo, ow = pix - oh * c.Wo;
+  int rl, rh, sl, sh;
+  tap_range(oh * c.sh - c.ph, c.H, c.dh, c.kh, rl, rh);
+  tap_range(ow * c.sw - c.pw, c.W, c.dw, c.kw, sl, sh);
+  return (((rl * (c.kh + 1) + rh) * (c.kw + 1) + sl) * (c.kw + 1) + sh) * N;
+}
+
 // Per-column epilogue constants of one 32-column piece, fetched BEFORE the warp waits for the accumulator (their
 // latency hides behind the wait).  MODE 0: one column per lane; 1: four (fp32 line stores); 2: eight (bf16).
-template <int MODE>
+// BE = false (convolutions): beta depends on the row as well and is read per row from the border-class table.
+template <int MODE, bool BE = true>
 struct EpiConst {
   static constexpr int W = MODE == 0 ? 1 : (MODE == 1 ? 4 : 8);
   float al[W], be[W];
@@ -154,7 +196,7 @@ struct EpiConst {
     for (int e = 0; e < W; ++e) {
       const bool ok = col + e < N;
       al[e] = ok ? __ldg(alpha + col + e) : 0.f;
-      be[e] = ok ? __ldg(beta + col + e) : 0.f;
+      if (BE) be[e] = ok ? __ldg(beta + col + e) : 0.f;
     }
   }
 };
@@ -164,16 +206,20 @@ struct EpiConst {
 // stores are whole 128-byte lines.  MODE 0: scalar stores (any N, any alignment); 1: fp32, 16-byte stores
 // (N % 4 == 0); 2: bf16, 16-byte stores of 8 values (N % 8 == 0).  All smem reads are issued before the first
 // store; `floor` is 0 for a fused ReLU and -inf otherwise (max.NaN: NaN propagates, -0 -> +0, like torch.relu).
-template <bool IS_INT, int MODE>
+// CONV: beta is the row's border-class vector, beta + boff(row); each lane parks its row's offset in the transpose
+// buffer's padding column 32 so that every lane can read the offsets of the rows it stores.
+template <bool IS_INT, int MODE, bool CONV>
 __device__ __forceinline__ void epilogue_piece(const uint32_t (&v)[32], float* stg, int lane, int row0, int col0, int M,
-                                               int N, const EpiConst<MODE>& k, void* __restrict__ out, float floor,
-                                               int out_bf16) {
+                                               int N, const EpiConst<MODE, !CONV>& k, void* __restrict__ out, float floor,
+                                               int out_bf16, const float* __restrict__ beta, int boff) {
 #pragma unroll
   for (int j = 0; j < 8; ++j)
     *reinterpret_cast<float4*>(stg + lane * kStgPitch + 4 * j) =
         make_float4(acc_value<IS_INT>(v[4 * j]), acc_value<IS_INT>(v[4 * j + 1]), acc_value<IS_INT>(v[4 * j + 2]),
                     acc_value<IS_INT>(v[4 * j + 3]));
+  if (CONV) reinterpret_cast<int*>(stg)[lane * kStgPitch + 32] = boff;
   __syncwarp();
+  const int* const boffs = reinterpret_cast<const int*>(stg) + 32;   // row r's offset: boffs[r * kStgPitch]
   const int rows = M - row0;                                    // >= 1; the common case is a full piece (>= 32)
   if (MODE == 1) {
     const int rsub = lane >> 3, c4 = (lane & 7) * 4, col = col0 + c4;
@@ -187,12 +233,16 @@ __device__ __forceinline__ void epilogue_piece(const uint32_t (&v)[32], float* s
         for (int i = 0; i < 4; ++i) t[i] = *reinterpret_cast<const float4*>(stg + ((h * 4 + i) * 4 + rsub) * kStgPitch + c4);
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
+          const int r = (h * 4 + i) * 4 + rsub;
+          float4 be;
+          if (CONV) be = __ldg(reinterpret_cast<const float4*>(beta + boffs[r * kStgPitch] + col));
+          else be = make_float4(k.be[0], k.be[1], k.be[2], k.be[3]);
           float4 o;
-          o.x = max_nan(__fadd_rn(__fmul_rn(t[i].x, k.al[0]), k.be[0]), floor);
-          o.y = max_nan(__fadd_rn(__fmul_rn(t[i].y, k.al[1]), k.be[1]), floor);
-          o.z = max_nan(__fadd_rn(__fmul_rn(t[i].z, k.al[2]), k.be[2]), floor);
-          o.w = max_nan(__fadd_rn(__fmul_rn(t[i].w, k.al[3]), k.be[3]), floor);
-          if ((h * 4 + i) * 4 + rsub < rows) st_stream(reinterpret_cast<float4*>(p + (h * 4 + i) * step), o);
+          o.x = max_nan(__fadd_rn(__fmul_rn(t[i].x, k.al[0]), be.x), floor);
+          o.y = max_nan(__fadd_rn(__fmul_rn(t[i].y, k.al[1]), be.y), floor);
+          o.z = max_nan(__fadd_rn(__fmul_rn(t[i].z, k.al[2]), be.z), floor);
+          o.w = max_nan(__fadd_rn(__fmul_rn(t[i].w, k.al[3]), be.w), floor);
+          if (r < rows) st_stream(reinterpret_cast<float4*>(p + (h * 4 + i) * step), o);
         }
       }
     }
@@ -212,10 +262,20 @@ __device__ __forceinline__ void epilogue_piece(const uint32_t (&v)[32], float* s
         }
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
+          const int r = (h * 2 + i) * 8 + rsub;
           float o[8] = {t[i][0].x, t[i][0].y, t[i][0].z, t[i][0].w, t[i][1].x, t[i][1].y, t[i][1].z, t[i][1].w};
+          float be[8];
+          if (CONV) {
+            const float4* bp = reinterpret_cast<const float4*>(beta + boffs[r * kStgPitch] + col);
+            const float4 b0 = __ldg(bp), b1 = __ldg(bp + 1);
+            be[0] = b0.x; be[1] = b0.y; be[2] = b0.z; be[3] = b0.w; be[4] = b1.x; be[5] = b1.y; be[6] = b1.z; be[7] = b1.w;
+          } else {
 #pragma unroll
-          for (int e = 0; e < 8; ++e) o[e] = max_nan(__fadd_rn(__fmul_rn(o[e], k.al[e]), k.be[e]), floor);
-          if ((h * 2 + i) * 8 + rsub < rows) st_stream(reinterpret_cast<uint4*>(p + (h * 2 + i) * step), Vec<__nv_bfloat16>::pack(o));
+            for (int e = 0; e < 8; ++e) be[e] = k.be[e];
+          }
+#pragma unroll
+          for (int e = 0; e < 8; ++e) o[e] = max_nan(__fadd_rn(__fmul_rn(o[e], k.al[e]), be[e]), floor);
+          if (r < rows) st_stream(reinterpret_cast<uint4*>(p + (h * 2 + i) * step), Vec<__nv_bfloat16>::pack(o));
         }
       }
     }
@@ -225,7 +285,8 @@ __device__ __forceinline__ void epilogue_piece(const uint32_t (&v)[32], float* s
     if (col < N) {
       const int nr = rows < 32 ? rows : 32;
       for (int r = 0; r < nr; ++r) {
-        const float o = max_nan(__fadd_rn(__fmul_rn(stg[r * kStgPitch + lane], k.al[0]), k.be[0]), floor);
+        const float be = CONV ? __ldg(beta + boffs[r * kStgPitch] + col) : k.be[0];
+        const float o = max_nan(__fadd_rn(__fmul_rn(stg[r * kStgPitch + lane], k.al[0]), be), floor);
         const size_t idx = static_cast<size_t>(row0 + r) * static_cast<size_t>(N) + static_cast<size_t>(col);
         if (out_bf16) static_cast<__nv_bfloat16*>(out)[idx] = __float2bfloat16_rn(o);
         else static_cast<float*>(out)[idx] = o;
@@ -241,11 +302,11 @@ __device__ __forceinline__ void epilogue_piece(const uint32_t (&v)[32], float* s
 // profiles/r02_qgemm_timeline_probe.log).  Inside a group a warp owns TMEM lane quarter q and 64 columns (two
 // 32-column pieces, read one at a time: 32 live accumulator registers).  The buffer is handed back to the MMA thread
 // by ONE arrival per warp, right after the warp's last TMEM read.
-template <bool IS_INT, int MODE>
+template <bool IS_INT, int MODE, bool CONV>
 __device__ __forceinline__ void epilogue_loop(uint32_t tmem, uint32_t bar_acc_full, uint32_t bar_acc_empty, float* stg,
                                               int lane, int q, int grp, int chalf, int num_tiles, int tiles_n, int M,
                                               int N, const float* __restrict__ alpha, const float* __restrict__ beta,
-                                              void* __restrict__ out, float floor, int out_bf16) {
+                                              void* __restrict__ out, float floor, int out_bf16, const ConvArgs& cv) {
   const uint32_t full = bar_acc_full + 8 * grp, empty = bar_acc_empty + 8 * grp;
   const uint32_t tbase = tmem + grp * kBN + (static_cast<uint32_t>(q * 32) << 16) + static_cast<uint32_t>(chalf * 64);
   uint32_t ti = grp;
@@ -253,8 +314,9 @@ __device__ __forceinline__ void epilogue_loop(uint32_t tmem, uint32_t bar_acc_fu
     const int m0 = (tile / tiles_n) * kBM, n0 = (tile % tiles_n) * kBN;
     const int col0 = n0 + chalf * 64, row0 = m0 + q * 32;
     const bool has0 = col0 < N, has1 = col0 + 32 < N;            // warp-uniform
-    EpiConst<MODE> k0;
+    EpiConst<MODE, !CONV> k0;
     k0.load(alpha, beta, col0, lane, N);
+    const int boff = CONV ? conv_beta_offset(cv, row0 + lane, N) : 0;   // this lane's row (the table covers rows >= M too)
     mbar_wait(full, (ti >> 1) & 1);
     tc_fence_after();
     uint32_t v[32];
@@ -264,24 +326,32 @@ __device__ __forceinline__ void epilogue_loop(uint32_t tmem, uint32_t bar_acc_fu
       __syncwarp();
       if (lane == 0) mbar_arrive(empty);
     }
-    if (has0 && row0 < M) epilogue_piece<IS_INT, MODE>(v, stg, lane, row0, col0, M, N, k0, out, floor, out_bf16);
+    if (has0 && row0 < M)
+      epilogue_piece<IS_INT, MODE, CONV>(v, stg, lane, row0, col0, M, N, k0, out, floor, out_bf16, beta, boff);
     if (has1) {
-      EpiConst<MODE> k1;                                        // L1-resident by now; fetched here to keep registers free
+      EpiConst<MODE, !CONV> k1;                                 // L1-resident by now; fetched here to keep registers free
       k1.load(alpha, beta, col0 + 32, lane, N);
       tmem_ld32(tbase + 32, v);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(empty);
-      if (row0 < M) epilogue_piece<IS_INT, MODE>(v, stg, lane, row0, col0 + 32, M, N, k1, out, floor, out_bf16);
+      if (row0 < M)
+        epilogue_piece<IS_INT, MODE, CONV>(v, stg, lane, row0, col0 + 32, M, N, k1, out, floor, out_bf16, beta, boff);
     }
   }
 }
 
-template <int KIND>
-__global__ void __launch_bounds__(kGemmThreads, 1)   // 576 threads: ptxas caps the kernel at 96 registers
-qgemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
-             const float* __restrict__ alpha, const float* __restrict__ beta, void* __restrict__ out, int M, int N,
-             int K, uint32_t idesc, int relu, int out_bf16, int vec_ok) {
+// The kernel body, shared by the GEMM (CHUNK = 0: A is a [M, K] matrix, 128-byte K blocks) and the implicit-GEMM
+// convolution (CHUNK = 128 / 64: A is the im2col view of channels-last codes; one K block = one filter tap x CHUNK
+// channels, K = kh*kw*Cin in (r, s, c) order, so B is the [n, K] matrix of channels-last weight codes and a K block
+// never straddles a tap).  Only the A producer, the K-block width and the epilogue's beta differ.
+template <int KIND, int CHUNK>
+__device__ __forceinline__ void gemm_pipeline(const CUtensorMap* map_a, const CUtensorMap* map_b,
+                                              const float* __restrict__ alpha, const float* __restrict__ beta,
+                                              void* __restrict__ out, int M, int N, int K, uint32_t idesc, int relu,
+                                              int out_bf16, int vec_ok, const ConvArgs& cv) {
+  constexpr int kKb = CHUNK == 0 ? kBK : CHUNK;                 // K bytes per block
+  constexpr uint32_t kTx = CHUNK == 0 ? kStageBytes : 2 * kBM * CHUNK;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;                 // the swizzle atoms need 1024-byte alignment
@@ -295,7 +365,7 @@ qgemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int tiles_n = (N + kBN - 1) / kBN, tiles_m = (M + kBM - 1) / kBM;
   const int num_tiles = tiles_m * tiles_n;
-  const int num_kb = (K + kBK - 1) / kBK;
+  const int num_kb = (K + kKb - 1) / kKb;
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < kStages; ++s) {
@@ -326,13 +396,31 @@ qgemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
       uint32_t it = 0;
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
         const int m0 = (tile / tiles_n) * kBM, n0 = (tile % tiles_n) * kBN;
-        for (int kb = 0; kb < num_kb; ++kb, ++it) {
-          const uint32_t s = it % kStages, ph = (it / kStages) & 1;
-          mbar_wait(bar_empty + 8 * s, ph ^ 1);                 // slot free (passes at once in the first round)
-          mbar_expect_tx(bar_full + 8 * s, kStageBytes);        // a box always delivers its full byte count (OOB = 0)
-          const uint32_t dst = base + s * kStageBytes;
-          tma_load_2d(dst, &map_a, bar_full + 8 * s, kb * kBK, m0);
-          tma_load_2d(dst + kABytes, &map_b, bar_full + 8 * s, kb * kBK, n0);
+        if constexpr (CHUNK == 0) {
+          for (int kb = 0; kb < num_kb; ++kb, ++it) {
+            const uint32_t s = it % kStages, ph = (it / kStages) & 1;
+            mbar_wait(bar_empty + 8 * s, ph ^ 1);               // slot free (passes at once in the first round)
+            mbar_expect_tx(bar_full + 8 * s, kTx);              // a box always delivers its full byte count (OOB = 0)
+            const uint32_t dst = base + s * kStageBytes;
+            tma_load_2d(dst, map_a, bar_full + 8 * s, kb * kBK, m0);
+            tma_load_2d(dst + kABytes, map_b, bar_full + 8 * s, kb * kBK, n0);
+          }
+        } else {
+          // window corner of the tile's first output pixel; the im2col box walks the next 127 by itself
+          const int img = m0 / cv.HoWo, pix = m0 - img * cv.HoWo, oh = pix / cv.Wo, ow = pix - oh * cv.Wo;
+          const int hb = oh * cv.sh - cv.ph, wb = ow * cv.sw - cv.pw;
+          int kb = 0;
+          for (int r = 0; r < cv.kh; ++r)
+            for (int t = 0; t < cv.kw; ++t)
+              for (int cc = 0; cc < cv.cchunks; ++cc, ++kb, ++it) {
+                const uint32_t s = it % kStages, ph = (it / kStages) & 1;
+                mbar_wait(bar_empty + 8 * s, ph ^ 1);
+                mbar_expect_tx(bar_full + 8 * s, kTx);
+                const uint32_t dst = base + s * kStageBytes;
+                tma_load_im2col(dst, map_a, bar_full + 8 * s, cc * CHUNK, wb, hb, img, static_cast<uint16_t>(t * cv.dw),
+                                static_cast<uint16_t>(r * cv.dh));
+                tma_load_2d(dst + kABytes, map_b, bar_full + 8 * s, kb * CHUNK, n0);
+              }
         }
       }
     }
@@ -350,10 +438,19 @@ qgemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
           mbar_wait(bar_full + 8 * s, ph);
           tc_fence_after();
           const uint32_t a = base + s * kStageBytes, b = a + kABytes;
-          const int left = K - kb * kBK;                        // bytes of K beyond this block are zero-filled: skip them
-          const int steps = left >= kBK ? kBK / kUmmaK : (left + kUmmaK - 1) / kUmmaK;
-          for (int k = 0; k < steps; ++k)
-            umma<KIND>(d, umma_desc(a + k * kUmmaK), umma_desc(b + k * kUmmaK), idesc, (kb | k) != 0 ? 1u : 0u);
+          if constexpr (CHUNK == 0) {
+            const int left = K - kb * kBK;                      // bytes of K beyond this block are zero-filled: skip them
+            const int steps = left >= kBK ? kBK / kUmmaK : (left + kUmmaK - 1) / kUmmaK;
+            for (int k = 0; k < steps; ++k)
+              umma<KIND>(d, umma_desc(a + k * kUmmaK), umma_desc(b + k * kUmmaK), idesc, (kb | k) != 0 ? 1u : 0u);
+          } else {                                              // a tap's channel chunk: never a K tail
+#pragma unroll
+            for (int k = 0; k < CHUNK / kUmmaK; ++k) {
+              const uint64_t da = CHUNK == 128 ? umma_desc(a + k * kUmmaK) : umma_desc_sw64(a + k * kUmmaK);
+              const uint64_t db = CHUNK == 128 ? umma_desc(b + k * kUmmaK) : umma_desc_sw64(b + k * kUmmaK);
+              umma<KIND>(d, da, db, idesc, (kb | k) != 0 ? 1u : 0u);
+            }
+          }
           tc_commit(bar_empty + 8 * s);                         // the slot returns to the producer when these complete
         }
         tc_commit(bar_acc_full + 8 * ab);                       // ... and this tile's accumulators are final
@@ -369,14 +466,14 @@ qgemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
     float* const stg = stg_all + ew * (32 * kStgPitch);
     const float floor = relu ? 0.f : __int_as_float(0xff800000);
     if (vec_ok && !out_bf16)
-      epilogue_loop<IS_INT, 1>(tmem, bar_acc_full, bar_acc_empty, stg, lane, q, grp, chalf, num_tiles, tiles_n, M, N,
-                               alpha, beta, out, floor, out_bf16);
+      epilogue_loop<IS_INT, 1, CHUNK != 0>(tmem, bar_acc_full, bar_acc_empty, stg, lane, q, grp, chalf, num_tiles, tiles_n, M, N,
+                               alpha, beta, out, floor, out_bf16, cv);
     else if (vec_ok)
-      epilogue_loop<IS_INT, 2>(tmem, bar_acc_full, bar_acc_empty, stg, lane, q, grp, chalf, num_tiles, tiles_n, M, N,
-                               alpha, beta, out, floor, out_bf16);
+      epilogue_loop<IS_INT, 2, CHUNK != 0>(tmem, bar_acc_full, bar_acc_empty, stg, lane, q, grp, chalf, num_tiles, tiles_n, M, N,
+                               alpha, beta, out, floor, out_bf16, cv);
     else
-      epilogue_loop<IS_INT, 0>(tmem, bar_acc_full, bar_acc_empty, stg, lane, q, grp, chalf, num_tiles, tiles_n, M, N,
-                               alpha, beta, out, floor, out_bf16);
+      epilogue_loop<IS_INT, 0, CHUNK != 0>(tmem, bar_acc_full, bar_acc_empty, stg, lane, q, grp, chalf, num_tiles, tiles_n, M, N,
+                               alpha, beta, out, floor, out_bf16, cv);
   }
   tc_fence_before();
   __syncthreads();
@@ -386,6 +483,24 @@ qgemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
                  "r"(static_cast<uint32_t>(kTmemCols))
                  : "memory");
   }
+}
+
+template <int KIND>
+__global__ void __launch_bounds__(kGemmThreads, 1)   // 576 threads: ptxas caps the kernel at 96 registers
+qgemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
+             const float* __restrict__ alpha, const float* __restrict__ beta, void* __restrict__ out, int M, int N,
+             int K, uint32_t idesc, int relu, int out_bf16, int vec_ok) {
+  gemm_pipeline<KIND, 0>(&map_a, &map_b, alpha, beta, out, M, N, K, idesc, relu, out_bf16, vec_ok, ConvArgs{});
+}
+
+// Implicit-GEMM convolution: map_a is an im2col map of the [B, H, W, Cin] codes, map_b the [n, kh*kw*Cin] weight
+// codes; beta is the border-class table; out [B*Ho*Wo, n] (channels-last).
+template <int KIND, int CHUNK>
+__global__ void __launch_bounds__(kGemmThreads, 1)
+qconv_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
+             const float* __restrict__ alpha, const float* __restrict__ beta, void* __restrict__ out, int M, int N,
+             int K, uint32_t idesc, int relu, int out_bf16, int vec_ok, const ConvArgs cv) {
+  gemm_pipeline<KIND, CHUNK>(&map_a, &map_b, alpha, beta, out, M, N, K, idesc, relu, out_bf16, vec_ok, cv);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -543,6 +658,51 @@ qgemm_prepare_kernel(const uint8_t* __restrict__ w_codes, int64_t n, int64_t k, 
   }
 }
 
+// Convolution: alpha[n] as above; beta for every border class of output pixel.  One block per output channel: the
+// per-tap code sums S[r][s] = sum_c cw[n, r, s, c] go to smem, then every class (r_lo, r_hi1, s_lo, s_hi1) - the
+// taps of the window that lie inside the image, each range in [0, k] - gets
+//     beta[class][n] = RN(RN(t * m_w[n]) * float(sum_{r_lo <= r < r_hi1, s_lo <= s < s_hi1} S[r][s]))  (+ bias[n])
+// class = ((r_lo*(kh+1) + r_hi1)*(kw+1) + s_lo)*(kw+1) + s_hi1: the epilogue's conv_beta_offset.
+constexpr int kConvPrepThreads = 128;
+
+__global__ void __launch_bounds__(kConvPrepThreads)
+qconv_prepare_kernel(const uint8_t* __restrict__ w_codes, int64_t n, int cin, int kh, int kw, int encoding, int act_form,
+                     const float* __restrict__ act_scale, const float* __restrict__ act_offset, float act_g,
+                     float act_lo, float act_hi, int wt_form, const float* __restrict__ wt_scale, float wt_g,
+                     float wt_lo, float wt_hi, int64_t wt_channels, const float* __restrict__ bias,
+                     float* __restrict__ alpha, float* __restrict__ beta) {
+  extern __shared__ int tap_sum[];
+  const int64_t row = blockIdx.x;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, taps = kh * kw;
+  const uint8_t* wr = w_codes + row * static_cast<int64_t>(taps) * cin;
+  for (int tap = warp; tap < taps; tap += kConvPrepThreads / 32) {
+    int sum = 0;
+    for (int c = lane; c < cin; c += 32) sum += decode_code(wr[static_cast<int64_t>(tap) * cin + c], encoding, wt_lo < 0.f);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+    if (lane == 0) tap_sum[tap] = sum;
+  }
+  __syncthreads();
+  const ChanParams pa = params_of(act_form, act_scale, act_offset, 0, act_g, act_lo, act_hi);
+  const ChanParams pw = params_of(wt_form, wt_scale, nullptr, wt_channels == 1 ? 0 : row, wt_g, wt_lo, wt_hi);
+  const float z_a = act_form == DLMCQ_FORM_ZP ? pa.off : 0.f;
+  const float o_a = (act_form == DLMCQ_FORM_A1 || act_form == DLMCQ_FORM_AFFINE) ? pa.off : 0.f;
+  const float tm = __fmul_rn(__fsub_rn(o_a, __fmul_rn(z_a, pa.mul)), pw.mul);
+  const float bn = bias ? __ldg(bias + row) : 0.f;
+  if (threadIdx.x == 0) alpha[row] = __fmul_rn(pa.mul, pw.mul);
+  const int classes = (kh + 1) * (kh + 1) * (kw + 1) * (kw + 1);
+  for (int cls = threadIdx.x; cls < classes; cls += kConvPrepThreads) {
+    const int sh1 = cls % (kw + 1), sl = (cls / (kw + 1)) % (kw + 1);
+    const int rh1 = (cls / ((kw + 1) * (kw + 1))) % (kh + 1), rl = cls / ((kw + 1) * (kw + 1) * (kh + 1));
+    int sum = 0;
+    for (int r = rl; r < rh1; ++r)
+      for (int t = sl; t < sh1; ++t) sum += tap_sum[r * kw + t];
+    float b = __fmul_rn(tm, static_cast<float>(sum));
+    if (bias) b = __fadd_rn(b, bn);
+    beta[static_cast<int64_t>(cls) * n + row] = b;
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // host side: tensor maps
 // ---------------------------------------------------------------------------------------------------------------
@@ -562,16 +722,53 @@ EncodeTiledFn encode_tiled() {
   return fn;
 }
 
-// [rows, k] bytes, row-major (K-major): box = 128 bytes of K x 128 rows, 128-byte swizzle, out-of-bounds = 0
-bool make_map(CUtensorMap* m, const void* ptr, int64_t rows, int64_t k, int box_rows) {
+// [rows, k] bytes, row-major (K-major): box = box_k (128 or 64) bytes of K x 128 rows, swizzle of the same width,
+// out-of-bounds = 0
+bool make_map(CUtensorMap* m, const void* ptr, int64_t rows, int64_t k, int box_rows, int box_k = kBK) {
   EncodeTiledFn enc = encode_tiled();
   if (!enc) return false;
   const cuuint64_t dims[2] = {static_cast<cuuint64_t>(k), static_cast<cuuint64_t>(rows)};
   const cuuint64_t strides[1] = {static_cast<cuuint64_t>(k)};
-  const cuuint32_t box[2] = {static_cast<cuuint32_t>(kBK), static_cast<cuuint32_t>(box_rows)};
+  const cuuint32_t box[2] = {static_cast<cuuint32_t>(box_k), static_cast<cuuint32_t>(box_rows)};
   const cuuint32_t estr[2] = {1, 1};
   return enc(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+             CU_TENSOR_MAP_INTERLEAVE_NONE, box_k == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
+             CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
+typedef CUresult (*EncodeIm2colFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                   const cuuint64_t*, const int*, const int*, cuuint32_t, cuuint32_t, const cuuint32_t*,
+                                   CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
+                                   CUtensorMapFloatOOBfill);
+
+EncodeIm2colFn encode_im2col() {
+  static const EncodeIm2colFn fn = [] {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &p, cudaEnableDefault, &q) != cudaSuccess ||
+        q != cudaDriverEntryPointSuccess)
+      p = nullptr;
+    return reinterpret_cast<EncodeIm2colFn>(p);
+  }();
+  return fn;
+}
+
+// Channels-last codes [B, H, W, Cin] as an im2col map: 128 pixels x `chunk` channels per box.  The bounding box of
+// window corners is [-pad, size - 1 + pad - dil*(k-1)] per spatial axis, walked with the convolution's stride, so the
+// box's pixels are exactly the output pixels in N*Ho*Wo order.  Arrays are innermost first (C, W, H, N).
+bool make_im2col_map(CUtensorMap* m, const void* ptr, const dlmcq_conv_geom* g, int chunk) {
+  EncodeIm2colFn enc = encode_im2col();
+  if (!enc) return false;
+  const cuuint64_t dims[4] = {static_cast<cuuint64_t>(g->cin), static_cast<cuuint64_t>(g->w),
+                              static_cast<cuuint64_t>(g->h), static_cast<cuuint64_t>(g->batch)};
+  const cuuint64_t strides[3] = {static_cast<cuuint64_t>(g->cin), static_cast<cuuint64_t>(g->cin * g->w),
+                                 static_cast<cuuint64_t>(g->cin * g->w * g->h)};
+  const int lower[2] = {-g->pad_w, -g->pad_h};
+  const int upper[2] = {g->pad_w - g->dil_w * (g->kw - 1), g->pad_h - g->dil_h * (g->kh - 1)};
+  const cuuint32_t estr[4] = {1, static_cast<cuuint32_t>(g->stride_w), static_cast<cuuint32_t>(g->stride_h), 1};
+  return enc(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, const_cast<void*>(ptr), dims, strides, lower, upper,
+             static_cast<cuuint32_t>(chunk), static_cast<cuuint32_t>(kBM), estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+             chunk == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
@@ -611,6 +808,58 @@ int gemm_launch(const CUtensorMap& ma, const CUtensorMap& mb, const float* alpha
   qgemm_kernel<KIND><<<grid, kGemmThreads, kGemmSmem, st>>>(ma, mb, alpha, beta, out, m, n, k,
                                                             make_idesc(KIND, a_signed), relu, out_bf16, vec_ok);
   DLMCQ_LAUNCH_CHECK();
+  return DLMCQ_OK;
+}
+
+template <int KIND, int CHUNK>
+int conv_launch(const CUtensorMap& ma, const CUtensorMap& mb, const float* alpha, const float* beta, void* out, int m,
+                int n, int k, const ConvArgs& cv, int a_signed, int relu, int out_bf16, cudaStream_t st) {
+  static bool opted_in[64] = {};
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) dev = 0;
+  if (dev < 0 || dev >= 64 || !opted_in[dev]) {
+    const cudaError_t e = cudaFuncSetAttribute(qconv_kernel<KIND, CHUNK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               static_cast<int>(kGemmSmem));
+    if (e != cudaSuccess) return set_cuda_error(e);
+    if (dev >= 0 && dev < 64) opted_in[dev] = true;
+  }
+  const int64_t tiles = static_cast<int64_t>((n + kBN - 1) / kBN) * ((m + kBM - 1) / kBM);
+  const int sms = num_sms();
+  const unsigned grid = static_cast<unsigned>(tiles < sms ? tiles : sms);
+  // the beta table is read with 16-byte loads in the vector epilogues: its rows start at multiples of n
+  const int vec_ok = aligned16(out) && aligned16(beta) && (n % (out_bf16 ? 8 : 4) == 0);
+  qconv_kernel<KIND, CHUNK><<<grid, kGemmThreads, kGemmSmem, st>>>(ma, mb, alpha, beta, out, m, n, k,
+                                                                   make_idesc(KIND, a_signed), relu, out_bf16, vec_ok, cv);
+  DLMCQ_LAUNCH_CHECK();
+  return DLMCQ_OK;
+}
+
+// Geometry checks shared by dlmcq_qconv_prepare (full = 0: only the filter and channel counts) and dlmcq_qconv.
+int conv_check(const dlmcq_conv_geom* g, int full, int64_t* ho, int64_t* wo) {
+  if (!g || g->cin < 1 || g->n < 1 || g->kh < 1 || g->kw < 1 || g->groups < 1) return DLMCQ_EINVAL;
+  if (g->groups != 1 || g->cin % 64 != 0) return DLMCQ_EUNSUPPORTED;
+  const int64_t k = static_cast<int64_t>(g->kh) * g->kw * g->cin;
+  const int64_t classes = static_cast<int64_t>(g->kh + 1) * (g->kh + 1) * (g->kw + 1) * (g->kw + 1);
+  if (g->kh > 255 || g->kw > 255 || k > 0x7fffff00LL || g->n > 0x7fffff00LL || classes * g->n > 0x7fffffffLL)
+    return DLMCQ_EUNSUPPORTED;
+  if (!full) return DLMCQ_OK;
+  if (g->batch < 1 || g->h < 1 || g->w < 1 || g->stride_h < 1 || g->stride_w < 1 || g->pad_h < 0 || g->pad_w < 0 ||
+      g->dil_h < 1 || g->dil_w < 1)
+    return DLMCQ_EINVAL;
+  const int64_t eh = static_cast<int64_t>(g->dil_h) * (g->kh - 1), ew = static_cast<int64_t>(g->dil_w) * (g->kw - 1);
+  if (g->h + 2LL * g->pad_h - eh < 1 || g->w + 2LL * g->pad_w - ew < 1) return DLMCQ_EINVAL;   // no output pixel
+  *ho = (g->h + 2LL * g->pad_h - eh - 1) / g->stride_h + 1;
+  *wo = (g->w + 2LL * g->pad_w - ew - 1) / g->stride_w + 1;
+  // TMA im2col limits: traversal stride <= 8, bounding-box corners -pad and pad - dil*(k-1) in [-128, 127]
+  if (g->stride_h > 8 || g->stride_w > 8 || g->pad_h > 128 || g->pad_w > 128 || g->pad_h - eh < -128 ||
+      g->pad_w - ew < -128 || g->pad_h - eh > 127 || g->pad_w - ew > 127)
+    return DLMCQ_EUNSUPPORTED;
+  // 32-bit coordinates and row indices
+  const int64_t m = g->batch * *ho * *wo;
+  if (g->batch > 0x7fffffffLL || g->h > 0x7fffffffLL || g->w > 0x7fffffffLL || m > 0x7fffff00LL ||
+      g->h * g->w > (1LL << 40) / g->cin)                         // TMA strides < 2^40 bytes
+    return DLMCQ_EUNSUPPORTED;
+  if (((m + kBM - 1) / kBM) * ((g->n + kBN - 1) / kBN) > 0x7fffffffLL) return DLMCQ_EUNSUPPORTED;
   return DLMCQ_OK;
 }
 
@@ -676,4 +925,58 @@ extern "C" int dlmcq_qgemm(const void* a_codes, const void* w_codes, const float
                                            static_cast<int>(k), a_signed, relu, bf, st)
              : gemm_launch<DLMCQ_QGEMM_E4M3>(ma, mb, alpha, beta, out, static_cast<int>(m), static_cast<int>(n),
                                              static_cast<int>(k), a_signed, relu, bf, st);
+}
+
+extern "C" int dlmcq_qconv_prepare(const void* w_codes, const dlmcq_conv_geom* geom, int encoding,
+                                   const dlmcq_qparams* act_qp, const dlmcq_qparams* wt_qp, int64_t wt_channels,
+                                   const float* bias, float* alpha, float* beta, void* stream) {
+  if (!w_codes || !act_qp || !wt_qp || !act_qp->scale || !wt_qp->scale || !alpha || !beta) return DLMCQ_EINVAL;
+  int64_t ho = 0, wo = 0;
+  if (int e = conv_check(geom, 0, &ho, &wo)) return e;
+  const int64_t n = geom->n;
+  if (wt_channels != 1 && wt_channels != n) return DLMCQ_EINVAL;
+  if (int e = code_range_ok(act_qp, encoding)) return e;
+  if (int e = code_range_ok(wt_qp, encoding)) return e;
+  if (wt_qp->form == DLMCQ_FORM_ZP || wt_qp->offset != nullptr) return DLMCQ_EUNSUPPORTED;
+  if (encoding == DLMCQ_QGEMM_I8 && wt_qp->lo >= 0 && wt_qp->hi > 127) return DLMCQ_EUNSUPPORTED;
+  const size_t smem = static_cast<size_t>(geom->kh) * geom->kw * sizeof(int);
+  if (smem > 48 * 1024) return DLMCQ_EUNSUPPORTED;
+  qconv_prepare_kernel<<<static_cast<unsigned>(n), kConvPrepThreads, smem, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const uint8_t*>(w_codes), n, static_cast<int>(geom->cin), geom->kh, geom->kw, encoding, act_qp->form,
+      act_qp->scale, act_qp->offset, act_qp->g, static_cast<float>(act_qp->lo), static_cast<float>(act_qp->hi),
+      wt_qp->form, wt_qp->scale, wt_qp->g, static_cast<float>(wt_qp->lo), static_cast<float>(wt_qp->hi), wt_channels,
+      bias, alpha, beta);
+  DLMCQ_LAUNCH_CHECK();
+  return DLMCQ_OK;
+}
+
+extern "C" int dlmcq_qconv(const void* a_codes, const void* w_codes, const float* alpha, const float* beta, void* out,
+                           const dlmcq_conv_geom* geom, int encoding, int a_signed, int relu, int out_dtype,
+                           void* stream) {
+  if (!alpha || !beta) return DLMCQ_EINVAL;
+  if (encoding != DLMCQ_QGEMM_I8 && encoding != DLMCQ_QGEMM_E4M3) return DLMCQ_EINVAL;
+  if (out_dtype != DLMCQ_F32 && out_dtype != DLMCQ_BF16) return DLMCQ_EINVAL;
+  int64_t ho = 0, wo = 0;
+  if (int e = conv_check(geom, 1, &ho, &wo)) return e;
+  if (!a_codes || !w_codes || !out) return DLMCQ_EINVAL;
+  if (!aligned16(a_codes) || !aligned16(w_codes)) return DLMCQ_EALIGN;
+  const int chunk = geom->cin % 128 == 0 ? 128 : 64;
+  CUtensorMap ma, mb;
+  const int64_t k = static_cast<int64_t>(geom->kh) * geom->kw * geom->cin;
+  if (!make_im2col_map(&ma, a_codes, geom, chunk) || !make_map(&mb, w_codes, geom->n, k, kBN, chunk))
+    return DLMCQ_EUNSUPPORTED;
+  ConvArgs cv;
+  cv.H = static_cast<int>(geom->h); cv.W = static_cast<int>(geom->w);
+  cv.Ho = static_cast<int>(ho); cv.Wo = static_cast<int>(wo); cv.HoWo = static_cast<int>(ho * wo);
+  cv.kh = geom->kh; cv.kw = geom->kw; cv.sh = geom->stride_h; cv.sw = geom->stride_w;
+  cv.ph = geom->pad_h; cv.pw = geom->pad_w; cv.dh = geom->dil_h; cv.dw = geom->dil_w;
+  cv.cchunks = static_cast<int>(geom->cin / chunk);
+  const int m = static_cast<int>(geom->batch * ho * wo), n = static_cast<int>(geom->n);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int bf = out_dtype == DLMCQ_BF16;
+  if (encoding == DLMCQ_QGEMM_I8)
+    return chunk == 128 ? conv_launch<DLMCQ_QGEMM_I8, 128>(ma, mb, alpha, beta, out, m, n, static_cast<int>(k), cv, a_signed, relu, bf, st)
+                        : conv_launch<DLMCQ_QGEMM_I8, 64>(ma, mb, alpha, beta, out, m, n, static_cast<int>(k), cv, a_signed, relu, bf, st);
+  return chunk == 128 ? conv_launch<DLMCQ_QGEMM_E4M3, 128>(ma, mb, alpha, beta, out, m, n, static_cast<int>(k), cv, a_signed, relu, bf, st)
+                      : conv_launch<DLMCQ_QGEMM_E4M3, 64>(ma, mb, alpha, beta, out, m, n, static_cast<int>(k), cv, a_signed, relu, bf, st);
 }

@@ -8,9 +8,11 @@ per-output-channel affine map (include/dlmcq.h, `dlmcq_qgemm`).  The integer pro
 (csrc/qgemm_kernels.cu); the activation is read at one byte per element instead of four.
 
 Two levels:
-  * functional: `codes_forward`, `qgemm_prepare`, `qgemm` - thin wrappers over the C ABI;
+  * functional: `codes_forward`, `qgemm_prepare`, `qgemm`, and for k x k / strided / padded convolutions
+    `qconv_prepare`, `qconv` (implicit GEMM over channels-last codes) - thin wrappers over the C ABI;
   * module: `enable_code_gemm(model)` switches every eligible quantised `nn.Linear` / 1x1 `nn.Conv2d` of a model to
-    the code path for inference (`module.eval()`, no autograd); training / calibration / ineligible layers keep the
+    the code path for inference (`module.eval()`, no autograd), `enable_code_gemm(model, convolutions=True)` also the
+    other quantised `nn.Conv2d` layers `qconv` serves; training / calibration / ineligible layers keep the
     reference's path (fake-quant kernels + the library convolution).  Opt-in: results equal the fake-quant path up
     to the rounding of the fp32 product (the integer accumulation itself is exact; cuDNN's TF32 / fp32 sums are not).
 """
@@ -23,9 +25,10 @@ from torch import nn
 
 from . import _lib
 from . import functional as F
-from ._lib import BF16, F32, FORM_AFFINE, FORM_SYM, FORM_ZP, QGEMM_E4M3, QGEMM_I8, DlmcqError, QParams
+from ._lib import BF16, F32, FORM_AFFINE, FORM_SYM, FORM_ZP, QGEMM_E4M3, QGEMM_I8, ConvGeom, DlmcqError, QParams
 
-__all__ = ["codes_forward", "qgemm_prepare", "qgemm", "enable_code_gemm", "disable_code_gemm", "QGEMM_I8", "QGEMM_E4M3"]
+__all__ = ["codes_forward", "qgemm_prepare", "qgemm", "qconv_prepare", "qconv", "enable_code_gemm", "disable_code_gemm",
+           "QGEMM_I8", "QGEMM_E4M3"]
 
 
 def _qp(form, lo, hi, g, scale, offset):
@@ -48,14 +51,7 @@ def codes_forward(x, scale, offset, lo, hi, form, g=0.0, ch_axis=None, encoding=
     return codes
 
 
-def qgemm_prepare(w_codes, act, wt, bias=None, encoding=QGEMM_I8):
-    """alpha[n], beta[n] of `qgemm` from device-resident quantizer parameters (no host sync).
-    act = (scale, offset_or_zero_point, lo, hi, form, g), wt = (scale [n] or [1], lo, hi, form, g); w_codes [n, k]."""
-    F._require_cuda(w_codes, "w_codes")
-    if w_codes.dtype != torch.uint8 or w_codes.dim() != 2 or not w_codes.is_contiguous():
-        raise DlmcqError("w_codes must be a contiguous [n, k] uint8 tensor")
-    n, k = w_codes.shape
-    dev = w_codes.device
+def _prepare_args(dev, n, act, wt, bias):
     a_s, a_o, a_lo, a_hi, a_form, a_g = act
     w_s, w_lo, w_hi, w_form, w_g = wt
     a_s = F._qvec(a_s, 1, dev, "activation scale")
@@ -67,13 +63,97 @@ def qgemm_prepare(w_codes, act, wt, bias=None, encoding=QGEMM_I8):
         b = bias.detach().to(device=dev, dtype=torch.float32).contiguous()
         if b.numel() != n:
             raise DlmcqError("bias must have n entries")
+    # the QParams hold raw pointers: the tensors are returned with them so that they outlive the call
+    return _qp(a_form, a_lo, a_hi, a_g, a_s, a_o), _qp(w_form, w_lo, w_hi, w_g, w_s, None), w_ch, b, (a_s, a_o, w_s)
+
+
+def qgemm_prepare(w_codes, act, wt, bias=None, encoding=QGEMM_I8):
+    """alpha[n], beta[n] of `qgemm` from device-resident quantizer parameters (no host sync).
+    act = (scale, offset_or_zero_point, lo, hi, form, g), wt = (scale [n] or [1], lo, hi, form, g); w_codes [n, k]."""
+    F._require_cuda(w_codes, "w_codes")
+    if w_codes.dtype != torch.uint8 or w_codes.dim() != 2 or not w_codes.is_contiguous():
+        raise DlmcqError("w_codes must be a contiguous [n, k] uint8 tensor")
+    n, k = w_codes.shape
+    dev = w_codes.device
+    qa, qw, w_ch, b, keep = _prepare_args(dev, n, act, wt, bias)
     alpha = torch.empty(n, dtype=torch.float32, device=dev)
     beta = torch.empty(n, dtype=torch.float32, device=dev)
-    qa, qw = _qp(a_form, a_lo, a_hi, a_g, a_s, a_o), _qp(w_form, w_lo, w_hi, w_g, w_s, None)
     with F._on(dev):
         _lib.check(_lib.lib().dlmcq_qgemm_prepare(F._ptr(w_codes), n, k, int(encoding), C.byref(qa), C.byref(qw), w_ch,
                                                   F._ptr(b), F._ptr(alpha), F._ptr(beta), F._stream_ptr()))
+    del keep
     return alpha, beta
+
+
+def _pair(v, name):
+    t = (v, v) if isinstance(v, int) else tuple(v)
+    if len(t) != 2 or not all(isinstance(e, int) for e in t):
+        raise DlmcqError(f"{name} must be an int or a pair of ints")
+    return t
+
+
+def _geom(batch, h, w, cin, n, kh, kw, stride=1, padding=0, dilation=1):
+    (sh, sw), (ph, pw), (dh, dw) = _pair(stride, "stride"), _pair(padding, "padding"), _pair(dilation, "dilation")
+    return ConvGeom(batch, h, w, cin, n, kh, kw, sh, sw, ph, pw, dh, dw, 1)
+
+
+def conv_out_size(size, k, stride, padding, dilation):
+    return (size + 2 * padding - dilation * (k - 1) - 1) // stride + 1
+
+
+def qconv_prepare(w_codes, act, wt, bias=None, encoding=QGEMM_I8):
+    """alpha [n] and the border-class beta table [(kh+1)^2 (kw+1)^2, n] of `qconv` from device-resident quantizer
+    parameters (no host sync): beta[class] covers the filter taps of a window that lie inside the image
+    (include/dlmcq.h, `dlmcq_qconv_prepare`).  w_codes: [n, kh, kw, cin] uint8 (channels-last weight codes);
+    act, wt as in `qgemm_prepare`."""
+    F._require_cuda(w_codes, "w_codes")
+    if w_codes.dtype != torch.uint8 or w_codes.dim() != 4 or not w_codes.is_contiguous():
+        raise DlmcqError("w_codes must be a contiguous [n, kh, kw, cin] uint8 tensor")
+    n, kh, kw, cin = w_codes.shape
+    dev = w_codes.device
+    qa, qw, w_ch, b, keep = _prepare_args(dev, n, act, wt, bias)
+    alpha = torch.empty(n, dtype=torch.float32, device=dev)
+    beta = torch.empty((kh + 1) ** 2 * (kw + 1) ** 2, n, dtype=torch.float32, device=dev)
+    g = _geom(1, 1, 1, cin, n, kh, kw)
+    with F._on(dev):
+        _lib.check(_lib.lib().dlmcq_qconv_prepare(F._ptr(w_codes), C.byref(g), int(encoding), C.byref(qa), C.byref(qw),
+                                                  w_ch, F._ptr(b), F._ptr(alpha), F._ptr(beta), F._stream_ptr()))
+    del keep
+    return alpha, beta
+
+
+def qconv(a_codes, w_codes, alpha, beta, stride=1, padding=0, dilation=1, relu=False, out_dtype=torch.float32,
+          a_signed=False, encoding=QGEMM_I8, out=None):
+    """Convolution of channels-last codes: a_codes [B, H, W, cin], w_codes [n, kh, kw, cin] (uint8, contiguous) ->
+    out [B, Ho, Wo, n] = alpha[n] * acc + beta[border class][n] (two fp32 roundings), optional ReLU; zero padding
+    of the fake-quantised tensor, i.e. padded taps contribute neither to acc nor to beta."""
+    F._require_cuda(a_codes, "a_codes")
+    F._require_cuda(w_codes, "w_codes")
+    if a_codes.dtype != torch.uint8 or w_codes.dtype != torch.uint8 or a_codes.dim() != 4 or w_codes.dim() != 4:
+        raise DlmcqError("a_codes [B, H, W, cin] and w_codes [n, kh, kw, cin] must be uint8 tensors")
+    if not (a_codes.is_contiguous() and w_codes.is_contiguous()):
+        raise DlmcqError("code tensors must be contiguous (channels innermost)")
+    bsz, h, w, cin = a_codes.shape
+    n, kh, kw, cin2 = w_codes.shape
+    if cin != cin2 or alpha.numel() != n or tuple(beta.shape) != ((kh + 1) ** 2 * (kw + 1) ** 2, n):
+        raise DlmcqError("shape mismatch between a_codes, w_codes, alpha, beta")
+    if out_dtype not in (torch.float32, torch.bfloat16):
+        raise DlmcqError("out_dtype must be float32 or bfloat16")
+    g = _geom(bsz, h, w, cin, n, kh, kw, stride, padding, dilation)
+    ho = conv_out_size(h, kh, g.stride_h, g.pad_h, g.dil_h)
+    wo = conv_out_size(w, kw, g.stride_w, g.pad_w, g.dil_w)
+    if ho < 1 or wo < 1:
+        raise DlmcqError("the convolution has no output pixel")
+    shape = (bsz, ho, wo, n)
+    if out is None:
+        out = torch.empty(shape, dtype=out_dtype, device=a_codes.device)
+    elif tuple(out.shape) != shape or out.dtype != out_dtype or not out.is_contiguous() or out.device != a_codes.device:
+        raise DlmcqError("out must be a contiguous [B, Ho, Wo, n] tensor of out_dtype on the operands' device")
+    with F._on(a_codes.device):
+        _lib.check(_lib.lib().dlmcq_qconv(F._ptr(a_codes), F._ptr(w_codes), F._ptr(alpha), F._ptr(beta), F._ptr(out),
+                                          C.byref(g), int(encoding), int(bool(a_signed)), int(bool(relu)),
+                                          F32 if out_dtype == torch.float32 else BF16, F._stream_ptr()))
+    return out
 
 
 def qgemm(a_codes, w_codes, alpha, beta, relu=False, out_dtype=torch.float32, a_signed=False, encoding=QGEMM_I8,
@@ -128,6 +208,20 @@ def _geometry_ok(mod):
     return False
 
 
+def _conv_geometry_ok(mod):
+    """Conv2d layers the implicit-GEMM kernel serves (dlmcq_qconv): one group, zero padding, Cin a multiple of 64,
+    stride <= 8 and im2col bounding-box corners -pad, pad - dil*(k-1) in [-128, 127].  Stride-1 1x1 layers without
+    padding keep the plain GEMM (`_geometry_ok`)."""
+    if not isinstance(mod, nn.Conv2d) or isinstance(mod.padding, str) or _geometry_ok(mod):
+        return False
+    if mod.groups != 1 or mod.padding_mode != 'zeros' or mod.in_channels % 64 != 0:
+        return False
+    for k, s, p, d in zip(mod.kernel_size, mod.stride, mod.padding, mod.dilation):
+        if not (1 <= s <= 8 and 0 <= p <= 128 and -128 <= p - d * (k - 1) <= 127 and k <= 255):
+            return False
+    return True
+
+
 def _enabled(mod):
     q = mod.qconfig
     if hasattr(mod, 'act_quant'):            # FSPTQBase switches (change_quant_state)
@@ -138,8 +232,9 @@ def _enabled(mod):
 class _CodeGemmState:
     """Per-layer cache of the weight codes and the epilogue vectors, rebuilt when any tensor they derive from changes."""
 
-    def __init__(self, encoding):
+    def __init__(self, encoding, conv=False):
         self.encoding = encoding
+        self.conv = conv                     # implicit-GEMM convolution (qconv) instead of the [m, k] GEMM
         self.key = None
         self.w_codes = self.alpha = self.beta = None
         self.usable = None                   # None = not decided yet (needs initialised qparams)
@@ -173,8 +268,11 @@ class _CodeGemmState:
             self.w_codes = self.alpha = self.beta = None
             return False
         w = mod.weight.detach()
-        w2 = w.reshape(n, -1)                # 1x1 conv weights [n, k, 1, 1] are [n, k] matrices in either memory format
-        w2 = w2 if w2.is_contiguous() else w2.contiguous()
+        if self.conv:
+            w2 = w.permute(0, 2, 3, 1).contiguous()      # [n, kh, kw, cin]: K in (r, s, c) order
+        else:
+            w2 = w.reshape(n, -1)            # 1x1 conv weights [n, k, 1, 1] are [n, k] matrices in either memory format
+            w2 = w2 if w2.is_contiguous() else w2.contiguous()
         g_w = 1 / math.sqrt(w.numel() * hi_w) if w_form == FORM_AFFINE else 0.0
         per_ch = ws.numel() == n and n != 1
         self.w_codes = codes_forward(w2, ws.reshape(-1), None, lo_w, hi_w, w_form, g_w, ch_axis=0 if per_ch else None,
@@ -193,7 +291,8 @@ class _CodeGemmState:
             return self.alpha, self.beta
         g_a = 1 / math.sqrt(numel * mod.in_max_val) if a_form == FORM_AFFINE else 0.0
         act = (mod.in_scale.detach().reshape(-1), mod.in_offset, mod.in_min_val, mod.in_max_val, a_form, g_a)
-        self.alpha, self.beta = qgemm_prepare(self.w_codes, act, self._wt, mod.bias, self.encoding)
+        prepare = qconv_prepare if self.conv else qgemm_prepare
+        self.alpha, self.beta = prepare(self.w_codes, act, self._wt, mod.bias, self.encoding)
         self._ab_numel = numel
         self._g_a = g_a
         return self.alpha, self.beta
@@ -227,6 +326,10 @@ def _code_forward(self, input):
     alpha, beta = st.epilogue(self, forms, numel)
     a_codes = codes_forward(x, self.in_scale.detach().reshape(-1), self.in_offset, self.in_min_val, self.in_max_val,
                             a_form, st._g_a, encoding=st.encoding)
+    if st.conv:
+        out = qconv(a_codes.permute(0, 2, 3, 1), st.w_codes, alpha, beta, self.stride, self.padding, self.dilation,
+                    out_dtype=input.dtype, a_signed=self.in_min_val < 0, encoding=st.encoding)
+        return out.permute(0, 3, 1, 2)                           # NCHW view of channels-last storage
     k = self.weight.shape[1] if isinstance(self, nn.Conv2d) else self.weight.shape[-1]
     # elementwise codes keep x's memory order: channels-last NCHW storage is the [B*H*W, C] matrix
     a2 = a_codes.permute(0, 2, 3, 1).reshape(rows, k) if isinstance(self, nn.Conv2d) else a_codes.reshape(rows, k)
@@ -245,17 +348,22 @@ def _auto_encoding(mod):
     return QGEMM_E4M3 if small else QGEMM_I8
 
 
-def enable_code_gemm(model, encoding=None):
+def enable_code_gemm(model, encoding=None, convolutions=False):
     """Route every eligible quantised Linear / 1x1 Conv2d of `model` through the integer-code GEMM in eval mode
-    (`encoding`: QGEMM_I8, QGEMM_E4M3, or None = per layer by code range).
+    (`encoding`: QGEMM_I8, QGEMM_E4M3, or None = per layer by code range).  With `convolutions=True` also every
+    quantised Conv2d the implicit-GEMM kernel serves (k x k, strided, padded, dilated; one group, zero padding,
+    Cin % 64 == 0): `qconv` on the channels-last codes.
     Returns the list of module names switched.  Eligibility that depends on calibrated state (per-tensor activation
     scale, zero weight offset, ...) is re-checked lazily and a layer that fails it silently keeps its original path."""
     names = []
     for name, mod in model.named_modules():
         forms = _family(mod)
-        if forms is None or not _geometry_ok(mod) or '_code_gemm' in mod.__dict__:
+        if forms is None or '_code_gemm' in mod.__dict__:
             continue
-        mod.__dict__['_code_gemm'] = _CodeGemmState(_auto_encoding(mod) if encoding is None else encoding)
+        conv = convolutions and _conv_geometry_ok(mod)
+        if not (conv or _geometry_ok(mod)):
+            continue
+        mod.__dict__['_code_gemm'] = _CodeGemmState(_auto_encoding(mod) if encoding is None else encoding, conv)
         mod.__dict__['_code_gemm_forms'] = forms
         mod.__dict__['_code_gemm_orig_forward'] = mod.forward
         mod.forward = types.MethodType(_code_forward, mod)

@@ -523,6 +523,46 @@ int dlmcq_qgemm_prepare(const void* w_codes, int64_t n, int64_t k, int encoding,
 int dlmcq_qgemm(const void* a_codes, const void* w_codes, const float* alpha, const float* beta, void* out, int64_t m,
                 int64_t n, int64_t k, int encoding, int a_signed, int relu, int out_dtype, void* stream);
 
+/* ---- the convolution on the integer codes: implicit GEMM over channels-last codes -----------------------------------
+ * Replaces `_forward_func(q_input, q_weight)` = F.conv2d(q_input, q_weight, bias, stride, padding, dilation) of a
+ * QConv2d (modules/conv.py `_conv_forward`, entered from modules/base.py:140; FSPTQuant/base.py:111-113) for the
+ * same quantizer forms as dlmcq_qgemm, any kh x kw filter, stride, zero padding and dilation.  The A operand is read
+ * straight from the [B, H, W, Cin] activation codes by TMA im2col loads (one K block = one filter tap x 128 or 64
+ * channels); nothing is unfolded in memory.
+ *
+ * Padding.  The reference pads the FAKE-QUANTISED tensor with real zeros.  A zero code is not a zero value when the
+ * activation has an offset or zero-point (t = o_a - z_a*m_a != 0), so beta depends on which taps of an output pixel's
+ * window lie inside the image.  Those taps are a contiguous range [r_lo, r_hi1) of filter rows times [s_lo, s_hi1) of
+ * filter columns (each end in [0, k]; empty when lo >= hi1), the border class of the pixel:
+ *     out[p, n] = RN(RN(float(acc[p, n]) * alpha[n]) + beta[class(p)][n]),  optionally max(., 0)
+ *     acc[p, n] = sum over the valid taps (r, s) and c of ca[pixel under tap (r, s)][c] * cw[n, r, s, c]   (exact)
+ *     beta[class][n] = RN(RN(t * m_w[n]) * float(sum_{r_lo <= r < r_hi1, s_lo <= s < s_hi1} sum_c cw[n, r, s, c]))
+ *                      (+ bias[n]),   t = RN(o_a - RN(z_a * m_a)),  alpha[n] = RN(m_a * m_w[n])
+ * For an interior pixel this is dlmcq_qgemm's formula over the whole K = kh*kw*Cin.
+ *
+ * dlmcq_conv_geom   input [batch, h, w, cin] channels-last, n output channels, kh x kw filter, stride / pad / dilation
+ *                   per axis, groups.  Ho = (h + 2*pad_h - dil_h*(kh-1) - 1) / stride_h + 1 (Wo likewise).
+ * dlmcq_qconv_prepare  alpha [n] and the border-class table beta [(kh+1)^2 * (kw+1)^2][n] fp32 (the caller allocates
+ *                   both; class = ((r_lo*(kh+1) + r_hi1)*(kw+1) + s_lo)*(kw+1) + s_hi1) from DEVICE-resident qparams
+ *                   (no host sync).  Reads only n, cin, kh, kw, groups of geom: the table serves every input size.
+ *                   w_codes: [n, kh, kw, cin] bytes (the storage of a channels-last weight), same encodings and qparams
+ *                   rules as dlmcq_qgemm_prepare.
+ * dlmcq_qconv       a_codes [batch, h, w, cin], w_codes [n, kh, kw, cin] bytes, 16-byte aligned (DLMCQ_EALIGN);
+ *                   out [batch, Ho, Wo, n] row-major fp32 / bf16 (channels-last).  a_signed: activation codes are int8.
+ * Both return DLMCQ_EUNSUPPORTED before any launch for groups != 1, cin % 64 != 0, kh or kw > 255, stride > 8,
+ * bounding-box corners -pad or pad - dil*(k-1) outside [-128, 127], and sizes beyond 32-bit coordinates (batch*Ho*Wo,
+ * n or K above 2^31 - 256, (kh+1)^2 (kw+1)^2 n above 2^31 - 1); DLMCQ_EINVAL for non-positive sizes, negative padding
+ * or a geometry without an output pixel. */
+typedef struct {
+  int64_t batch, h, w, cin, n;
+  int32_t kh, kw, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w, groups;
+} dlmcq_conv_geom;
+int dlmcq_qconv_prepare(const void* w_codes, const dlmcq_conv_geom* geom, int encoding, const dlmcq_qparams* act_qp,
+                        const dlmcq_qparams* wt_qp, int64_t wt_channels, const float* bias, float* alpha, float* beta,
+                        void* stream);
+int dlmcq_qconv(const void* a_codes, const void* w_codes, const float* alpha, const float* beta, void* out,
+                const dlmcq_conv_geom* geom, int encoding, int a_signed, int relu, int out_dtype, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
