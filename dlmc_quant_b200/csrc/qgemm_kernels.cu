@@ -607,6 +607,16 @@ int code_range_ok(const dlmcq_qparams* qp, int encoding) {
   return DLMCQ_OK;
 }
 
+// Exactness of the accumulation: every partial sum of k products is at most k * max|a| * max|w|.  The fp32
+// accumulators of kind::f8f6f4 hold every integer up to 2^24, the s32 accumulators of kind::i8 up to 2^31 - 1.
+// Call after code_range_ok (|code| <= 255).
+int accumulator_ok(int64_t k, const dlmcq_qparams* act_qp, const dlmcq_qparams* wt_qp, int encoding) {
+  const int64_t ma = act_qp->hi > -act_qp->lo ? act_qp->hi : -act_qp->lo;
+  const int64_t mw = wt_qp->hi > -wt_qp->lo ? wt_qp->hi : -wt_qp->lo;
+  const int64_t bound = encoding == DLMCQ_QGEMM_E4M3 ? (1LL << 24) : 0x7fffffffLL;
+  return (ma * mw == 0 || k <= bound / (ma * mw)) ? DLMCQ_OK : DLMCQ_EUNSUPPORTED;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // alpha[n], beta[n] from the device-resident quantizer parameters; one warp per output channel
 // ---------------------------------------------------------------------------------------------------------------
@@ -894,6 +904,7 @@ extern "C" int dlmcq_qgemm_prepare(const void* w_codes, int64_t n, int64_t k, in
   // the product only factors for weights without an additive term: y_w = code * m_w
   if (wt_qp->form == DLMCQ_FORM_ZP || wt_qp->offset != nullptr) return DLMCQ_EUNSUPPORTED;
   if (encoding == DLMCQ_QGEMM_I8 && wt_qp->lo >= 0 && wt_qp->hi > 127) return DLMCQ_EUNSUPPORTED;   // B operand is s8
+  if (int e = accumulator_ok(k, act_qp, wt_qp, encoding)) return e;
   const int64_t blocks = (n + kRowWarps - 1) / kRowWarps;
   if (blocks > 0x7fffffffLL) return DLMCQ_EUNSUPPORTED;
   qgemm_prepare_kernel<<<static_cast<unsigned>(blocks), kRowWarps * 32, 0, static_cast<cudaStream_t>(stream)>>>(
@@ -939,6 +950,7 @@ extern "C" int dlmcq_qconv_prepare(const void* w_codes, const dlmcq_conv_geom* g
   if (int e = code_range_ok(wt_qp, encoding)) return e;
   if (wt_qp->form == DLMCQ_FORM_ZP || wt_qp->offset != nullptr) return DLMCQ_EUNSUPPORTED;
   if (encoding == DLMCQ_QGEMM_I8 && wt_qp->lo >= 0 && wt_qp->hi > 127) return DLMCQ_EUNSUPPORTED;
+  if (int e = accumulator_ok(static_cast<int64_t>(geom->kh) * geom->kw * geom->cin, act_qp, wt_qp, encoding)) return e;
   const size_t smem = static_cast<size_t>(geom->kh) * geom->kw * sizeof(int);
   if (smem > 48 * 1024) return DLMCQ_EUNSUPPORTED;
   qconv_prepare_kernel<<<static_cast<unsigned>(n), kConvPrepThreads, smem, static_cast<cudaStream_t>(stream)>>>(

@@ -149,6 +149,8 @@ def qconv(a_codes, w_codes, alpha, beta, stride=1, padding=0, dilation=1, relu=F
         out = torch.empty(shape, dtype=out_dtype, device=a_codes.device)
     elif tuple(out.shape) != shape or out.dtype != out_dtype or not out.is_contiguous() or out.device != a_codes.device:
         raise DlmcqError("out must be a contiguous [B, Ho, Wo, n] tensor of out_dtype on the operands' device")
+    if bsz == 0:
+        return out                           # an empty batch, as qgemm with m = 0 (dlmcq_qconv refuses batch 0)
     with F._on(a_codes.device):
         _lib.check(_lib.lib().dlmcq_qconv(F._ptr(a_codes), F._ptr(w_codes), F._ptr(alpha), F._ptr(beta), F._ptr(out),
                                           C.byref(g), int(encoding), int(bool(a_signed)), int(bool(relu)),
@@ -263,6 +265,7 @@ class _CodeGemmState:
             usable = usable and lo_w >= -16 and hi_w <= 16 and lo_a >= -16 and hi_a <= 16
         else:
             usable = usable and lo_w >= -128 and hi_w <= 127 and lo_a >= -128 and hi_a <= 255 and (lo_a >= 0 or hi_a <= 127)
+        usable = usable and accumulator_exact(self.encoding, mod.weight[0].numel(), lo_a, hi_a, lo_w, hi_w)
         self.usable = usable
         if not usable:
             self.w_codes = self.alpha = self.beta = None
@@ -340,17 +343,31 @@ def _code_forward(self, input):
     return out.view(*input.shape[:-1], n)
 
 
+def accumulator_exact(encoding, k, a_lo, a_hi, w_lo, w_hi):
+    """Whether every partial sum of k code products fits the encoding's accumulator exactly (include/dlmcq.h):
+    k * max|a| * max|w| <= 2^24 for e4m3 (fp32 accumulators), <= 2^31 - 1 for the integer kind (s32).  The prepare
+    entries refuse the layers that fail it."""
+    bound = (1 << 24) if encoding == QGEMM_E4M3 else (1 << 31) - 1
+    return k * max(-a_lo, a_hi) * max(-w_lo, w_hi) <= bound
+
+
 def _auto_encoding(mod):
     """e4m3 operands (fp32 accumulators: no int -> float conversion in the epilogue) when every code of the layer is
-    exactly representable (|code| <= 16, i.e. up to 4-bit unsigned / 5-bit signed ranges), the integer kind otherwise.
-    Both are bit-identical where both apply (tests/qgemm_cases.py)."""
+    exactly representable (|code| <= 16, i.e. up to 4-bit unsigned / 5-bit signed ranges) and the layer's K keeps the
+    fp32 accumulation exact, the integer kind otherwise, None when neither accumulates exactly.  Both are bit-identical
+    where both apply (tests/qgemm_cases.py)."""
+    k = mod.weight[0].numel()
+    ranges = (mod.in_min_val, mod.in_max_val, mod.wt_min_val, mod.wt_max_val)
     small = mod.wt_min_val >= -16 and mod.wt_max_val <= 16 and mod.in_min_val >= -16 and mod.in_max_val <= 16
-    return QGEMM_E4M3 if small else QGEMM_I8
+    if small and accumulator_exact(QGEMM_E4M3, k, *ranges):
+        return QGEMM_E4M3
+    return QGEMM_I8 if accumulator_exact(QGEMM_I8, k, *ranges) else None
 
 
 def enable_code_gemm(model, encoding=None, convolutions=False):
     """Route every eligible quantised Linear / 1x1 Conv2d of `model` through the integer-code GEMM in eval mode
-    (`encoding`: QGEMM_I8, QGEMM_E4M3, or None = per layer by code range).  With `convolutions=True` also every
+    (`encoding`: QGEMM_I8, QGEMM_E4M3, or None = per layer by code range and K, `_auto_encoding`; a layer that
+    no encoding accumulates exactly is not switched).  With `convolutions=True` also every
     quantised Conv2d the implicit-GEMM kernel serves (k x k, strided, padded, dilated; one group, zero padding,
     Cin % 64 == 0): `qconv` on the channels-last codes.
     Returns the list of module names switched.  Eligibility that depends on calibrated state (per-tensor activation
@@ -363,7 +380,10 @@ def enable_code_gemm(model, encoding=None, convolutions=False):
         conv = convolutions and _conv_geometry_ok(mod)
         if not (conv or _geometry_ok(mod)):
             continue
-        mod.__dict__['_code_gemm'] = _CodeGemmState(_auto_encoding(mod) if encoding is None else encoding, conv)
+        enc = _auto_encoding(mod) if encoding is None else encoding
+        if enc is None:
+            continue                         # no operand encoding accumulates this layer's K exactly
+        mod.__dict__['_code_gemm'] = _CodeGemmState(enc, conv)
         mod.__dict__['_code_gemm_forms'] = forms
         mod.__dict__['_code_gemm_orig_forward'] = mod.forward
         mod.forward = types.MethodType(_code_forward, mod)

@@ -498,7 +498,12 @@ int dlmcq_host_ctx_fq_codes(dlmcq_host_ctx* ctx, const void* x_host, const void*
  * accumulators).  Activations are read at ONE byte per element instead of four.
  *   encoding DLMCQ_QGEMM_I8    one byte per code, uint8 (lo >= 0) or two's complement; tcgen05.mma kind::i8, s32
  *                              accumulators: exact for every range dlmcq_export_codes accepts (weights: hi <= 127)
- *   encoding DLMCQ_QGEMM_E4M3  the code as an e4m3 byte, kind::f8f6f4, fp32 accumulators: |code| <= 16 only
+ *                              while K * max|a| * max|w| <= 2^31 - 1
+ *   encoding DLMCQ_QGEMM_E4M3  the code as an e4m3 byte, kind::f8f6f4, fp32 accumulators: |code| <= 16 only, exact
+ *                              while K * max|a| * max|w| <= 2^24 (fp32 holds every integer up to 2^24)
+ * The bound covers every partial sum of the accumulation, whatever order the tensor core adds the products in.
+ * max|a|, max|w| are max(|lo|, |hi|) of the quantizer's code range; the prepare entries return DLMCQ_EUNSUPPORTED
+ * when K * max|a| * max|w| exceeds the encoding's bound (K = kh*kw*Cin for the convolution).
  *
  * dlmcq_codes_forward   x -> codes, one byte each; the same arithmetic (and therefore the same codes) as
  *                       dlmcq_fq_forward / dlmcq_export_codes for every form and layout; NaN -> 0.

@@ -20,6 +20,7 @@ if ROOT not in sys.path:
 import torch  # noqa: E402
 
 from tests.qconv_oracle import A1, AFFINE, GEOMETRIES, SYM, ZP, code_conv, conv_problem, conv_reference  # noqa: E402
+from tests.qgemm_cases import PATTERNS, act_codes_of, blocked_acc, wt_codes_of  # noqa: E402
 
 I8, E4M3 = 0, 1
 
@@ -43,15 +44,26 @@ def _assert_equal(got, want, what):
 
 
 def case_raw(geom, encoding, batch=2, cin=64, n=40, a_signed=False, relu=False, bf16=False, zp=False, seed=0,
-             a_hi=15, w_hi=7):
-    """random codes -> qconv_prepare (A1 offset or ZP zero-point activation, per-channel SYM weight) -> qconv vs
-    code_conv, bit for bit."""
+             a_hi=15, w_hi=7, pattern="random"):
+    """codes of a pattern (tests/qgemm_cases.py PATTERNS; the weights' K order is the kernel's (r, s, c)) ->
+    qconv_prepare (A1 offset or ZP zero-point activation, per-channel SYM weight) -> qconv vs code_conv, bit for bit.
+    The worst-case patterns report K, the largest |acc| and the largest |partial sum| of the exact accumulation."""
     from dlmc_quant_b200 import qgemm as Q
     kh, kw, stride, padding, dilation, h, w = geom
     g = torch.Generator().manual_seed(seed)
     a_lo = -a_hi if a_signed else 0
-    ca = torch.randint(a_lo, a_hi + 1, (batch, cin, h, w), generator=g)
-    cw = torch.randint(-w_hi, w_hi + 1, (n, cin, kh, kw), generator=g)
+    report = {}
+    if pattern == "random":
+        ca = torch.randint(a_lo, a_hi + 1, (batch, cin, h, w), generator=g)
+        cw = torch.randint(-w_hi, w_hi + 1, (n, cin, kh, kw), generator=g)
+    else:
+        ca = act_codes_of(pattern, (batch, cin, h, w), a_hi, a_signed, g)
+        cw_k = wt_codes_of(pattern, n, kh * kw * cin, w_hi, g)                 # [n, K], K = (r, s, c)
+        cw = cw_k.reshape(n, kh, kw, cin).permute(0, 3, 1, 2).contiguous()
+        cols = torch.nn.functional.unfold(ca.double(), (kh, kw), dilation=dilation, padding=padding, stride=stride)
+        cols = cols.reshape(batch, cin, kh, kw, -1).permute(0, 4, 2, 3, 1).reshape(-1, kh * kw * cin)
+        acc, peak = blocked_acc(cols, cw_k)
+        report.update(K=kh * kw * cin, max_abs_acc=int(acc.abs().max().item()), peak_abs_partial_sum=int(peak))
     s_a = torch.tensor([0.0371])
     off = torch.tensor([3.0 if zp else -0.21])
     s_w = (torch.rand(n, generator=g) * 0.01 + 1e-3)
@@ -69,7 +81,7 @@ def case_raw(geom, encoding, batch=2, cin=64, n=40, a_signed=False, relu=False, 
     if bf16:
         want = want.to(torch.bfloat16)
     _assert_equal(out.cpu(), want, "vs code_conv")
-    return {"pixels": out.shape[0] * out.shape[1] * out.shape[2], "n": n}
+    return {"pixels": out.shape[0] * out.shape[1] * out.shape[2], "n": n, **report}
 
 
 def case_pipeline(geom, a_form, w_form, encoding, dtype=torch.float32, cin=64, n=48, n_bits=4, a_signed=False,
@@ -289,6 +301,19 @@ def case_errors():
             "huge": EUNSUPPORTED}
     assert got == want, got
     assert run() == 0
+    # the accumulator bound of qconv_prepare (K = kh*kw*Cin): accepted at K * 16 * 16 = 2^24 (e4m3) and at the largest
+    # Cin of 8-bit 3x3 codes below 2^31 - 1 (integer kind), refused one channel block above
+    act = lambda hi: (torch.ones(1).cuda(), torch.zeros(1).cuda(), 0, hi, A1, 0.0)  # noqa: E731
+    for enc, a_hi, w_hi, taps, cin_ok in ((E4M3, 16, 16, 1, 65536), (I8, 255, 127, 3, 7360)):
+        for cin, ok in ((cin_ok, True), (cin_ok + 64, False)):
+            try:
+                Q.qconv_prepare(torch.zeros(4, taps, taps, cin, dtype=torch.uint8).cuda(), act(a_hi),
+                                (al, -w_hi, w_hi, SYM, 0.0), None, enc)
+                accepted = True
+            except _lib.DlmcqError as e:
+                assert "unsupported" in str(e), e
+                accepted = False
+            assert accepted == ok, (enc, cin)
     torch.cuda.synchronize()
     return {}
 
@@ -310,6 +335,27 @@ def build_cases():
         # 392 tiles over 148 SMs: persistent walk, both TMEM buffers reused; 28x28 planes: tiles straddle images
         cases.append((f"raw_{tag}_persistent", case_raw, dict(geom=(3, 3, 1, 1, 1, 28, 28), encoding=enc, batch=32,
                                                                cin=128, n=256)))
+    # n = 1 (scalar epilogue, one-row beta table), n = 2048 (16 N tiles), a single output pixel, batch 1 below one tile
+    for enc, tag in ((I8, "i8"), (E4M3, "e4m3")):
+        cases.append((f"raw_{tag}_n1", case_raw, dict(geom=GEOMETRIES["3x3_pad1"], encoding=enc, n=1)))
+        cases.append((f"raw_{tag}_n2048", case_raw, dict(geom=GEOMETRIES["3x3_pad1_stride2"], encoding=enc, n=2048)))
+        cases.append((f"raw_{tag}_one_output_pixel", case_raw, dict(geom=(3, 3, 1, 0, 1, 3, 3), encoding=enc, batch=1,
+                                                                     cin=128, n=96)))
+        cases.append((f"raw_{tag}_batch1_below_one_tile", case_raw, dict(geom=(3, 3, 1, 1, 1, 9, 11), encoding=enc,
+                                                                          batch=1, n=72)))
+    # worst-case accumulators (tests/qgemm_cases.py PATTERNS): the ResNet-50 3x3 layers' K = 9 * 64 ... 9 * 512 on
+    # both kinds; e4m3 with |code| = 16 at K = 9 * 7232 (K * 256 just below 2^24); 8-bit codes on the integer kind at
+    # K = 9 * 7360 (K * 255 * 127 just below 2^31 - 1)
+    g_acc = (3, 3, 1, 1, 1, 12, 11)
+    for pattern in PATTERNS[1:]:
+        for enc, tag in ((I8, "i8"), (E4M3, "e4m3")):
+            for cin in (64, 128, 256, 512):
+                cases.append((f"acc_{tag}_{pattern}_k{9 * cin}", case_raw,
+                              dict(geom=g_acc, encoding=enc, cin=cin, n=64, pattern=pattern, seed=cin)))
+        cases.append((f"acc_e4m3_{pattern}_k{9 * 7232}", case_raw,
+                      dict(geom=g_acc, encoding=E4M3, cin=7232, n=64, a_hi=16, w_hi=16, pattern=pattern)))
+        cases.append((f"acc_i8_8bit_{pattern}_k{9 * 7360}", case_raw,
+                      dict(geom=g_acc, encoding=I8, cin=7360, n=64, a_hi=255, w_hi=127, pattern=pattern)))
     cases.append(("raw_i8_8bit_signed", case_raw, dict(geom=(3, 3, 1, 1, 1, 9, 9), encoding=I8, cin=512, n=64,
                                                        a_signed=True, a_hi=127, w_hi=127)))
     cases.append(("raw_i8_8bit", case_raw, dict(geom=(3, 3, 1, 1, 1, 7, 7), encoding=I8, cin=512, n=64, a_hi=255,

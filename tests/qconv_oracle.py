@@ -22,7 +22,7 @@ def code_conv(a_codes, w_codes, m_a, o_a, z_a, m_w, bias=None, stride=1, padding
         out = RN(RN(float(acc) * alpha[n]) + beta),  acc = sum over the taps inside the image (exact)
         beta = RN(RN(t * m_w[n]) * float(sum of cw over the taps inside the image)) (+ bias[n]),  t = o_a - z_a*m_a.
     whole_k_beta=True uses sum_k cw for every pixel (the 1x1 rule; wrong at borders when t != 0)."""
-    f32, f64 = torch.float32, torch.float64
+    f64 = torch.float64
     ca, cw = a_codes.to(f64), w_codes.to(f64)
     kw_ = dict(stride=stride, padding=padding, dilation=dilation)
     acc = F.conv2d(ca, cw, **kw_)
@@ -31,16 +31,77 @@ def code_conv(a_codes, w_codes, m_a, o_a, z_a, m_w, bias=None, stride=1, padding
     else:
         ones = torch.ones(1, 1, *ca.shape[2:], dtype=f64)
         wsum = F.conv2d(ones, _tap_weight_sums(cw), **kw_)                   # [1, n, Ho, Wo]: valid taps only
-    m_a, o_a, z_a = (torch.as_tensor(v, dtype=f32).reshape(()) for v in (m_a, o_a, z_a))
-    n = cw.shape[0]
-    m_w = torch.as_tensor(m_w, dtype=f32).reshape(-1).expand(n).reshape(1, n, 1, 1)
+    return conv_epilogue(acc, wsum, m_a, o_a, z_a, m_w, bias, relu)
+
+
+def conv_epilogue(acc, wsum, m_a, o_a, z_a, m_w, bias=None, relu=False):
+    """The kernels' two fp32 roundings on an exact integer convolution acc [B, n, Ho, Wo] and the per-pixel sum of
+    the weight codes over the taps inside the image wsum [1, n, Ho, Wo] (both float64, on any device)."""
+    f32 = torch.float32
+    dev = acc.device
+    m_a, o_a, z_a = (torch.as_tensor(v, dtype=f32).to(dev).reshape(()) for v in (m_a, o_a, z_a))
+    n = acc.shape[1]
+    m_w = torch.as_tensor(m_w, dtype=f32).to(dev).reshape(-1).expand(n).reshape(1, n, 1, 1)
     alpha = m_a * m_w
     t = o_a - z_a * m_a
     beta = (t * m_w) * wsum.to(f32)
     if bias is not None:
-        beta = beta + bias.to(f32).reshape(1, n, 1, 1)
+        beta = beta + bias.to(device=dev, dtype=f32).reshape(1, n, 1, 1)
     out = acc.to(f32) * alpha + beta
     return torch.relu(out) if relu else out
+
+
+def conv_pairs(stride, padding, dilation):
+    """(stride_h, stride_w), (pad_h, pad_w), (dil_h, dil_w) of an int-or-pair geometry."""
+    return tuple((v, v) if isinstance(v, int) else tuple(v) for v in (stride, padding, dilation))
+
+
+def _out_size(size, k, s, p, d):
+    return (size + 2 * p - d * (k - 1) - 1) // s + 1
+
+
+def exact_conv_acc(a_codes, w_codes, stride=1, padding=0, dilation=1):
+    """The integer convolution of a_codes [B, Cin, H, W] with w_codes [n, Cin, kh, kw] (integer-valued, any memory
+    format) as one float64 matmul per filter tap over a zero-padded, strided view of the channels-last codes, on the
+    codes' device.  Every product and partial sum is an integer below 2^53, so the sum is exact in any order (no
+    library convolution: its algorithm choice is not ours).  Returns float64 [B, n, Ho, Wo] (channels-last storage)."""
+    (sh, sw), (ph, pw), (dh, dw) = conv_pairs(stride, padding, dilation)
+    b, cin, h, w = a_codes.shape
+    n, _, kh, kw = w_codes.shape
+    ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
+    f64 = torch.float64
+    x = torch.zeros(b, h + 2 * ph, w + 2 * pw, cin, dtype=f64, device=a_codes.device)
+    x[:, ph:ph + h, pw:pw + w] = a_codes.permute(0, 2, 3, 1).to(f64)
+    wt = w_codes.to(device=a_codes.device, dtype=f64).permute(2, 3, 1, 0)          # [kh, kw, Cin, n]
+    acc = torch.zeros(b * ho * wo, n, dtype=f64, device=a_codes.device)
+    for r in range(kh):
+        for s in range(kw):
+            tap = x[:, r * dh:r * dh + (ho - 1) * sh + 1:sh, s * dw:s * dw + (wo - 1) * sw + 1:sw]
+            acc.addmm_(tap.reshape(-1, cin), wt[r, s])
+    return acc.view(b, ho, wo, n).permute(0, 3, 1, 2)
+
+
+def valid_tap_wsum(w_codes, h, w, stride=1, padding=0, dilation=1):
+    """[1, n, Ho, Wo] float64: per output pixel, the sum of the weight codes over the filter taps inside the image
+    (the border rule of beta), on w_codes' device."""
+    (sh, sw), (ph, pw), (dh, dw) = conv_pairs(stride, padding, dilation)
+    n, _, kh, kw = w_codes.shape
+    ho, wo = _out_size(h, kh, sh, ph, dh), _out_size(w, kw, sw, pw, dw)
+    dev, f64 = w_codes.device, torch.float64
+
+    def valid(k, o, s, p, d, size):                                     # [k, o]: tap inside the image
+        pos = (torch.arange(o, device=dev) * s - p).reshape(1, -1) + (torch.arange(k, device=dev) * d).reshape(-1, 1)
+        return ((pos >= 0) & (pos < size)).to(f64)
+    taps = w_codes.to(f64).sum(dim=1)                                   # [n, kh, kw]
+    return torch.einsum("rh,sw,nrs->nhw", valid(kh, ho, sh, ph, dh, h), valid(kw, wo, sw, pw, dw, w), taps)[None]
+
+
+def exact_conv(a_codes, w_codes, m_a, o_a, z_a, m_w, bias=None, stride=1, padding=0, dilation=1, relu=False):
+    """code_conv's result from exact_conv_acc and valid_tap_wsum: the same value, on the codes' device."""
+    kw_ = dict(stride=stride, padding=padding, dilation=dilation)
+    acc = exact_conv_acc(a_codes, w_codes, **kw_)
+    wsum = valid_tap_wsum(w_codes.to(acc.device), a_codes.shape[2], a_codes.shape[3], **kw_)
+    return conv_epilogue(acc, wsum, m_a, o_a, z_a, m_w, bias, relu)
 
 
 def conv_reference(q_input, q_weight, bias=None, stride=1, padding=0, dilation=1):
@@ -68,6 +129,22 @@ GEOMETRIES = {
     "3x3_odd_hw": (3, 3, 1, 1, 1, 7, 5),
     "7x7_image_3x3_stride2": (3, 3, 2, 1, 1, 7, 7),
     "3x3_pad_eq_dil_k": (3, 3, 1, 4, 2, 8, 9),              # padding = d*(k-1): upper corner 0
+    # per-axis strides / dilations / paddings: an h <-> w swap anywhere in the kernel's geometry shows here
+    "3x3_stride_1x2": (3, 3, (1, 2), 1, 1, 9, 13),
+    "3x3_stride_2x1": (3, 3, (2, 1), 1, 1, 13, 9),
+    "3x3_stride_3x1": (3, 3, (3, 1), 1, 1, 14, 8),
+    "3x3_dil_2x1": (3, 3, 1, 0, (2, 1), 11, 9),
+    "3x3_dil_2x1_pad_2x1": (3, 3, 1, (2, 1), (2, 1), 10, 9),
+    "3x3_stride4": (3, 3, 4, 1, 1, 17, 15),
+    "3x3_stride8": (3, 3, 8, 1, 1, 30, 27),
+    # windows clipped on both sides of an axis: the image is smaller than the filter's span
+    "3x3_pad1_1x1_image": (3, 3, 1, 1, 1, 1, 1),
+    "3x3_pad1_1xW_image": (3, 3, 1, 1, 1, 1, 9),
+    "5x5_pad2_2x3_image": (5, 5, 1, 2, 1, 2, 3),
+    "3x3_dil3_pad3_2x2_image": (3, 3, 1, 3, 3, 2, 2),       # the middle tap of a window can be the only one inside
+    # the im2col bounding-box corner extremes: -pad = pad - dil*(k-1) = -128 (tap offset 256); pad - dil*(k-1) = 127
+    "3x1_dil128_pad128_corner": (3, 1, 1, (128, 0), (128, 1), 3, 4),
+    "1x1_pad127_stride8_corner": (1, 1, 8, 127, 1, 3, 5),
 }
 
 

@@ -30,19 +30,78 @@ def _bytes_of(codes_int, encoding):
     return codes_int.to(torch.float32).to(torch.float8_e4m3fn).view(torch.uint8)
 
 
-def case_raw_gemm(m, n, k, encoding, a_signed, relu=False, bf16=False, seed=0, a_hi=15, w_hi=7):
-    """random codes -> dlmcq_qgemm vs the integer oracle, bit for bit."""
+PATTERNS = ("random", "saturated", "biased", "cancel")
+TAIL = 48                                    # trailing K entries of the "cancel" pattern: codes +-1, then one 0
+
+
+def act_codes_of(pattern, shape, a_hi, a_signed, g):
+    """Activation codes of a pattern: "random" draws the whole range; "saturated" is a_hi everywhere; "biased" and
+    "cancel" draw the upper half [a_hi // 2 + 1, a_hi] (positive: one sign, so the running sum only grows)."""
+    if pattern == "random":
+        return torch.randint(-a_hi if a_signed else 0, a_hi + 1, shape, generator=g)
+    if pattern == "saturated":
+        return torch.full(shape, a_hi, dtype=torch.int64)
+    return torch.randint(a_hi // 2 + 1, a_hi + 1, shape, generator=g)
+
+
+def wt_codes_of(pattern, n, k, w_hi, g):
+    """[n, k] weight codes of a pattern, K in accumulation order: "saturated" is -w_hi everywhere (|acc| = K * max|a| *
+    max|w|, negative); "biased" draws [w_hi // 2 + 1, w_hi] (odd increments: a constant would add multiples of 32 per
+    MMA step and hide a short accumulator); "cancel" is biased positive over the first half of K, negative over the
+    second, then TAIL - 1 entries of +-1 and one 0, so the exact result is small but needs every bit up to the
+    running sum's peak."""
+    if pattern == "random":
+        return torch.randint(-w_hi, w_hi + 1, (n, k), generator=g)
+    if pattern == "saturated":
+        return torch.full((n, k), -w_hi, dtype=torch.int64)
+    cw = torch.randint(w_hi // 2 + 1, w_hi + 1, (n, k), generator=g)
+    if pattern == "cancel":
+        body = k - TAIL
+        cw[:, body // 2:body] *= -1
+        cw[:, body:] = torch.randint(0, 2, (n, TAIL), generator=g) * 2 - 1
+        cw[:, -1] = 0
+    return cw
+
+
+def blocked_acc(ca, cw, step=16, chunk=64):
+    """acc = ca [m, K] @ cw [n, K]^T accumulated in K order, one K block of `step` at a time (float64: every partial
+    sum is an integer below 2^53, so exact), and the largest |partial sum| at any block boundary."""
+    m, k = ca.shape
+    n = cw.shape[0]
+    a, w = ca.to(torch.float64), cw.to(torch.float64)
+    acc = torch.zeros(m, n, dtype=torch.float64)
+    peak = 0.0
+    for k0 in range(0, k, step * chunk):
+        k1 = min(k, k0 + step * chunk)
+        nb = (k1 - k0) // step
+        blocks = torch.einsum("mbs,nbs->bmn", a[:, k0:k1].reshape(m, nb, step), w[:, k0:k1].reshape(n, nb, step))
+        run = acc + blocks.cumsum(0)
+        peak = max(peak, run.abs().max().item())
+        acc = run[-1]
+    return acc, peak
+
+
+def case_raw_gemm(m, n, k, encoding, a_signed, relu=False, bf16=False, seed=0, a_hi=15, w_hi=7, pattern="random"):
+    """codes of a pattern -> dlmcq_qgemm vs the integer oracle, bit for bit.  The worst-case patterns report K, the
+    largest |acc| and the largest |partial sum| of the exact accumulation in K order."""
     from dlmc_quant_b200 import qgemm as Q
     g = torch.Generator().manual_seed(seed)
-    a_lo = -a_hi if a_signed else 0
-    ca = torch.randint(a_lo, a_hi + 1, (m, k), generator=g)
-    cw = torch.randint(-w_hi, w_hi + 1, (n, k), generator=g)
+    ca = act_codes_of(pattern, (m, k), a_hi, a_signed, g)
+    cw = wt_codes_of(pattern, n, k, w_hi, g)
+    if pattern == "cancel":
+        ca[:, k - TAIL:] = 1                  # the tail adds an odd sum of +-1
     alpha = (torch.rand(n, generator=g) * 0.01 + 1e-3).float()
     beta = torch.randn(n, generator=g).float()
     out = Q.qgemm(_bytes_of(ca, encoding).cuda(), _bytes_of(cw, encoding).cuda(), alpha.cuda(), beta.cuda(), relu=relu,
                   out_dtype=torch.bfloat16 if bf16 else torch.float32, a_signed=a_signed, encoding=encoding)
     torch.cuda.synchronize()
-    want = (ca @ cw.t()).to(torch.float32) * alpha + beta
+    report = {"elements": m * n}
+    if pattern == "random":
+        acc = ca @ cw.t()
+    else:
+        acc, peak = blocked_acc(ca, cw)
+        report.update(K=k, max_abs_acc=int(acc.abs().max().item()), peak_abs_partial_sum=int(peak))
+    want = acc.to(torch.float32) * alpha + beta
     if relu:
         want = torch.relu(want)
     if bf16:
@@ -53,7 +112,7 @@ def case_raw_gemm(m, n, k, encoding, a_signed, relu=False, bf16=False, seed=0, a
         idx = bad.nonzero()[0].tolist()
         raise AssertionError(f"{int(bad.sum())} of {bad.numel()} differ; first at {idx}: got {got[tuple(idx)].item()} "
                              f"want {want[tuple(idx)].item()}")
-    return {"elements": m * n}
+    return report
 
 
 def _mult(form, scale, g):
@@ -375,6 +434,20 @@ def case_errors():
         raise AssertionError("k % 16 != 0 was accepted")
     empty = Q.qgemm(torch.zeros(0, 32, dtype=torch.uint8).cuda(), torch.zeros(8, 32, dtype=torch.uint8).cuda(), al, al)
     assert empty.shape == (0, 8)
+    # the accumulator bound of qgemm_prepare: accepted at K * max|a| * max|w| = 2^24 (e4m3) and at the largest K of
+    # 8-bit codes below 2^31 - 1 (integer kind), refused one K block above
+    act = lambda hi: (torch.ones(1).cuda(), torch.zeros(1).cuda(), 0, hi, A1, 0.0)  # noqa: E731
+    for enc, a_hi, w_hi, k_ok in ((E4M3, 16, 16, 65536), (I8, 255, 127, 66304)):
+        for k, ok in ((k_ok, True), (k_ok + 16, False)):
+            try:
+                Q.qgemm_prepare(torch.zeros(8, k, dtype=torch.uint8).cuda(), act(a_hi), (al, -w_hi, w_hi, SYM, 0.0),
+                                None, enc)
+                accepted = True
+            except DlmcqError as e:
+                assert "unsupported" in str(e), e
+                accepted = False
+            assert accepted == ok, (enc, k)
+    torch.cuda.synchronize()
     return {}
 
 
@@ -398,6 +471,18 @@ def build_cases():
     cases.append(("raw_i8_8bit", case_raw_gemm, dict(m=256, n=128, k=8192, encoding=I8, a_signed=False, a_hi=255, w_hi=127)))
     cases.append(("raw_i8_8bit_signed", case_raw_gemm, dict(m=64, n=48, k=1024, encoding=I8, a_signed=True, a_hi=127,
                                                             w_hi=127)))
+    # worst-case accumulators: the ResNet-50 3x3 layers' K (9 * 64 ... 9 * 512) and 2048 with 4-bit codes on both
+    # kinds; e4m3 at K = 65520 on its extreme codes (|code| = 16: K * 16 * 16 just below 2^24); the integer kind with
+    # 8-bit codes at the largest multiple of 16 with K * 255 * 127 <= 2^31 - 1
+    for pattern in PATTERNS[1:]:
+        for enc, tag in ((I8, "i8"), (E4M3, "e4m3")):
+            for k in (576, 1152, 2048, 2304, 4608):
+                cases.append((f"acc_{tag}_{pattern}_k{k}", case_raw_gemm,
+                              dict(m=136, n=144, k=k, encoding=enc, a_signed=False, pattern=pattern, seed=k)))
+        cases.append((f"acc_e4m3_{pattern}_k65520", case_raw_gemm,
+                      dict(m=128, n=128, k=65520, encoding=E4M3, a_signed=False, a_hi=16, w_hi=16, pattern=pattern)))
+        cases.append((f"acc_i8_8bit_{pattern}_k66304", case_raw_gemm,
+                      dict(m=128, n=128, k=66304, encoding=I8, a_signed=False, a_hi=255, w_hi=127, pattern=pattern)))
     for enc in (I8, E4M3):
         tag = "i8" if enc == I8 else "e4m3"
         cases.append((f"pipe_{tag}_affine", case_pipeline, dict(m=300, n=72, k=256, a_form=AFFINE, w_form=AFFINE, encoding=enc)))

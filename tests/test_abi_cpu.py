@@ -112,6 +112,79 @@ def test_code_gemm_argument_validation_without_gpu(libpath):
     assert h.dlmcq_codes_forward(None, None, ctypes.byref(empty), ctypes.byref(act), 0, None) == 0
 
 
+def test_code_gemm_prepare_refuses_inexact_accumulation(libpath):
+    """dlmcq_qgemm_prepare / dlmcq_qconv_prepare refuse a K whose partial sums can leave the accumulator's exact range:
+    K * max|a| * max|w| above 2^24 for e4m3 (fp32 accumulators), above 2^31 - 1 for the integer kind (s32) - before
+    any CUDA call.  (The accepted side of each bound runs on the GPU: tests/qgemm_cases.py, tests/qconv_cases.py.)"""
+    from dlmc_quant_b200 import _lib
+    from dlmc_quant_b200 import qgemm as Q
+    h = _lib.lib()
+    EUNSUPPORTED = -5
+    one = ctypes.c_void_p(4096)
+    qp = lambda form, lo, hi: _lib.QParams(form, lo, hi, 0.0, one, one if form != 3 else None)  # noqa: E731
+    gemm = lambda k, enc, act, wt: h.dlmcq_qgemm_prepare(one, 8, k, enc, ctypes.byref(act), ctypes.byref(wt), 8, None,  # noqa: E731
+                                                          one, one, None)
+
+    def conv(kh, kw, cin, enc, act, wt):
+        g = Q._geom(1, 1, 1, cin, 8, kh, kw)
+        return h.dlmcq_qconv_prepare(one, ctypes.byref(g), enc, ctypes.byref(act), ctypes.byref(wt), 8, None, one, one,
+                                     None)
+    e4_a, e4_w = qp(1, 0, 16), qp(3, -16, 16)
+    assert 65536 * 16 * 16 == 2 ** 24
+    assert gemm(65552, 1, e4_a, e4_w) == EUNSUPPORTED
+    assert gemm(2 ** 20, 1, qp(2, 0, 15), qp(3, -8, 7)) == EUNSUPPORTED              # 2^20 * 15 * 8 > 2^24
+    assert gemm(139824, 1, qp(1, 0, 15), qp(3, -8, 7)) == EUNSUPPORTED               # 4-bit codes: K <= 139810
+    assert gemm(66320, 0, qp(2, 0, 255), qp(3, -127, 127)) == EUNSUPPORTED           # 8-bit codes: K <= 66311
+    assert gemm(2 ** 40, 0, qp(2, 0, 15), qp(3, -7, 7)) == EUNSUPPORTED
+    assert gemm(132112, 0, qp(3, -127, 127), qp(3, -128, 127)) == EUNSUPPORTED       # max|w| = 128, not 127
+    assert conv(3, 3, 7296, 1, e4_a, e4_w) == EUNSUPPORTED                           # K = 65664 > 2^16
+    assert conv(1, 1, 65600, 1, e4_a, e4_w) == EUNSUPPORTED
+    assert conv(3, 3, 7424, 0, qp(2, 0, 255), qp(3, -127, 127)) == EUNSUPPORTED       # K = 66816
+    assert conv(7, 7, 1408, 0, qp(2, 0, 255), qp(3, -127, 127)) == EUNSUPPORTED       # K = 68992
+    # the Python mirror of the bound, at its edges
+    assert Q.accumulator_exact(Q.QGEMM_E4M3, 65536, 0, 16, -16, 16)
+    assert not Q.accumulator_exact(Q.QGEMM_E4M3, 65537, 0, 16, -16, 16)
+    assert Q.accumulator_exact(Q.QGEMM_I8, 66311, 0, 255, -127, 127)
+    assert not Q.accumulator_exact(Q.QGEMM_I8, 66312, 0, 255, -127, 127)
+    assert Q.accumulator_exact(Q.QGEMM_I8, 131071, -128, 127, -128, 127)
+    assert not Q.accumulator_exact(Q.QGEMM_I8, 131073, -128, 127, -128, 127)
+
+
+def test_code_gemm_encoding_follows_the_accumulator_bound():
+    """enable_code_gemm picks e4m3 only while K * max|a| * max|w| <= 2^24, the integer kind while it is <= 2^31 - 1,
+    and leaves a layer on its original path when neither accumulates its K exactly; a layer switched to an explicit
+    encoding that cannot hold its K keeps its original path too."""
+    import copy
+    import torch
+    from dlmc_quant_b200 import quantize_model
+    from dlmc_quant_b200.qgemm import QGEMM_E4M3, QGEMM_I8, enable_code_gemm
+    nn = torch.nn
+
+    def quantised(bits, *layers):
+        net = nn.Sequential(*layers)
+        cfg = {"weight": {"enable": True, "type": "minmax_channel", "args": {"n_bits": bits, "signed": True, "ch_axis": 0}},
+               "input": {"enable": True, "type": "minmax_tensor", "args": {"n_bits": bits, "signed": False}},
+               "exclude_layers": [], "override_options": [], "momentum": 0.1}
+        quantize_model(net, copy.deepcopy(cfg), None)
+        return net
+    # 4-bit codes: max|a| = 15, max|w| = 7 -> e4m3 up to K = 159783
+    net4 = quantised(4, nn.Linear(159776, 1), nn.Linear(159792, 1), nn.Conv2d(17792, 1, 3, padding=1))
+    assert (net4[0].in_min_val, net4[0].in_max_val, net4[0].wt_min_val, net4[0].wt_max_val) == (0, 15, -7, 7)
+    assert enable_code_gemm(net4, convolutions=True) == ["0", "1", "2"]
+    assert [net4[i].__dict__["_code_gemm"].encoding for i in range(3)] == [QGEMM_E4M3, QGEMM_I8, QGEMM_I8]
+    # 8-bit codes: max|a| = 255, max|w| = 127 -> the integer kind up to K = 66311, then no exact encoding
+    net8 = quantised(8, nn.Linear(66304, 1), nn.Linear(66320, 1), nn.Conv2d(7424, 1, 3, padding=1))
+    assert (net8[0].in_min_val, net8[0].in_max_val, net8[0].wt_min_val, net8[0].wt_max_val) == (0, 255, -127, 127)
+    assert enable_code_gemm(net8, convolutions=True) == ["0"]
+    assert net8[0].__dict__["_code_gemm"].encoding == QGEMM_I8
+    assert all("_code_gemm" not in net8[i].__dict__ and "forward" not in net8[i].__dict__ for i in (1, 2))
+    # explicit encodings: the state refuses what the prepare entry would refuse, so the layer keeps its path
+    for net, enc in ((quantised(4, nn.Linear(159792, 1)), QGEMM_E4M3), (quantised(8, nn.Linear(66320, 1)), QGEMM_I8)):
+        assert enable_code_gemm(net, enc) == ["0"]
+        st = net[0].__dict__["_code_gemm"]
+        assert st.refresh(net[0], net[0].__dict__["_code_gemm_forms"]) is False and st.usable is False
+
+
 def test_code_gemm_module_switch_is_host_logic():
     """enable_code_gemm / disable_code_gemm: which layers qualify (Linear with K % 16 == 0, stride-1 1x1 Conv2d) and
     that switching is reversible - no device needed."""

@@ -49,6 +49,22 @@ def test_e4m3_kind_conv_is_bit_exact(report):
     assert not _failed(report, "raw_e4m3_"), _failed(report, "raw_e4m3_")
 
 
+def test_worst_case_accumulators_are_exact(report):
+    """Saturated, one-sign biased and cancelling codes at the ResNet-50 3x3 layers' K on both kinds, at K = 65088
+    with |code| = 16 on e4m3 and at K = 66240 with 8-bit codes on the integer kind: bit-exact, and each case reached
+    the magnitude it was built for."""
+    acc = {k: v for k, v in report["cases"].items() if k.startswith("acc_")}
+    assert len(acc) == 30, sorted(acc)
+    assert not _failed(report, "acc_"), _failed(report, "acc_")
+    for name, c in acc.items():
+        assert c["peak_abs_partial_sum"] >= c["max_abs_acc"] > 0, (name, c)
+        if "saturated" in name:                                  # interior pixels see every tap
+            hi_a, hi_w = (255, 127) if "8bit" in name else (16, 16) if "k65088" in name else (15, 7)
+            assert c["max_abs_acc"] == c["K"] * hi_a * hi_w, (name, c)
+    assert acc["acc_e4m3_saturated_k65088"]["max_abs_acc"] > 2 ** 24 - 2 ** 17
+    assert acc["acc_i8_8bit_saturated_k66240"]["max_abs_acc"] > 2 ** 31 - 2 ** 22
+
+
 def test_codes_prepare_conv_pipeline(report):
     """fp32 / bf16 x -> codes_forward -> qconv_prepare -> qconv: bit-exact vs the oracle, <= 1e-5 vs the reference."""
     assert not _failed(report, "pipe_"), _failed(report, "pipe_")

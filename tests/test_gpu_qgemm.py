@@ -52,6 +52,23 @@ def test_e4m3_kind_gemm_is_bit_exact(report):
     assert not _failed(report, "raw_e4m3_"), _failed(report, "raw_e4m3_")
 
 
+def test_worst_case_accumulators_are_exact(report):
+    """Saturated, one-sign biased and cancelling codes at the ResNet-50 3x3 layers' K on both kinds, at K = 65520
+    with |code| = 16 on e4m3 (partial sums up to 2^24) and at K = 66304 with 8-bit codes on the integer kind (up to
+    2^31 - 1): bit-exact, and each case reached the magnitude it was built for."""
+    acc = {k: v for k, v in report["cases"].items() if k.startswith("acc_")}
+    assert len(acc) == 36, sorted(acc)
+    assert not _failed(report, "acc_"), _failed(report, "acc_")
+    for name, c in acc.items():
+        assert c["peak_abs_partial_sum"] >= c["max_abs_acc"] > 0, (name, c)
+        if "saturated" in name:
+            hi_a, hi_w = (255, 127) if "8bit" in name else (16, 16) if "k65520" in name else (15, 7)
+            assert c["max_abs_acc"] == c["K"] * hi_a * hi_w, (name, c)
+    assert acc["acc_e4m3_saturated_k65520"]["max_abs_acc"] > 2 ** 24 - 2 ** 13
+    assert acc["acc_i8_8bit_saturated_k66304"]["max_abs_acc"] > 2 ** 31 - 2 ** 19
+    assert acc["acc_e4m3_biased_k65520"]["peak_abs_partial_sum"] > 2 ** 23
+
+
 def test_codes_prepare_gemm_pipeline(report):
     """x, w -> code bytes (== the fake-quant kernels' codes) -> alpha / beta from device qparams -> GEMM: bit-exact
     against the integer oracle, <= 1e-5 relative against the reference product in float64, for the AFFINE, ZP, A1

@@ -5,8 +5,10 @@ image - equals the reference's F.conv2d of the two fake-quantised tensors (float
 A version with the 1x1 rule's whole-K beta must fail that bar at the border: the test sees the border rule."""
 import pytest
 import torch
+import torch.nn.functional as F
 
-from tests.qconv_oracle import A1, AFFINE, GEOMETRIES, SYM, ZP, code_conv, conv_problem, conv_reference
+from tests.qconv_oracle import (A1, AFFINE, GEOMETRIES, SYM, ZP, code_conv, conv_pairs, conv_problem, conv_reference,
+                                exact_conv, exact_conv_acc)
 
 FORMS = [(AFFINE, AFFINE), (AFFINE, SYM), (ZP, SYM), (A1, SYM), (SYM, SYM)]
 
@@ -41,7 +43,7 @@ def test_eight_bit_and_signed_activations(geom):
     assert (got >= 0).all() and err.max().item() <= 1e-5
 
 
-@pytest.mark.parametrize("geom", [g for g in sorted(GEOMETRIES) if GEOMETRIES[g][3] != 0])
+@pytest.mark.parametrize("geom", [g for g in sorted(GEOMETRIES) if any(conv_pairs(*GEOMETRIES[g][2:5])[1])])
 @pytest.mark.parametrize("a_form", [AFFINE, ZP, A1])
 def test_whole_k_beta_fails_at_the_border(geom, a_form):
     """With t = o_a - z_a*m_a != 0 the padded taps would contribute t*m_w*sum(cw) if beta ignored the border; the bar
@@ -49,14 +51,14 @@ def test_whole_k_beta_fails_at_the_border(geom, a_form):
     p = conv_problem(a_form, SYM, GEOMETRIES[geom], seed=7)
     _, err = _err(p, whole_k_beta=True)
     kh, kw, stride, padding, dilation, h, w = GEOMETRIES[geom]
-    ph, pw = (padding, padding) if isinstance(padding, int) else padding
+    (sh, sw), (ph, pw), (dh, dw) = conv_pairs(stride, padding, dilation)
     assert err.max().item() > 1e-3
     # interior pixels (window fully inside) agree with the border-aware form
     ho, wo = err.shape[2], err.shape[3]
-    oh = torch.arange(ho) * stride - ph
-    ow = torch.arange(wo) * stride - pw
-    inside_h = (oh >= 0) & (oh + dilation * (kh - 1) < h)
-    inside_w = (ow >= 0) & (ow + dilation * (kw - 1) < w)
+    oh = torch.arange(ho) * sh - ph
+    ow = torch.arange(wo) * sw - pw
+    inside_h = (oh >= 0) & (oh + dh * (kh - 1) < h)
+    inside_w = (ow >= 0) & (ow + dw * (kw - 1) < w)
     interior = err[:, :, inside_h][:, :, :, inside_w]
     if interior.numel():
         assert interior.max().item() <= 1e-5
@@ -70,6 +72,24 @@ def test_integer_convolution_is_exact():
     want = torch.nn.functional.conv2d(ca.to(torch.int64).double(), cw.double(), padding=1)
     assert want.abs().max() > 2 ** 24                           # the s32 -> fp32 conversion rounds
     assert torch.equal(out, want.float())
+
+
+@pytest.mark.parametrize("geom", sorted(GEOMETRIES))
+def test_tapwise_exact_conv_equals_code_conv(geom):
+    """exact_conv (one float64 matmul per filter tap, the border sums from tap validity; the GPU reference of the
+    batch-128 cases) equals code_conv (float64 conv2d) bit for bit on 8-bit codes, for every geometry."""
+    kh, kw, stride, padding, dilation, h, w = GEOMETRIES[geom]
+    g = torch.Generator().manual_seed(len(geom))
+    ca = torch.randint(0, 256, (2, 64, h, w), generator=g)
+    cw = torch.randint(-127, 128, (5, 64, kh, kw), generator=g)
+    kw_ = dict(stride=stride, padding=padding, dilation=dilation)
+    acc = exact_conv_acc(ca, cw, **kw_)
+    assert torch.equal(acc, F.conv2d(ca.double(), cw.double(), **kw_))
+    m_w = torch.rand(5, generator=g) * 0.01 + 1e-3
+    bias = torch.randn(5, generator=g)
+    for relu in (False, True):
+        args = (ca, cw, torch.tensor(0.0371), torch.tensor(-0.21), torch.tensor(3.0), m_w, bias)
+        assert torch.equal(exact_conv(*args, relu=relu, **kw_), code_conv(*args, relu=relu, **kw_))
 
 
 def test_python_entry_argument_checks_need_no_gpu():
