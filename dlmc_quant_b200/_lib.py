@@ -148,6 +148,8 @@ SIGNATURES = {
     "dlmcq_fold_grouped": (_I, [_P, _P, _I, _L, _P]),
     "dlmcq_bnq_workspace_bytes": (_Z, [C.POINTER(BnqDesc)]),
     "dlmcq_bnq_forward": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.POINTER(BnqDesc), _QP, _P, _Z, _P]),
+    "dlmcq_bnq_forward_codes": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.POINTER(BnqDesc), _QP, _I, _P, _Z,
+                                     _P]),
     "dlmcq_bnq_backward": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.POINTER(BnqDesc), _QP, _P, _Z,
                                 _P]),
     "dlmcq_host_ctx_create": (_I, [C.POINTER(C.c_void_p), _L]),

@@ -24,6 +24,12 @@
 // same `fq_vec<FORM_AFFINE>` code as the stand-alone kernels: given the BatchNorm output `a` (which the kernel
 // can also write), a_q is BIT-IDENTICAL to dlmcq_fq_forward(a) - that is how parity with the reference's
 // quantizer chain is carried over (tests: fused a_q == fq_forward(fused a)).
+//
+// Inference hand-off to the code GEMM (dlmcq_bnq_forward_codes): the apply pass can write the quantizer's CODES, one
+// byte each in the consumer's operand encoding, instead of a_q - the consumer then reads 1 B/elem instead of running
+// its own x -> codes pass over a 4 B/elem a_q.  The codes are the same intermediate a_q is dequantised from, so given a
+// they equal dlmcq_codes_forward(a) byte for byte.
+#include "codes.cuh"
 #include "fq_math.cuh"
 
 namespace dlmcq {
@@ -446,26 +452,51 @@ __device__ __forceinline__ TileLoop make_tile_loop(const BnqGeom& gm, int U, int
 template <typename T, int VN, bool QUANT>
 __device__ __forceinline__ void apply_generic_vec(const float (&fx)[VN], const float* fi, const BnCh<VN>& c, bool relu,
                                                   const ChanParams& p, float lo, float hi, float (&act)[VN],
-                                                  float (&y)[VN]) {
+                                                  float (&y)[VN], float (&code)[VN]) {
   bn_act_vec<VN>(fx, c, fi, relu, act);
   if (QUANT) {
-    float src[VN], code[VN];
+    float src[VN];
 #pragma unroll
     for (int e = 0; e < VN; ++e) src[e] = sizeof(T) == 2 ? to_f32<T>(from_f32<T>(act[e])) : act[e];
     fq_vec<DLMCQ_FORM_AFFINE, VN>(src, p, lo, hi, code, y);
   }
 }
 
-template <typename T, bool HAS_ID, bool QUANT>
+// The VN codes of one thread's vector as VN contiguous bytes of the [rows, C] code matrix (4 B for fp32, 8 B for
+// bf16), stored with q_out's streaming policy.  `idx` is the vector's index in the activation.
+template <int ENC, int VN>
+__device__ __forceinline__ void st_codes(uint8_t* codes, int64_t idx, const float (&code)[VN]) {
+  uint32_t w[VN / 4];
+#pragma unroll
+  for (int i = 0; i < VN / 4; ++i) {
+    w[i] = code_byte<ENC>(code[4 * i]) | (code_byte<ENC>(code[4 * i + 1]) << 8) |
+           (code_byte<ENC>(code[4 * i + 2]) << 16) | (code_byte<ENC>(code[4 * i + 3]) << 24);
+  }
+  uint8_t* p = codes + idx * VN;
+  if (VN == 4) {
+    asm volatile("st.global.L1::no_allocate.u32 [%0], %1;" ::"l"(p), "r"(w[0]) : "memory");
+  } else {
+    asm volatile("st.global.L1::no_allocate.v2.u32 [%0], {%1,%2};" ::"l"(p), "r"(w[0]), "r"(w[VN / 4 - 1]) : "memory");
+  }
+}
+
+// OUT: kBnqOutT writes a_q (T) to q_out; DLMCQ_QGEMM_I8 / DLMCQ_QGEMM_E4M3 write the codes of a_q, one byte each in that
+// encoding, to q_out instead (QUANT must be true) - the quantizer's code, before dequantisation.
+constexpr int kBnqOutT = -1;
+template <typename T, bool HAS_ID, bool QUANT, int OUT = kBnqOutT>
 __global__ void __launch_bounds__(kBnqThreads, 3)
 bnq_apply_kernel(const T* __restrict__ x, const T* __restrict__ idn, const float* __restrict__ gamma,
                  const float* __restrict__ beta, const float* __restrict__ mean, const float* __restrict__ invstd,
-                 T* __restrict__ a_out, T* __restrict__ q_out, BnqGeom gm, int relu, const float* __restrict__ scale,
+                 T* __restrict__ a_out, void* __restrict__ q_out, BnqGeom gm, int relu, const float* __restrict__ scale,
                  const float* __restrict__ offset, float g, float lo, float hi) {
   using V = Vec<T>;
   using raw = typename V::raw;
   constexpr int VN = V::N;
-  constexpr int U = kBnqU;
+  constexpr bool CODES = OUT != kBnqOutT;
+  // bf16 codes: two rows in flight per thread - with four, the 8-wide vectors spill at 80 registers (3 CTAs / SM)
+  constexpr int U = (CODES && VN == 8) ? 2 : kBnqU;
+  static_assert(!CODES || QUANT, "codes are the quantizer's output");
+  uint8_t* cb = static_cast<uint8_t*>(q_out);
   const int tx = static_cast<int>(threadIdx.x) % gm.txw;
   const int ty = static_cast<int>(threadIdx.x) / gm.txw;
   const int col = static_cast<int>(blockIdx.y) * gm.txw + tx;
@@ -502,48 +533,82 @@ bnq_apply_kernel(const T* __restrict__ x, const T* __restrict__ idn, const float
   const bool fast_ok = c2.safe && (!QUANT || k.fast);
   const float floor = relu ? 0.f : -INFINITY;
   while (t < tl.nfull) {
-    float fx[U][VN], fi[U][VN];
-    float m = 0.f;
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      V::unpack(rx[u], fx[u]);
-      m = absmax_vec<VN>(fx[u], m);
-      if (HAS_ID) {
-        V::unpack(ri[u], fi[u]);
-        m = absmax_vec<VN>(fi[u], m);
-      }
-    }
-    if (fast_ok && m <= kBnqSafe) {
+    if constexpr (CODES) {
+      // codes: the fast-path test per vector, so that only one vector is unpacked at a time (registers, see U)
 #pragma unroll
       for (int u = 0; u < U; ++u) {
-        float act[VN], y[VN];
+        float fx[VN], fi[VN], act[VN], y[VN], code[VN];
+        V::unpack(rx[u], fx);
+        float m = absmax_vec<VN>(fx, 0.f);
+        if (HAS_ID) {
+          V::unpack(ri[u], fi);
+          m = absmax_vec<VN>(fi, m);
+        }
+        if (fast_ok && m <= kBnqSafe) {
 #pragma unroll
-        for (int e = 0; e < VN; e += 2) {
-          const float2 tt = __fadd2_rn(make_float2(fx[u][e], fx[u][e + 1]), c2.nmean[e / 2]);
-          float2 z = __ffma2_rn(tt, c2.a[e / 2], c2.b[e / 2]);
-          if (HAS_ID) z = __fadd2_rn(z, make_float2(fi[u][e], fi[u][e + 1]));
-          const float2 a2 = act_pair(z, floor);
-          act[e] = a2.x;
-          act[e + 1] = a2.y;
-          if (QUANT) {
+          for (int e = 0; e < VN; e += 2) {
+            const float2 tt = __fadd2_rn(make_float2(fx[e], fx[e + 1]), c2.nmean[e / 2]);
+            float2 z = __ffma2_rn(tt, c2.a[e / 2], c2.b[e / 2]);
+            if (HAS_ID) z = __fadd2_rn(z, make_float2(fi[e], fi[e + 1]));
+            const float2 a2 = act_pair(z, floor);
+            act[e] = a2.x;
+            act[e + 1] = a2.y;
             float2 q, cc, cd;
             quant_pair(round_to_storage<T>(a2), k, q, cc, cd);
-            const float2 yy = dequant_pair(cd, k);
-            y[e] = yy.x;
-            y[e + 1] = yy.y;
+            code[e] = cd.x;
+            code[e + 1] = cd.y;
           }
+        } else {
+          apply_generic_vec<T, VN, true>(fx, HAS_ID ? fi : nullptr, unpack_bnch<VN>(c2), relu != 0, k.p, lo, hi, act,
+                                         y, code);
         }
-        if (av) av[off + u * tl.du] = V::pack(act);   // re-read by the backward pass / the next block: default L2 policy
-        if (QUANT) st_stream(qv + off + u * tl.du, V::pack(y));
+        if (av) av[off + u * tl.du] = V::pack(act);
+        st_codes<OUT, VN>(cb, off + u * tl.du, code);
       }
     } else {
-      const BnCh<VN> c = unpack_bnch<VN>(c2);
+      float fx[U][VN], fi[U][VN];
+      float m = 0.f;
 #pragma unroll
       for (int u = 0; u < U; ++u) {
-        float act[VN], y[VN];
-        apply_generic_vec<T, VN, QUANT>(fx[u], HAS_ID ? fi[u] : nullptr, c, relu != 0, k.p, lo, hi, act, y);
-        if (av) av[off + u * tl.du] = V::pack(act);
-        if (QUANT) st_stream(qv + off + u * tl.du, V::pack(y));
+        V::unpack(rx[u], fx[u]);
+        m = absmax_vec<VN>(fx[u], m);
+        if (HAS_ID) {
+          V::unpack(ri[u], fi[u]);
+          m = absmax_vec<VN>(fi[u], m);
+        }
+      }
+      if (fast_ok && m <= kBnqSafe) {
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+          float act[VN], y[VN], code[VN];
+#pragma unroll
+          for (int e = 0; e < VN; e += 2) {
+            const float2 tt = __fadd2_rn(make_float2(fx[u][e], fx[u][e + 1]), c2.nmean[e / 2]);
+            float2 z = __ffma2_rn(tt, c2.a[e / 2], c2.b[e / 2]);
+            if (HAS_ID) z = __fadd2_rn(z, make_float2(fi[u][e], fi[u][e + 1]));
+            const float2 a2 = act_pair(z, floor);
+            act[e] = a2.x;
+            act[e + 1] = a2.y;
+            if (QUANT) {
+              float2 q, cc, cd;
+              quant_pair(round_to_storage<T>(a2), k, q, cc, cd);
+              const float2 yy = dequant_pair(cd, k);
+              y[e] = yy.x;
+              y[e + 1] = yy.y;
+            }
+          }
+          if (av) av[off + u * tl.du] = V::pack(act);   // re-read by the backward pass / the next block: default L2 policy
+          if (QUANT) st_stream(qv + off + u * tl.du, V::pack(y));
+        }
+      } else {
+        const BnCh<VN> c = unpack_bnch<VN>(c2);
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+          float act[VN], y[VN], code[VN];
+          apply_generic_vec<T, VN, QUANT>(fx[u], HAS_ID ? fi[u] : nullptr, c, relu != 0, k.p, lo, hi, act, y, code);
+          if (av) av[off + u * tl.du] = V::pack(act);
+          if (QUANT) st_stream(qv + off + u * tl.du, V::pack(y));
+        }
       }
     }
     t += gridDim.x;
@@ -563,12 +628,13 @@ bnq_apply_kernel(const T* __restrict__ x, const T* __restrict__ idn, const float
       const int64_t row = tl.tail_r0 + ty + static_cast<int64_t>(u) * gm.ty;
       if (row >= gm.rows) break;
       const int64_t idx = row * gm.cv + col;
-      float fx[VN], fi[VN], act[VN], y[VN];
+      float fx[VN], fi[VN], act[VN], y[VN], code[VN];
       V::unpack(ld_stream(xv + idx), fx);
       if (HAS_ID) V::unpack(ld_stream(iv + idx), fi);
-      apply_generic_vec<T, VN, QUANT>(fx, HAS_ID ? fi : nullptr, c, relu != 0, k.p, lo, hi, act, y);
+      apply_generic_vec<T, VN, QUANT>(fx, HAS_ID ? fi : nullptr, c, relu != 0, k.p, lo, hi, act, y, code);
       if (av) av[idx] = V::pack(act);
-      if (QUANT) st_stream(qv + idx, V::pack(y));
+      if (CODES) st_codes<OUT, VN>(cb, idx, code);
+      else if (QUANT) st_stream(qv + idx, V::pack(y));
     }
   }
 }
@@ -1073,10 +1139,19 @@ static inline size_t bnq_smem(const BnqGeom& g) {
   return static_cast<size_t>(g.ty) * g.txw * 2 * VN * sizeof(float);
 }
 
+// the apply kernel for one output mode: a_q (out = kBnqOutT) or its codes in encoding `out`
+template <typename T, int OUT>
+static auto bnq_apply_for(bool idn, bool quant) {
+  if (OUT != kBnqOutT) return idn ? bnq_apply_kernel<T, true, true, OUT> : bnq_apply_kernel<T, false, true, OUT>;
+  return idn ? (quant ? bnq_apply_kernel<T, true, true> : bnq_apply_kernel<T, true, false>)
+             : (quant ? bnq_apply_kernel<T, false, true> : bnq_apply_kernel<T, false, false>);
+}
+
+// q_out: a_q (out = kBnqOutT), or the codes in encoding `out` (eval mode only: dlmcq_bnq_forward_codes)
 template <typename T>
 static int bnq_forward_t(const void* x, const void* idn, const float* gamma, const float* beta, float* rmean,
                          float* rvar, float* smean, float* sinv, void* a_out, void* q_out, const dlmcq_bnq_desc* d,
-                         const dlmcq_qparams* qp, void* ws, size_t ws_bytes, cudaStream_t st) {
+                         const dlmcq_qparams* qp, void* ws, size_t ws_bytes, cudaStream_t st, int out = kBnqOutT) {
   constexpr int VN = Vec<T>::N;
   const BnqGeom g = make_bnq_geom<T>(d->rows, d->channels);
   if (ws_bytes < kWsHeaderBytes + bnq_ws_floats(g) * sizeof(float)) return DLMCQ_EWORKSPACE;
@@ -1102,11 +1177,12 @@ static int bnq_forward_t(const void* x, const void* idn, const float* gamma, con
   const float* of = quant ? qp->offset : nullptr;
   const float gq = quant ? qp->g : 0.f;
   const dim3 grid(apply_grid(g, 8), g.gy);
-  auto k = idn ? (quant ? bnq_apply_kernel<T, true, true> : bnq_apply_kernel<T, true, false>)
-               : (quant ? bnq_apply_kernel<T, false, true> : bnq_apply_kernel<T, false, false>);
+  auto k = out == DLMCQ_QGEMM_I8     ? bnq_apply_for<T, DLMCQ_QGEMM_I8>(idn != nullptr, quant)
+           : out == DLMCQ_QGEMM_E4M3 ? bnq_apply_for<T, DLMCQ_QGEMM_E4M3>(idn != nullptr, quant)
+                                     : bnq_apply_for<T, kBnqOutT>(idn != nullptr, quant);
   cudaError_t e = launch_pdl(k, grid, dim3(kBnqThreads), 0, st, xt, static_cast<const T*>(idn), gamma, beta,
                              static_cast<const float*>(smean), static_cast<const float*>(sinv), static_cast<T*>(a_out),
-                             static_cast<T*>(q_out), g, relu, sc, of, gq, lo, hi);
+                             q_out, g, relu, sc, of, gq, lo, hi);
   if (e != cudaSuccess) return set_cuda_error(e);
   return DLMCQ_OK;
 }
@@ -1196,6 +1272,28 @@ extern "C" int dlmcq_bnq_forward(const void* x, const void* identity, const floa
                                     q_out, desc, qp, workspace, workspace_bytes, st)
              : bnq_forward_t<__nv_bfloat16>(x, identity, gamma, beta, running_mean, running_var, save_mean, save_invstd,
                                             a_out, q_out, desc, qp, workspace, workspace_bytes, st);
+}
+
+extern "C" int dlmcq_bnq_forward_codes(const void* x, const void* identity, const float* gamma, const float* beta,
+                                       float* running_mean, float* running_var, float* save_mean, float* save_invstd,
+                                       void* a_out, void* codes_out, const dlmcq_bnq_desc* desc,
+                                       const dlmcq_qparams* qp, int encoding, void* workspace, size_t workspace_bytes,
+                                       void* stream) {
+  if (int e = bnq_check(desc)) return e;
+  if (desc->flags & DLMCQ_BNQ_TRAINING) return DLMCQ_EUNSUPPORTED;      // an inference hand-off: no backward
+  if (!qp || !qp->scale || qp->form != DLMCQ_FORM_AFFINE) return DLMCQ_EINVAL;
+  if (int e = code_range_ok(qp, encoding)) return e;                    // unknown encoding: DLMCQ_EINVAL
+  if (desc->rows == 0) return DLMCQ_OK;
+  if (!x || !codes_out || !save_mean || !save_invstd || !workspace || !running_mean || !running_var) return DLMCQ_EINVAL;
+  if (((desc->flags & DLMCQ_BNQ_RESIDUAL) != 0) != (identity != nullptr)) return DLMCQ_EINVAL;
+  if (!aligned16(x) || !aligned16(identity) || !aligned16(a_out) || !aligned16(codes_out)) return DLMCQ_EALIGN;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  return desc->dtype == DLMCQ_F32
+             ? bnq_forward_t<float>(x, identity, gamma, beta, running_mean, running_var, save_mean, save_invstd, a_out,
+                                    codes_out, desc, qp, workspace, workspace_bytes, st, encoding)
+             : bnq_forward_t<__nv_bfloat16>(x, identity, gamma, beta, running_mean, running_var, save_mean,
+                                            save_invstd, a_out, codes_out, desc, qp, workspace, workspace_bytes, st,
+                                            encoding);
 }
 
 extern "C" int dlmcq_bnq_backward(const void* x, const void* a_saved, const void* d_a, const void* d_q,

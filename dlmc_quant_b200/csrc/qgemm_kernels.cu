@@ -29,6 +29,7 @@
 #include <cuda.h>       // CUtensorMap + enums only; the encoder is fetched through cudaGetDriverEntryPoint
 #include <cuda_fp8.h>
 
+#include "codes.cuh"
 #include "fq_math.cuh"
 
 namespace dlmcq {
@@ -504,16 +505,8 @@ qconv_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// x -> one byte per code
+// x -> one byte per code (code_byte: codes.cuh)
 // ---------------------------------------------------------------------------------------------------------------
-template <int ENC>
-__device__ __forceinline__ uint32_t code_byte(float code) {
-  if (ENC == DLMCQ_QGEMM_E4M3)                                   // exact: the caller guarantees |code| <= 16
-    return static_cast<uint32_t>(__nv_cvt_float_to_fp8(code == code ? code : 0.f, __NV_SATFINITE, __NV_E4M3));
-  const int c = (code == code) ? static_cast<int>(code) : 0;     // NaN code -> 0 (as dlmcq_export_codes)
-  return static_cast<uint32_t>(c) & 0xFFu;
-}
-
 // per-tensor, 16-byte aligned: every thread turns 16 elements into one 16-byte store (the arithmetic is fq_vec,
 // i.e. bit-identical codes to dlmcq_fq_forward)
 template <int FORM, typename T, int ENC>
@@ -598,13 +591,6 @@ int codes_form(const void* x, void* out, const dlmcq_layout* l, const dlmcq_qpar
     case DLMCQ_FORM_SYM: return codes_launch<DLMCQ_FORM_SYM, T, ENC>(x, out, l, qp, st);
   }
   return DLMCQ_EINVAL;
-}
-
-int code_range_ok(const dlmcq_qparams* qp, int encoding) {
-  if (encoding == DLMCQ_QGEMM_E4M3) return (qp->lo >= -16 && qp->hi <= 16) ? DLMCQ_OK : DLMCQ_EUNSUPPORTED;
-  if (encoding != DLMCQ_QGEMM_I8) return DLMCQ_EINVAL;
-  if (qp->lo < -128 || qp->hi > 255 || (qp->lo < 0 && qp->hi > 127)) return DLMCQ_EUNSUPPORTED;
-  return DLMCQ_OK;
 }
 
 // Exactness of the accumulation: every partial sum of k products is at most k * max|a| * max|w|.  The fp32

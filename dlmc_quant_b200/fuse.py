@@ -26,6 +26,7 @@ from torch import nn
 
 from . import _lib
 from . import functional as F
+from . import qgemm
 from ._lib import BNQ_RELU, BNQ_RESIDUAL, BNQ_TRAINING, FORM_AFFINE, BnqDesc, QParams
 from .scalar.modules.base import QBase
 
@@ -184,6 +185,36 @@ def bn_act_quant(x, bn, consumer=None, identity=None, relu=True, want_plain=Fals
                                     want_plain or identity is not None)
 
 
+def _bn_act_codes(x, bn, consumer, identity, relu, want_plain):
+    """Inference hand-off to the code GEMM: (a | None, codes) with codes = the consumer's input codes of
+    a = relu(bn(x) + identity), one byte each in the consumer's operand encoding (dlmcq_bnq_forward_codes), when the
+    fused kernels take x and `consumer` runs on codes in this call (qgemm.code_input_spec); else None."""
+    if consumer is None or not fusable(x, bn, identity) or bn.training or bn.running_mean is None:
+        return None
+    cq = _consumer_q(consumer, x)
+    if cq is None:
+        return None
+    spec = qgemm.code_input_spec(consumer, x.numel(), x.dtype, x.dim())
+    if spec is None:
+        return None
+    encoding, g = spec
+    scale, (offset, lo, hi, _) = cq
+    rows, ch = _rows_channels(x)
+    flags = (BNQ_RELU if relu else 0) | (BNQ_RESIDUAL if identity is not None else 0)
+    desc = BnqDesc(rows, ch, F._dtype_code(x), flags, float(bn.eps), float(bn.momentum))
+    stats = torch.empty(2, ch, dtype=torch.float32, device=x.device)          # save_mean, save_invstd
+    a = torch.empty_like(x) if want_plain else None
+    codes = torch.empty_like(x, dtype=torch.uint8)     # x's memory format: [rows, C] bytes
+    qp = QParams(FORM_AFFINE, int(lo), int(hi), float(g), scale.data_ptr(), offset.data_ptr())
+    with F._on(x.device):
+        ws, n = _bnq_ws(x.device, desc)
+        _lib.check(_lib.lib().dlmcq_bnq_forward_codes(
+            F._ptr(x), F._ptr(identity), F._ptr(bn.weight), F._ptr(bn.bias), F._ptr(bn.running_mean),
+            F._ptr(bn.running_var), stats.data_ptr(), stats.data_ptr() + 4 * ch, F._ptr(a), F._ptr(codes),
+            C.byref(desc), C.byref(qp), int(encoding), F._ptr(ws), n, F._stream_ptr()))
+    return a, codes
+
+
 def _feed(consumer, a, aq):
     """Run the consumer layer on the fused op's result."""
     if aq is not None:
@@ -192,14 +223,24 @@ def _feed(consumer, a, aq):
 
 
 def bn_act_into(x, bn, consumer, relu=True):
-    """consumer(fake_quant(relu(bn(x)))) with the first three stages fused."""
+    """consumer(fake_quant(relu(bn(x)))) with the first three stages fused; a consumer switched to the code GEMM is
+    handed its input codes instead of the fake-quantised tensor."""
+    r = _bn_act_codes(x, bn, consumer, None, relu, want_plain=False)
+    if r is not None:
+        return qgemm.forward_codes(consumer, r[1], x.dtype)
     a, aq = bn_act_quant(x, bn, consumer, None, relu, want_plain=False)
     return _feed(consumer, a, aq)
 
 
 def bn_add_act(x, bn, identity, next_consumer=None, relu=True):
     """relu(bn(x) + identity) as a plain tensor; when `next_consumer` is a ready quantised layer its input fake-quant
-    is produced by the same kernel and travels with the tensor (`_dlmcq_q`), where QBase.forward picks it up."""
+    is produced by the same kernel and travels with the tensor (`_dlmcq_q`), where QBase.forward picks it up - or, when
+    the layer runs on the code GEMM, its input codes (`_dlmcq_codes`), which the code path picks up."""
+    r = _bn_act_codes(x, bn, next_consumer, identity, relu, want_plain=True)
+    if r is not None:
+        a, codes = r
+        a._dlmcq_codes = (next_consumer, codes)
+        return a
     a, aq = bn_act_quant(x, bn, next_consumer, identity, relu, want_plain=True)
     if aq is not None:
         a._dlmcq_q = (next_consumer, aq)

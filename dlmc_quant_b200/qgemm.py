@@ -301,46 +301,74 @@ class _CodeGemmState:
         return self.alpha, self.beta
 
 
-def _code_forward(self, input):
-    st = self.__dict__.get('_code_gemm')
-    forms = self.__dict__.get('_code_gemm_forms')
+def _code_state(mod, dtype, dim):
+    """The layer's _CodeGemmState when this call runs on the code path, else None: a switched, enabled and initialised
+    layer in eval mode without autograd, an input it serves, and qparams the state finds usable."""
+    st = mod.__dict__.get('_code_gemm')
     # inference only: under autograd the layer keeps the differentiable fake-quant path
-    if (st is None or self.training or torch.is_grad_enabled() or not input.is_cuda
-            or input.dtype not in (torch.float32, torch.bfloat16) or not _enabled(self)
-            or not (self._ready('in', self.in_init_state) and self._ready('wt', self.wt_init_state))):
+    if (st is None or mod.training or torch.is_grad_enabled() or dtype not in (torch.float32, torch.bfloat16)
+            or not _enabled(mod) or not (mod._ready('in', mod.in_init_state) and mod._ready('wt', mod.wt_init_state))):
+        return None
+    if isinstance(mod, nn.Conv2d) and dim != 4:
+        return None
+    return st if st.refresh(mod, mod.__dict__['_code_gemm_forms']) else None
+
+
+def code_input_spec(consumer, numel, dtype, dim):
+    """(encoding, g) when `consumer` - a layer switched by enable_code_gemm - takes its input of `numel` elements as
+    codes in this call: the operand encoding and the AFFINE quantizer's grad_scale factor g = 1/sqrt(numel * qmax)
+    (modules/base.py:96) its own x -> codes pass would use.  None otherwise (the layer then quantises what it is
+    given).  Producers that can emit the codes themselves (fuse.py) ask this before every call."""
+    st = _code_state(consumer, dtype, dim)
+    if st is None or consumer.__dict__['_code_gemm_forms'][0] != FORM_AFFINE:
+        return None
+    return st.encoding, 1 / math.sqrt(numel * consumer.in_max_val)
+
+
+def forward_codes(mod, a_codes, out_dtype):
+    """The switched layer on its input's codes (uint8, the input's shape: [..., K] for Linear, an NCHW view of
+    channels-last [B, H, W, Cin] storage for Conv2d), in the encoding of the layer's state.  Call only when
+    `code_input_spec` (or `_code_state`) accepted the layer for this input."""
+    st = mod.__dict__['_code_gemm']
+    mod.__dict__.pop('_wq', None)                        # a weight group's pre-hook may have staged its copy: unused here
+    alpha, beta = st.epilogue(mod, mod.__dict__['_code_gemm_forms'], a_codes.numel())
+    if st.conv:
+        out = qconv(a_codes.permute(0, 2, 3, 1), st.w_codes, alpha, beta, mod.stride, mod.padding, mod.dilation,
+                    out_dtype=out_dtype, a_signed=mod.in_min_val < 0, encoding=st.encoding)
+        return out.permute(0, 3, 1, 2)                           # NCHW view of channels-last storage
+    n = mod.weight.shape[0]
+    if isinstance(mod, nn.Conv2d):
+        b, k, h, w = a_codes.shape
+        # elementwise codes keep x's memory order: channels-last NCHW storage is the [B*H*W, C] matrix
+        out = qgemm(a_codes.permute(0, 2, 3, 1).reshape(b * h * w, k), st.w_codes, alpha, beta, out_dtype=out_dtype,
+                    a_signed=mod.in_min_val < 0, encoding=st.encoding)
+        return out.view(b, h, w, n).permute(0, 3, 1, 2)          # NCHW view of channels-last storage
+    k = a_codes.shape[-1]
+    out = qgemm(a_codes.reshape(-1, k), st.w_codes, alpha, beta, out_dtype=out_dtype, a_signed=mod.in_min_val < 0,
+                encoding=st.encoding)
+    return out.view(*a_codes.shape[:-1], n)
+
+
+def _code_forward(self, input):
+    st = _code_state(self, input.dtype, input.dim()) if input.is_cuda else None
+    if st is None:
         return self._code_gemm_orig_forward(input)
-    if getattr(input, '_dlmcq_q', None) is not None:
+    pre = getattr(input, '_dlmcq_codes', None)           # (consumer, codes) from a fused producer (fuse.py)
+    if pre is not None and pre[0] is self:
+        return forward_codes(self, pre[1], input.dtype)
+    pre = getattr(input, '_dlmcq_q', None)
+    if pre is not None and pre[0] is self:
         return self._code_gemm_orig_forward(input)      # a fused producer already handed over the fake-quantised tensor
-    if not st.refresh(self, forms):
-        return self._code_gemm_orig_forward(input)
-    a_form, _ = forms
-    self.__dict__.pop('_wq', None)                       # a weight group's pre-hook may have staged its copy: unused here
+    a_form, _ = self.__dict__['_code_gemm_forms']
     if isinstance(self, nn.Conv2d):
-        if input.dim() != 4:
-            return self._code_gemm_orig_forward(input)
-        b, c, h, w = input.shape
         x = input if input.is_contiguous(memory_format=torch.channels_last) else \
             input.contiguous(memory_format=torch.channels_last)
-        rows = b * h * w
     else:
         x = input if input.is_contiguous() else input.contiguous()
-        rows = x.numel() // x.shape[-1]
-    numel = x.numel()
-    alpha, beta = st.epilogue(self, forms, numel)
+    st.epilogue(self, self.__dict__['_code_gemm_forms'], x.numel())
     a_codes = codes_forward(x, self.in_scale.detach().reshape(-1), self.in_offset, self.in_min_val, self.in_max_val,
                             a_form, st._g_a, encoding=st.encoding)
-    if st.conv:
-        out = qconv(a_codes.permute(0, 2, 3, 1), st.w_codes, alpha, beta, self.stride, self.padding, self.dilation,
-                    out_dtype=input.dtype, a_signed=self.in_min_val < 0, encoding=st.encoding)
-        return out.permute(0, 3, 1, 2)                           # NCHW view of channels-last storage
-    k = self.weight.shape[1] if isinstance(self, nn.Conv2d) else self.weight.shape[-1]
-    # elementwise codes keep x's memory order: channels-last NCHW storage is the [B*H*W, C] matrix
-    a2 = a_codes.permute(0, 2, 3, 1).reshape(rows, k) if isinstance(self, nn.Conv2d) else a_codes.reshape(rows, k)
-    out = qgemm(a2, st.w_codes, alpha, beta, out_dtype=input.dtype, a_signed=self.in_min_val < 0, encoding=st.encoding)
-    n = self.weight.shape[0]
-    if isinstance(self, nn.Conv2d):
-        return out.view(b, h, w, n).permute(0, 3, 1, 2)          # NCHW view of channels-last storage
-    return out.view(*input.shape[:-1], n)
+    return forward_codes(self, a_codes, input.dtype)
 
 
 def accumulator_exact(encoding, k, a_lo, a_hi, w_lo, w_hi):

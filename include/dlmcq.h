@@ -458,6 +458,20 @@ int dlmcq_bnq_backward(const void* x, const void* a_saved, const void* d_a, cons
                        void* dx, void* dz_out, float* dgamma, float* dbeta, float* dscale,
                        const dlmcq_bnq_desc* desc, const dlmcq_qparams* qp, void* workspace,
                        size_t workspace_bytes, void* stream);
+/* dlmcq_bnq_forward_codes: the eval-mode forward of dlmcq_bnq_forward that hands the consumer layer its input as
+ * INTEGER CODES for the code GEMM (dlmcq_qgemm / dlmcq_qconv below) instead of the fake-quantised tensor:
+ *     codes = the code of every element of a_q (modules/base.py:96-102: clamp(round((a - offset) / s'))), one byte each
+ *             in the operand encoding `encoding` (DLMCQ_QGEMM_I8 / DLMCQ_QGEMM_E4M3), NaN -> 0
+ * codes_out is a [rows, channels] byte matrix (16-byte aligned); a_out (optional, may be NULL) is written exactly as
+ * dlmcq_bnq_forward writes it, and so are save_mean / save_invstd.  Given a, codes_out is bit-identical to
+ * dlmcq_codes_forward(a) with the same qp and encoding.  Eval mode only (running buffers required): codes have no
+ * backward.  Refused before any CUDA call: DLMCQ_BNQ_TRAINING (DLMCQ_EUNSUPPORTED); codes_out NULL, qp missing or not
+ * FORM_AFFINE, an unknown encoding (DLMCQ_EINVAL); a code range the encoding cannot hold (DLMCQ_EUNSUPPORTED, as
+ * dlmcq_codes_forward); a misaligned pointer (DLMCQ_EALIGN). */
+int dlmcq_bnq_forward_codes(const void* x, const void* identity, const float* gamma, const float* beta,
+                            float* running_mean, float* running_var, float* save_mean, float* save_invstd,
+                            void* a_out, void* codes_out, const dlmcq_bnq_desc* desc, const dlmcq_qparams* qp,
+                            int encoding, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- host-buffer entries (end-to-end path), on a caller-owned context ----------------------
  * For callers whose tensors live in (pinned) HOST memory: per-tensor-scale fake-quant forward + backward with the
