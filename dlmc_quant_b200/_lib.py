@@ -82,6 +82,12 @@ class ConvGeom(C.Structure):
                                           "groups")])
 
 
+class BnqTail(C.Structure):
+    _fields_ = [("gamma", C.c_void_p), ("beta", C.c_void_p), ("running_mean", C.c_void_p), ("running_var", C.c_void_p),
+                ("eps", C.c_float), ("relu", C.c_int32), ("inter_dtype", C.c_int32), ("qp", C.POINTER(QParams)),
+                ("encoding", C.c_int32)]
+
+
 class DlmcqError(RuntimeError):
     pass
 
@@ -162,6 +168,8 @@ SIGNATURES = {
     "dlmcq_qgemm": (_I, [_P, _P, _P, _P, _P, _L, _L, _L, _I, _I, _I, _I, _P]),
     "dlmcq_qconv_prepare": (_I, [_P, C.POINTER(ConvGeom), _I, _QP, _QP, _L, _P, _P, _P, _P]),
     "dlmcq_qconv": (_I, [_P, _P, _P, _P, _P, C.POINTER(ConvGeom), _I, _I, _I, _I, _P]),
+    "dlmcq_qgemm_codes": (_I, [_P, _P, _P, _P, _P, _L, _L, _L, _I, _I, C.POINTER(BnqTail), _P]),
+    "dlmcq_qconv_codes": (_I, [_P, _P, _P, _P, _P, C.POINTER(ConvGeom), _I, _I, C.POINTER(BnqTail), _P]),
 }
 
 

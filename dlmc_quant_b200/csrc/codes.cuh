@@ -17,6 +17,11 @@ __device__ __forceinline__ uint32_t code_byte(float code) {
   return static_cast<uint32_t>(c) & 0xFFu;
 }
 
+// the same byte, the encoding chosen at run time (the code GEMM epilogue: one kernel serves both consumer encodings)
+__device__ __forceinline__ uint32_t code_byte_rt(float code, int encoding) {
+  return encoding == DLMCQ_QGEMM_E4M3 ? code_byte<DLMCQ_QGEMM_E4M3>(code) : code_byte<DLMCQ_QGEMM_I8>(code);
+}
+
 // Can `encoding` hold every code of [qp->lo, qp->hi]?  DLMCQ_EINVAL for an unknown encoding.
 inline int code_range_ok(const dlmcq_qparams* qp, int encoding) {
   if (encoding == DLMCQ_QGEMM_E4M3) return (qp->lo >= -16 && qp->hi <= 16) ? DLMCQ_OK : DLMCQ_EUNSUPPORTED;

@@ -29,8 +29,10 @@
 #include <cuda.h>       // CUtensorMap + enums only; the encoder is fetched through cudaGetDriverEntryPoint
 #include <cuda_fp8.h>
 
+#include <type_traits>
+
+#include "bnq_math.cuh"
 #include "codes.cuh"
-#include "fq_math.cuh"
 
 namespace dlmcq {
 namespace {
@@ -342,15 +344,165 @@ __device__ __forceinline__ void epilogue_loop(uint32_t tmem, uint32_t bar_acc_fu
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Code-output epilogue (dlmcq_qgemm_codes / dlmcq_qconv_codes).  The layer output v = RN(RN(acc * alpha[n]) + beta),
+// rounded to T (what the unchained layer stores), goes on through the consumer's eval BatchNorm, the optional ReLU
+// and the consumer's AFFINE input quantizer, and only the code byte is stored: element for element the arithmetic of
+// bnq_apply_kernel<T, false, true, ENC> (bnq_math.cuh) - the packed fast path under the same domain guard, the
+// literal chain for vectors outside it.  BatchNorm is NOT folded into alpha / beta: that would change the roundings.
+// Layout: a lane owns one output row of a 32-column piece (the layout tcgen05.ld delivers), so its 32 code bytes are
+// one 32-byte sector and no transpose is needed.  The warp's transpose buffer holds the per-column constants instead,
+// staged once per tile and read as warp-wide broadcasts.
+// ---------------------------------------------------------------------------------------------------------------
+struct CodeTail {
+  const float* gamma;
+  const float* beta;
+  const float* mean;       // running_mean
+  const float* var;        // running_var
+  const float* scale;      // consumer's quantizer
+  const float* offset;
+  float eps, g, lo, hi;
+  int relu, enc;
+};
+constexpr int kCstBeta = 4 * 64;          // floats: 64 x float4 {alpha, mean, gamma*invstd, bn beta}, then 64 x beta
+
+// The 64 columns col0 .. col0+63 of this warp's tile; returns whether their BatchNorm constants lie in the fast-path
+// domain (c2.safe of bnq_apply_kernel).
+template <bool CONV>
+__device__ __forceinline__ bool stage_code_consts(float* stg, const float* __restrict__ alpha,
+                                                  const float* __restrict__ beta, const CodeTail& t, int col0,
+                                                  int lane, int N) {
+  __syncwarp();                                                 // every lane is done with the previous tile's
+  float m = 0.f;
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const int j = lane + 32 * h, col = col0 + j;
+    float4 c = make_float4(0.f, 0.f, 0.f, 0.f);
+    float be = 0.f;
+    if (col < N) {
+      c.x = __ldg(alpha + col);
+      c.y = __ldg(t.mean + col);
+      c.z = bn_scale(t.gamma ? __ldg(t.gamma + col) : 1.f, bn_eval_invstd(__ldg(t.var + col), t.eps));
+      c.w = t.beta ? __ldg(t.beta + col) : 0.f;
+      if (!CONV) be = __ldg(beta + col);
+      m = fmaxf(m, fmaxf(fmaxf(fabsf(c.y), fabsf(c.z)), fabsf(c.w)));   // NaN constants flow through, as there
+    }
+    reinterpret_cast<float4*>(stg)[j] = c;
+    if (!CONV) stg[kCstBeta + j] = be;
+  }
+  const bool safe = __all_sync(0xffffffffu, m <= kBnqSafe);
+  __syncwarp();
+  return safe;
+}
+
+// One 32-column piece of row `row` (this lane): columns col .. col+31 (col + 16 >= N: only the first 16 exist, N % 16
+// == 0), constants at cbase .. cbase+31 of the staging buffer; CONV: brow = the row's border-class beta row + col.
+template <bool IS_INT, bool CONV, typename T>
+__device__ __forceinline__ void code_piece(const uint32_t (&v)[32], const float* stg, int cbase, int row, int col, int M,
+                                           int N, const float* __restrict__ brow, const QuantK& k, bool fast_ok,
+                                           float floor, const CodeTail& t, uint8_t* __restrict__ out) {
+  uint32_t w[8];
+#pragma unroll
+  for (int j = 0; j < 32; j += 4) {
+    float4 c[4];
+    float x[4], code[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      c[e] = reinterpret_cast<const float4*>(stg)[cbase + j + e];
+      const float be = CONV ? (col + j + e < N ? __ldg(brow + j + e) : 0.f) : stg[kCstBeta + cbase + j + e];
+      x[e] = to_f32<T>(from_f32<T>(__fadd_rn(__fmul_rn(acc_value<IS_INT>(v[j + e]), c[e].x), be)));
+    }
+    if (fast_ok && absmax_vec<4>(x, 0.f) <= kBnqSafe) {
+#pragma unroll
+      for (int e = 0; e < 4; e += 2) {
+        const float2 tt = __fadd2_rn(make_float2(x[e], x[e + 1]), make_float2(-c[e].y, -c[e + 1].y));
+        const float2 z = __ffma2_rn(tt, make_float2(c[e].z, c[e + 1].z), make_float2(c[e].w, c[e + 1].w));
+        float2 q, cc, cd;
+        quant_pair(round_to_storage<T>(act_pair(z, floor)), k, q, cc, cd);
+        code[e] = cd.x;
+        code[e + 1] = cd.y;
+      }
+    } else {
+      BnCh<4> bc;
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        bc.mean[e] = c[e].y;
+        bc.a[e] = c[e].z;
+        bc.b[e] = c[e].w;
+        bc.istd[e] = 0.f;                                       // not read by the forward
+      }
+      float act[4], y[4];
+      apply_generic_vec<T, 4, true>(x, nullptr, bc, t.relu != 0, k.p, k.lo, k.hi, act, y, code);
+    }
+    w[j / 4] = code_byte_rt(code[0], t.enc) | (code_byte_rt(code[1], t.enc) << 8) |
+               (code_byte_rt(code[2], t.enc) << 16) | (code_byte_rt(code[3], t.enc) << 24);
+  }
+  if (row < M) {
+    uint8_t* p = out + static_cast<size_t>(row) * N + col;
+    asm volatile("st.global.L1::no_allocate.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(w[0]), "r"(w[1]), "r"(w[2]),
+                 "r"(w[3])
+                 : "memory");
+    if (col + 16 < N)
+      asm volatile("st.global.L1::no_allocate.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p + 16), "r"(w[4]), "r"(w[5]),
+                   "r"(w[6]), "r"(w[7])
+                   : "memory");
+  }
+  __syncwarp();
+}
+
+// The tile loop of one epilogue warp for the code output: the same groups, TMEM reads and buffer hand-back as
+// epilogue_loop.
+template <bool IS_INT, bool CONV, typename T>
+__device__ __forceinline__ void code_epilogue_loop(uint32_t tmem, uint32_t bar_acc_full, uint32_t bar_acc_empty,
+                                                   float* stg, int lane, int q, int grp, int chalf, int num_tiles,
+                                                   int tiles_n, int M, int N, const float* __restrict__ alpha,
+                                                   const float* __restrict__ beta, uint8_t* __restrict__ out,
+                                                   const ConvArgs& cv, const CodeTail& t) {
+  const uint32_t full = bar_acc_full + 8 * grp, empty = bar_acc_empty + 8 * grp;
+  const uint32_t tbase = tmem + grp * kBN + (static_cast<uint32_t>(q * 32) << 16) + static_cast<uint32_t>(chalf * 64);
+  const QuantK k = make_quantk(t.scale, t.offset, t.g, t.lo, t.hi);
+  const float floor = t.relu ? 0.f : -INFINITY;
+  uint32_t ti = grp;
+  for (int tile = blockIdx.x + grp * gridDim.x; tile < num_tiles; tile += 2 * gridDim.x, ti += 2) {
+    const int m0 = (tile / tiles_n) * kBM, n0 = (tile % tiles_n) * kBN;
+    const int col0 = n0 + chalf * 64, row0 = m0 + q * 32, row = row0 + lane;
+    const bool has0 = col0 < N, has1 = col0 + 32 < N;            // warp-uniform
+    const bool fast_ok = stage_code_consts<CONV>(stg, alpha, beta, t, col0, lane, N) && k.fast;
+    const float* brow = CONV ? beta + conv_beta_offset(cv, row, N) + col0 : nullptr;
+    mbar_wait(full, (ti >> 1) & 1);
+    tc_fence_after();
+    uint32_t v[32];
+    if (has0) tmem_ld32(tbase, v);
+    if (!has1) {
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(empty);
+    }
+    if (has0 && row0 < M) code_piece<IS_INT, CONV, T>(v, stg, 0, row, col0, M, N, brow, k, fast_ok, floor, t, out);
+    if (has1) {
+      tmem_ld32(tbase + 32, v);
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(empty);
+      if (row0 < M)
+        code_piece<IS_INT, CONV, T>(v, stg, 32, row, col0 + 32, M, N, CONV ? brow + 32 : nullptr, k, fast_ok, floor, t,
+                                    out);
+    }
+  }
+}
+
 // The kernel body, shared by the GEMM (CHUNK = 0: A is a [M, K] matrix, 128-byte K blocks) and the implicit-GEMM
 // convolution (CHUNK = 128 / 64: A is the im2col view of channels-last codes; one K block = one filter tap x CHUNK
 // channels, K = kh*kw*Cin in (r, s, c) order, so B is the [n, K] matrix of channels-last weight codes and a K block
 // never straddles a tap).  Only the A producer, the K-block width and the epilogue's beta differ.
-template <int KIND, int CHUNK>
+// CT = void: out is the layer output (fp32 / bf16); CT = float / __nv_bfloat16: out is the consumer's code bytes
+// (code_epilogue_loop with *tail), CT being the dtype of the layer output the codes are computed from.
+template <int KIND, int CHUNK, typename CT = void>
 __device__ __forceinline__ void gemm_pipeline(const CUtensorMap* map_a, const CUtensorMap* map_b,
                                               const float* __restrict__ alpha, const float* __restrict__ beta,
                                               void* __restrict__ out, int M, int N, int K, uint32_t idesc, int relu,
-                                              int out_bf16, int vec_ok, const ConvArgs& cv) {
+                                              int out_bf16, int vec_ok, const ConvArgs& cv,
+                                              const CodeTail* tail = nullptr) {
   constexpr int kKb = CHUNK == 0 ? kBK : CHUNK;                 // K bytes per block
   constexpr uint32_t kTx = CHUNK == 0 ? kStageBytes : 2 * kBM * CHUNK;
   extern __shared__ uint8_t smem_raw[];
@@ -465,6 +617,10 @@ __device__ __forceinline__ void gemm_pipeline(const CUtensorMap* map_a, const CU
     const int grp = ew >> 3;                                    // accumulator buffer / tile parity this warp serves
     const int chalf = (ew >> 2) & 1;                            // which 64 of the tile's 128 columns
     float* const stg = stg_all + ew * (32 * kStgPitch);
+    if constexpr (!std::is_void<CT>::value) {
+      code_epilogue_loop<IS_INT, CHUNK != 0, CT>(tmem, bar_acc_full, bar_acc_empty, stg, lane, q, grp, chalf, num_tiles,
+                                                 tiles_n, M, N, alpha, beta, static_cast<uint8_t*>(out), cv, *tail);
+    } else {
     const float floor = relu ? 0.f : __int_as_float(0xff800000);
     if (vec_ok && !out_bf16)
       epilogue_loop<IS_INT, 1, CHUNK != 0>(tmem, bar_acc_full, bar_acc_empty, stg, lane, q, grp, chalf, num_tiles, tiles_n, M, N,
@@ -475,6 +631,7 @@ __device__ __forceinline__ void gemm_pipeline(const CUtensorMap* map_a, const CU
     else
       epilogue_loop<IS_INT, 0, CHUNK != 0>(tmem, bar_acc_full, bar_acc_empty, stg, lane, q, grp, chalf, num_tiles, tiles_n, M, N,
                                alpha, beta, out, floor, out_bf16, cv);
+    }
   }
   tc_fence_before();
   __syncthreads();
@@ -502,6 +659,16 @@ qconv_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ 
              const float* __restrict__ alpha, const float* __restrict__ beta, void* __restrict__ out, int M, int N,
              int K, uint32_t idesc, int relu, int out_bf16, int vec_ok, const ConvArgs cv) {
   gemm_pipeline<KIND, CHUNK>(&map_a, &map_b, alpha, beta, out, M, N, K, idesc, relu, out_bf16, vec_ok, cv);
+}
+
+// Code output: out is the [M, N] byte matrix of the consumer's codes (code_epilogue_loop); CHUNK = 0 for the GEMM,
+// 128 / 64 for the convolution (map_a, beta and cv as in qconv_kernel); T = the dtype of the unchained layer output.
+template <int KIND, int CHUNK, typename T>
+__global__ void __launch_bounds__(kGemmThreads, 1)
+qchain_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
+              const float* __restrict__ alpha, const float* __restrict__ beta, uint8_t* __restrict__ out, int M, int N,
+              int K, uint32_t idesc, const ConvArgs cv, const __grid_constant__ CodeTail tail) {
+  gemm_pipeline<KIND, CHUNK, T>(&map_a, &map_b, alpha, beta, out, M, N, K, idesc, 0, 0, 0, cv, &tail);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -830,6 +997,63 @@ int conv_launch(const CUtensorMap& ma, const CUtensorMap& mb, const float* alpha
   return DLMCQ_OK;
 }
 
+template <int KIND, int CHUNK, typename T>
+int chain_launch(const CUtensorMap& ma, const CUtensorMap& mb, const float* alpha, const float* beta, void* out, int m,
+                 int n, int k, const ConvArgs& cv, int a_signed, const CodeTail& t, cudaStream_t st) {
+  static bool opted_in[64] = {};
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) dev = 0;
+  if (dev < 0 || dev >= 64 || !opted_in[dev]) {
+    const cudaError_t e = cudaFuncSetAttribute(qchain_kernel<KIND, CHUNK, T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               static_cast<int>(kGemmSmem));
+    if (e != cudaSuccess) return set_cuda_error(e);
+    if (dev >= 0 && dev < 64) opted_in[dev] = true;
+  }
+  const int64_t tiles = static_cast<int64_t>((n + kBN - 1) / kBN) * ((m + kBM - 1) / kBM);
+  const int sms = num_sms();
+  const unsigned grid = static_cast<unsigned>(tiles < sms ? tiles : sms);
+  qchain_kernel<KIND, CHUNK, T><<<grid, kGemmThreads, kGemmSmem, st>>>(ma, mb, alpha, beta, static_cast<uint8_t*>(out), m, n,
+                                                                      k, make_idesc(KIND, a_signed), cv, t);
+  DLMCQ_LAUNCH_CHECK();
+  return DLMCQ_OK;
+}
+
+template <int CHUNK>
+int chain_dispatch(int encoding, int inter_bf16, const CUtensorMap& ma, const CUtensorMap& mb, const float* alpha,
+                   const float* beta, void* out, int m, int n, int k, const ConvArgs& cv, int a_signed,
+                   const CodeTail& t, cudaStream_t st) {
+  if (encoding == DLMCQ_QGEMM_I8)
+    return inter_bf16 ? chain_launch<DLMCQ_QGEMM_I8, CHUNK, __nv_bfloat16>(ma, mb, alpha, beta, out, m, n, k, cv, a_signed, t, st)
+                      : chain_launch<DLMCQ_QGEMM_I8, CHUNK, float>(ma, mb, alpha, beta, out, m, n, k, cv, a_signed, t, st);
+  return inter_bf16 ? chain_launch<DLMCQ_QGEMM_E4M3, CHUNK, __nv_bfloat16>(ma, mb, alpha, beta, out, m, n, k, cv, a_signed, t, st)
+                    : chain_launch<DLMCQ_QGEMM_E4M3, CHUNK, float>(ma, mb, alpha, beta, out, m, n, k, cv, a_signed, t, st);
+}
+
+// The tail's own refusals (dlmcq_qgemm_codes / dlmcq_qconv_codes), before any CUDA call.
+int tail_check(const dlmcq_bnq_tail* t) {
+  if (!t || !t->running_mean || !t->running_var || !t->qp) return DLMCQ_EINVAL;
+  if (!t->qp->scale || t->qp->form != DLMCQ_FORM_AFFINE) return DLMCQ_EINVAL;
+  if (t->inter_dtype != DLMCQ_F32 && t->inter_dtype != DLMCQ_BF16) return DLMCQ_EINVAL;
+  return code_range_ok(t->qp, t->encoding);                   // unknown encoding: DLMCQ_EINVAL
+}
+
+CodeTail make_tail(const dlmcq_bnq_tail* t) {
+  CodeTail c;
+  c.gamma = t->gamma;
+  c.beta = t->beta;
+  c.mean = t->running_mean;
+  c.var = t->running_var;
+  c.scale = t->qp->scale;
+  c.offset = t->qp->offset;
+  c.eps = t->eps;
+  c.g = t->qp->g;
+  c.lo = static_cast<float>(t->qp->lo);
+  c.hi = static_cast<float>(t->qp->hi);
+  c.relu = t->relu != 0;
+  c.enc = t->encoding;
+  return c;
+}
+
 // Geometry checks shared by dlmcq_qconv_prepare (full = 0: only the filter and channel counts) and dlmcq_qconv.
 int conv_check(const dlmcq_conv_geom* g, int full, int64_t* ho, int64_t* wo) {
   if (!g || g->cin < 1 || g->n < 1 || g->kh < 1 || g->kw < 1 || g->groups < 1) return DLMCQ_EINVAL;
@@ -857,6 +1081,16 @@ int conv_check(const dlmcq_conv_geom* g, int full, int64_t* ho, int64_t* wo) {
     return DLMCQ_EUNSUPPORTED;
   if (((m + kBM - 1) / kBM) * ((g->n + kBN - 1) / kBN) > 0x7fffffffLL) return DLMCQ_EUNSUPPORTED;
   return DLMCQ_OK;
+}
+
+ConvArgs conv_args(const dlmcq_conv_geom* geom, int64_t ho, int64_t wo, int chunk) {
+  ConvArgs cv;
+  cv.H = static_cast<int>(geom->h); cv.W = static_cast<int>(geom->w);
+  cv.Ho = static_cast<int>(ho); cv.Wo = static_cast<int>(wo); cv.HoWo = static_cast<int>(ho * wo);
+  cv.kh = geom->kh; cv.kw = geom->kw; cv.sh = geom->stride_h; cv.sw = geom->stride_w;
+  cv.ph = geom->pad_h; cv.pw = geom->pad_w; cv.dh = geom->dil_h; cv.dw = geom->dil_w;
+  cv.cchunks = static_cast<int>(geom->cin / chunk);
+  return cv;
 }
 
 }  // namespace
@@ -963,12 +1197,7 @@ extern "C" int dlmcq_qconv(const void* a_codes, const void* w_codes, const float
   const int64_t k = static_cast<int64_t>(geom->kh) * geom->kw * geom->cin;
   if (!make_im2col_map(&ma, a_codes, geom, chunk) || !make_map(&mb, w_codes, geom->n, k, kBN, chunk))
     return DLMCQ_EUNSUPPORTED;
-  ConvArgs cv;
-  cv.H = static_cast<int>(geom->h); cv.W = static_cast<int>(geom->w);
-  cv.Ho = static_cast<int>(ho); cv.Wo = static_cast<int>(wo); cv.HoWo = static_cast<int>(ho * wo);
-  cv.kh = geom->kh; cv.kw = geom->kw; cv.sh = geom->stride_h; cv.sw = geom->stride_w;
-  cv.ph = geom->pad_h; cv.pw = geom->pad_w; cv.dh = geom->dil_h; cv.dw = geom->dil_w;
-  cv.cchunks = static_cast<int>(geom->cin / chunk);
+  const ConvArgs cv = conv_args(geom, ho, wo, chunk);
   const int m = static_cast<int>(geom->batch * ho * wo), n = static_cast<int>(geom->n);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int bf = out_dtype == DLMCQ_BF16;
@@ -977,4 +1206,50 @@ extern "C" int dlmcq_qconv(const void* a_codes, const void* w_codes, const float
                         : conv_launch<DLMCQ_QGEMM_I8, 64>(ma, mb, alpha, beta, out, m, n, static_cast<int>(k), cv, a_signed, relu, bf, st);
   return chunk == 128 ? conv_launch<DLMCQ_QGEMM_E4M3, 128>(ma, mb, alpha, beta, out, m, n, static_cast<int>(k), cv, a_signed, relu, bf, st)
                       : conv_launch<DLMCQ_QGEMM_E4M3, 64>(ma, mb, alpha, beta, out, m, n, static_cast<int>(k), cv, a_signed, relu, bf, st);
+}
+
+extern "C" int dlmcq_qgemm_codes(const void* a_codes, const void* w_codes, const float* alpha, const float* beta,
+                                 void* codes_out, int64_t m, int64_t n, int64_t k, int encoding, int a_signed,
+                                 const dlmcq_bnq_tail* tail, void* stream) {
+  if (m < 0 || n < 1 || k < 1 || !alpha || !beta) return DLMCQ_EINVAL;
+  if (encoding != DLMCQ_QGEMM_I8 && encoding != DLMCQ_QGEMM_E4M3) return DLMCQ_EINVAL;
+  if (int e = tail_check(tail)) return e;
+  if (n % 16 != 0) return DLMCQ_EUNSUPPORTED;                  // whole 16-byte code stores per row piece
+  if (m == 0) return DLMCQ_OK;
+  if (!a_codes || !w_codes || !codes_out) return DLMCQ_EINVAL;
+  if (!aligned16(a_codes) || !aligned16(w_codes) || !aligned16(codes_out)) return DLMCQ_EALIGN;
+  if ((k & 15) != 0 || m > 0x7fffff00LL || n > 0x7fffff00LL || k > 0x7fffff00LL) return DLMCQ_EUNSUPPORTED;
+  if (((m + kBM - 1) / kBM) * ((n + kBN - 1) / kBN) > 0x7fffffffLL) return DLMCQ_EUNSUPPORTED;
+  CUtensorMap ma, mb;
+  if (!make_map(&ma, a_codes, m, k, kBM) || !make_map(&mb, w_codes, n, k, kBN)) return DLMCQ_EUNSUPPORTED;
+  return chain_dispatch<0>(encoding, tail->inter_dtype == DLMCQ_BF16, ma, mb, alpha, beta, codes_out,
+                           static_cast<int>(m), static_cast<int>(n), static_cast<int>(k), ConvArgs{}, a_signed,
+                           make_tail(tail), static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int dlmcq_qconv_codes(const void* a_codes, const void* w_codes, const float* alpha, const float* beta,
+                                 void* codes_out, const dlmcq_conv_geom* geom, int encoding, int a_signed,
+                                 const dlmcq_bnq_tail* tail, void* stream) {
+  if (!alpha || !beta) return DLMCQ_EINVAL;
+  if (encoding != DLMCQ_QGEMM_I8 && encoding != DLMCQ_QGEMM_E4M3) return DLMCQ_EINVAL;
+  if (int e = tail_check(tail)) return e;
+  int64_t ho = 0, wo = 0;
+  if (int e = conv_check(geom, 1, &ho, &wo)) return e;
+  if (geom->n % 16 != 0) return DLMCQ_EUNSUPPORTED;
+  if (!a_codes || !w_codes || !codes_out) return DLMCQ_EINVAL;
+  if (!aligned16(a_codes) || !aligned16(w_codes) || !aligned16(codes_out)) return DLMCQ_EALIGN;
+  const int chunk = geom->cin % 128 == 0 ? 128 : 64;
+  CUtensorMap ma, mb;
+  const int64_t k = static_cast<int64_t>(geom->kh) * geom->kw * geom->cin;
+  if (!make_im2col_map(&ma, a_codes, geom, chunk) || !make_map(&mb, w_codes, geom->n, k, kBN, chunk))
+    return DLMCQ_EUNSUPPORTED;
+  const ConvArgs cv = conv_args(geom, ho, wo, chunk);
+  const int m = static_cast<int>(geom->batch * ho * wo), n = static_cast<int>(geom->n);
+  const int bf = tail->inter_dtype == DLMCQ_BF16;
+  const CodeTail t = make_tail(tail);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  return chunk == 128 ? chain_dispatch<128>(encoding, bf, ma, mb, alpha, beta, codes_out, m, n, static_cast<int>(k), cv,
+                                            a_signed, t, st)
+                      : chain_dispatch<64>(encoding, bf, ma, mb, alpha, beta, codes_out, m, n, static_cast<int>(k), cv,
+                                           a_signed, t, st);
 }

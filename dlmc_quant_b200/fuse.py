@@ -54,17 +54,24 @@ def _rows_channels(x):
     return None
 
 
-def fusable(x, bn, identity=None):
-    """Can the fused kernels take this tensor / BatchNorm?  (Cheap host checks only.)"""
-    if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype in (torch.float32, torch.bfloat16)):
-        return False
-    rc = _rows_channels(x)
-    if rc is None or rc[0] == 0 or rc[1] % (4 if x.dtype is torch.float32 else 8) != 0:
-        return False
+def _rows_channels_ok(rc, dtype):
+    return rc is not None and rc[0] != 0 and rc[1] % (4 if dtype is torch.float32 else 8) == 0
+
+
+def _bn_ok(bn):
     if bn.momentum is None or (not bn.training and bn.running_mean is None):
         return False                                   # cumulative moving average / nothing to normalise with
     if (bn.weight is not None and bn.weight.dtype is not torch.float32) or \
             (bn.running_mean is not None and bn.running_mean.dtype is not torch.float32):
+        return False
+    return True
+
+
+def fusable(x, bn, identity=None):
+    """Can the fused kernels take this tensor / BatchNorm?  (Cheap host checks only.)"""
+    if not (isinstance(x, torch.Tensor) and x.is_cuda and x.dtype in (torch.float32, torch.bfloat16)):
+        return False
+    if not _rows_channels_ok(_rows_channels(x), x.dtype) or not _bn_ok(bn):
         return False
     if identity is not None and (identity.shape != x.shape or identity.dtype != x.dtype or
                                  identity.stride() != x.stride() or not identity.is_cuda):
@@ -215,6 +222,65 @@ def _bn_act_codes(x, bn, consumer, identity, relu, want_plain):
     return a, codes
 
 
+class _Output:
+    """numel() and device of a layer output that is never materialised (the chained site's BatchNorm input)."""
+
+    def __init__(self, shape, device):
+        self.shape, self.device = shape, device
+
+    def numel(self):
+        return math.prod(self.shape)
+
+
+def chain_spec(producer, in_shape, dtype, device, bn, consumer):
+    """(encoding, g) when the site producer -> bn -> (ReLU) -> consumer runs as ONE kernel in this call - the code GEMM
+    epilogue writes the consumer's input codes (qgemm.forward_codes with a tail) - else None.  It does exactly when the
+    two-kernel chain it replaces would run: the producer runs on codes (qgemm._code_state), its output is `fusable` for
+    the eval BatchNorm, and the consumer takes codes from a fused producer (_consumer_q, qgemm.code_input_spec); the
+    codes' row width (the consumer's K or Cin) must also be a multiple of 16.  The result is byte-identical to that
+    chain, so there is no switch: the site qualifies or it does not."""
+    if consumer is None or bn.training or bn.running_mean is None or not _bn_ok(bn):
+        return None
+    if bn.running_var.dtype is not torch.float32 or (bn.bias is not None and bn.bias.dtype is not torch.float32):
+        return None
+    if qgemm._code_state(producer, dtype, len(in_shape)) is None:
+        return None
+    out = qgemm.output_shape(producer, in_shape)
+    # the layouts `fusable` accepts for the output the code path writes: a Conv2d's [B, n, Ho, Wo] is channels-last
+    # ([B*Ho*Wo, n] rows), a Linear's output is a contiguous [..., n] and is a [rows, C] matrix only when it has two
+    # dimensions (a Linear on a 4-D input gives [B, C, H, n], which BatchNorm2d normalises along C: not fusable)
+    if len(out) == 4 and isinstance(producer, nn.Conv2d):
+        rc = (out[0] * out[2] * out[3], out[1])
+    elif len(out) == 2 and not isinstance(producer, nn.Conv2d):
+        rc = tuple(out)
+    else:
+        return None
+    if not _rows_channels_ok(rc, dtype) or rc[1] % 16 != 0 or bn.num_features != rc[1]:
+        return None
+    shape = _Output(out, device)
+    if _consumer_q(consumer, shape) is None:
+        return None
+    return qgemm.code_input_spec(consumer, shape.numel(), dtype, len(out))
+
+
+def _chain(producer, x, bn, relu, consumer, codes=None, dtype=None):
+    """The consumer's input codes when producer -> bn -> (ReLU) -> consumer runs chained in this call (chain_spec),
+    else None (nothing has run).  The producer's input is x, or - behind another chained site - its codes `codes`
+    (x then unused) with the dtype `dtype` of the layer outputs."""
+    src = x if codes is None else codes
+    dtype = x.dtype if codes is None else dtype
+    if consumer is None or not src.is_cuda:
+        return None
+    spec = chain_spec(producer, tuple(src.shape), dtype, src.device, bn, consumer)
+    if spec is None:
+        return None
+    if codes is None:
+        codes = qgemm.input_codes(producer, x)
+        if codes is None:
+            return None                                  # a fused producer handed the producer its fake-quantised input
+    return qgemm.forward_codes(producer, codes, dtype, tail=(bn, relu, consumer) + tuple(spec))
+
+
 def _feed(consumer, a, aq):
     """Run the consumer layer on the fused op's result."""
     if aq is not None:
@@ -256,10 +322,24 @@ def _is_bn(m):
 
 
 def _fused_sequential_run(mods, x):
-    """Run a list of modules with [BatchNorm, ReLU?, QBase?] runs fused."""
+    """Run a list of modules with [BatchNorm, ReLU?, QBase?] runs fused, and [QBase, BatchNorm, ReLU?, QBase] runs
+    chained where they qualify (chain_spec)."""
     i, n = 0, len(mods)
+    codes, dtype = None, x.dtype if isinstance(x, torch.Tensor) else None   # codes: mods[i]'s input from a chained site
     while i < n:
         m = mods[i]
+        if isinstance(m, QBase) and i + 1 < n and _is_bn(mods[i + 1]):
+            relu = i + 2 < n and isinstance(mods[i + 2], nn.ReLU)
+            j = i + (3 if relu else 2)
+            consumer = mods[j] if j < n and isinstance(mods[j], QBase) else None
+            nxt = _chain(m, x, mods[i + 1], relu, consumer, codes, dtype)
+            if nxt is not None:
+                codes, i = nxt, j
+                continue
+        if codes is not None:
+            x, codes = qgemm.forward_codes(m, codes, dtype), None
+            i += 1
+            continue
         if _is_bn(m):
             relu = i + 1 < n and isinstance(mods[i + 1], nn.ReLU)
             j = i + (2 if relu else 1)
@@ -281,18 +361,30 @@ def _sequential_forward(self, x):
 
 
 def _tv_bottleneck_forward(self, x):
-    """torchvision.models.resnet.Bottleneck.forward with the BatchNorm / ReLU / next-layer quantizer chains fused."""
-    out = self.conv1(x)
-    out = bn_act_into(out, self.bn1, self.conv2)
-    out = bn_act_into(out, self.bn2, self.conv3)
+    """torchvision.models.resnet.Bottleneck.forward with the BatchNorm / ReLU / next-layer quantizer chains fused, and
+    conv1 -> bn1 -> relu -> conv2 (then conv2 -> bn2 -> relu -> conv3) chained where they qualify."""
+    c2 = _chain(self.conv1, x, self.bn1, True, self.conv2)
+    if c2 is None:
+        out = self.conv1(x)
+        out = bn_act_into(out, self.bn1, self.conv2)
+        out = bn_act_into(out, self.bn2, self.conv3)
+    else:
+        c3 = _chain(self.conv2, None, self.bn2, True, self.conv3, c2, x.dtype)
+        if c3 is None:
+            out = bn_act_into(qgemm.forward_codes(self.conv2, c2, x.dtype), self.bn2, self.conv3)
+        else:
+            out = qgemm.forward_codes(self.conv3, c3, x.dtype)
     identity = x if self.downsample is None else self.downsample(x)
     return bn_add_act(out, self.bn3, identity, self._dlmcq_next)
 
 
 def _tv_basic_forward(self, x):
-    """torchvision.models.resnet.BasicBlock.forward, fused."""
-    out = self.conv1(x)
-    out = bn_act_into(out, self.bn1, self.conv2)
+    """torchvision.models.resnet.BasicBlock.forward, fused; conv1 -> bn1 -> relu -> conv2 chained where it qualifies."""
+    c2 = _chain(self.conv1, x, self.bn1, True, self.conv2)
+    if c2 is None:
+        out = bn_act_into(self.conv1(x), self.bn1, self.conv2)
+    else:
+        out = qgemm.forward_codes(self.conv2, c2, x.dtype)
     identity = x if self.downsample is None else self.downsample(x)
     return bn_add_act(out, self.bn2, identity, self._dlmcq_next)
 

@@ -25,10 +25,10 @@ from torch import nn
 
 from . import _lib
 from . import functional as F
-from ._lib import BF16, F32, FORM_AFFINE, FORM_SYM, FORM_ZP, QGEMM_E4M3, QGEMM_I8, ConvGeom, DlmcqError, QParams
+from ._lib import BF16, F32, FORM_AFFINE, FORM_SYM, FORM_ZP, QGEMM_E4M3, QGEMM_I8, BnqTail, ConvGeom, DlmcqError, QParams
 
-__all__ = ["codes_forward", "qgemm_prepare", "qgemm", "qconv_prepare", "qconv", "enable_code_gemm", "disable_code_gemm",
-           "QGEMM_I8", "QGEMM_E4M3"]
+__all__ = ["codes_forward", "qgemm_prepare", "qgemm", "qconv_prepare", "qconv", "bnq_tail", "qgemm_codes", "qconv_codes",
+           "enable_code_gemm", "disable_code_gemm", "QGEMM_I8", "QGEMM_E4M3"]
 
 
 def _qp(form, lo, hi, g, scale, offset):
@@ -183,6 +183,103 @@ def qgemm(a_codes, w_codes, alpha, beta, relu=False, out_dtype=torch.float32, a_
     return out
 
 
+def bnq_tail(running_mean, running_var, scale, offset, lo, hi, g, gamma=None, beta=None, eps=1e-5, relu=True,
+             inter_dtype=torch.float32, encoding=QGEMM_I8):
+    """What `qgemm_codes` / `qconv_codes` apply to the layer output in the epilogue (include/dlmcq.h, dlmcq_bnq_tail):
+    eval BatchNorm with the running buffers (gamma / beta None: 1 / 0), optional ReLU, then the consumer's per-tensor
+    AFFINE input quantizer (scale, offset: one fp32 element each; code range [lo, hi]; grad_scale factor g), whose codes
+    are written in `encoding`.  inter_dtype: the dtype the unchained layer output has (float32 or bfloat16)."""
+    if inter_dtype not in (torch.float32, torch.bfloat16):
+        raise DlmcqError("inter_dtype must be float32 or bfloat16")
+    F._require_cuda(running_mean, "running_mean")
+    dev, ch = running_mean.device, running_mean.numel()
+    bn = (running_mean, running_var, gamma, beta)
+    for name, v in zip(("running_mean", "running_var", "gamma", "beta"), bn):
+        if v is None and name.startswith("running"):
+            raise DlmcqError(f"{name} is required")
+        if v is not None and not (isinstance(v, torch.Tensor) and v.dtype is torch.float32 and v.device == dev and
+                                  v.numel() == ch and v.is_contiguous()):
+            raise DlmcqError(f"{name} must be a contiguous float32 tensor of {ch} elements on {dev}")
+    scale = F._qvec(scale, 1, dev, "scale")
+    offset = F._qvec(offset, 1, dev, "offset")
+    qp = _qp(FORM_AFFINE, lo, hi, g, scale, offset)
+    t = BnqTail(F._ptr(gamma), F._ptr(beta), F._ptr(running_mean), F._ptr(running_var), float(eps), int(bool(relu)),
+                F32 if inter_dtype == torch.float32 else BF16, C.pointer(qp), int(encoding))
+    # the descriptor holds raw pointers: keep the tensors alive with it
+    t._keep = [v.detach() for v in (*bn, scale, offset) if v is not None]
+    t._channels, t._device = ch, dev
+    return t
+
+
+def _check_tail(tail, n, device):
+    """The tail's BatchNorm covers the n output channels, on the operands' device (`bnq_tail` checked the rest)."""
+    if not isinstance(tail, BnqTail) or getattr(tail, '_channels', None) is None:
+        raise DlmcqError("tail must come from bnq_tail")
+    if tail._channels != n or tail._device != device:
+        raise DlmcqError(f"the tail's BatchNorm has {tail._channels} channels on {tail._device}; the layer has {n} "
+                         f"output channels on {device}")
+
+
+def qgemm_codes(a_codes, w_codes, alpha, beta, tail, a_signed=False, encoding=QGEMM_I8, out=None):
+    """`qgemm` followed by the BatchNorm / ReLU / quantizer `tail` (`bnq_tail`) in the same kernel: the consumer's codes
+    [m, n] (uint8), byte-identical to `qgemm` with out_dtype = the tail's inter_dtype and then the fused BatchNorm
+    producer's codes of that output (include/dlmcq.h, dlmcq_qgemm_codes).  n must be a multiple of 16."""
+    F._require_cuda(a_codes, "a_codes")
+    if a_codes.dtype != torch.uint8 or w_codes.dtype != torch.uint8 or a_codes.dim() != 2 or w_codes.dim() != 2:
+        raise DlmcqError("a_codes [m, k] and w_codes [n, k] must be uint8 matrices")
+    if not (a_codes.is_contiguous() and w_codes.is_contiguous()):
+        raise DlmcqError("code matrices must be contiguous (row-major, K innermost)")
+    m, k = a_codes.shape
+    n, k2 = w_codes.shape
+    if k != k2 or alpha.numel() != n or beta.numel() != n:
+        raise DlmcqError("shape mismatch between a_codes, w_codes, alpha, beta")
+    if out is None:
+        out = torch.empty(m, n, dtype=torch.uint8, device=a_codes.device)
+    elif out.shape != (m, n) or out.dtype != torch.uint8 or not out.is_contiguous() or out.device != a_codes.device:
+        raise DlmcqError("out must be a contiguous [m, n] uint8 tensor on the operands' device")
+    _check_tail(tail, n, a_codes.device)
+    with F._on(a_codes.device):
+        _lib.check(_lib.lib().dlmcq_qgemm_codes(F._ptr(a_codes), F._ptr(w_codes), F._ptr(alpha), F._ptr(beta),
+                                                F._ptr(out), m, n, k, int(encoding), int(bool(a_signed)), C.byref(tail),
+                                                F._stream_ptr()))
+    return out
+
+
+def qconv_codes(a_codes, w_codes, alpha, beta, tail, stride=1, padding=0, dilation=1, a_signed=False,
+                encoding=QGEMM_I8, out=None):
+    """`qconv` followed by the BatchNorm / ReLU / quantizer `tail` (`bnq_tail`) in the same kernel: the consumer's codes
+    [B, Ho, Wo, n] (uint8, channels-last), byte-identical to `qconv` with out_dtype = the tail's inter_dtype and then the
+    fused BatchNorm producer's codes of that output (include/dlmcq.h, dlmcq_qconv_codes).  n must be a multiple of 16."""
+    F._require_cuda(a_codes, "a_codes")
+    F._require_cuda(w_codes, "w_codes")
+    if a_codes.dtype != torch.uint8 or w_codes.dtype != torch.uint8 or a_codes.dim() != 4 or w_codes.dim() != 4:
+        raise DlmcqError("a_codes [B, H, W, cin] and w_codes [n, kh, kw, cin] must be uint8 tensors")
+    if not (a_codes.is_contiguous() and w_codes.is_contiguous()):
+        raise DlmcqError("code tensors must be contiguous (channels innermost)")
+    bsz, h, w, cin = a_codes.shape
+    n, kh, kw, cin2 = w_codes.shape
+    if cin != cin2 or alpha.numel() != n or tuple(beta.shape) != ((kh + 1) ** 2 * (kw + 1) ** 2, n):
+        raise DlmcqError("shape mismatch between a_codes, w_codes, alpha, beta")
+    g = _geom(bsz, h, w, cin, n, kh, kw, stride, padding, dilation)
+    ho = conv_out_size(h, kh, g.stride_h, g.pad_h, g.dil_h)
+    wo = conv_out_size(w, kw, g.stride_w, g.pad_w, g.dil_w)
+    if ho < 1 or wo < 1:
+        raise DlmcqError("the convolution has no output pixel")
+    shape = (bsz, ho, wo, n)
+    if out is None:
+        out = torch.empty(shape, dtype=torch.uint8, device=a_codes.device)
+    elif tuple(out.shape) != shape or out.dtype != torch.uint8 or not out.is_contiguous() or out.device != a_codes.device:
+        raise DlmcqError("out must be a contiguous [B, Ho, Wo, n] uint8 tensor on the operands' device")
+    _check_tail(tail, n, a_codes.device)
+    if bsz == 0:
+        return out
+    with F._on(a_codes.device):
+        _lib.check(_lib.lib().dlmcq_qconv_codes(F._ptr(a_codes), F._ptr(w_codes), F._ptr(alpha), F._ptr(beta),
+                                                F._ptr(out), C.byref(g), int(encoding), int(bool(a_signed)),
+                                                C.byref(tail), F._stream_ptr()))
+    return out
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # module level
 # ---------------------------------------------------------------------------------------------------------------
@@ -325,49 +422,94 @@ def code_input_spec(consumer, numel, dtype, dim):
     return st.encoding, 1 / math.sqrt(numel * consumer.in_max_val)
 
 
-def forward_codes(mod, a_codes, out_dtype):
+def output_shape(mod, in_shape):
+    """Shape of a switched layer's output (and of its codes from `forward_codes` with a tail) for an input of
+    `in_shape`."""
+    n = mod.weight.shape[0]
+    if not isinstance(mod, nn.Conv2d):
+        return tuple(in_shape[:-1]) + (n,)
+    b, _, h, w = in_shape
+    if not mod.__dict__['_code_gemm'].conv:
+        return (b, n, h, w)
+    (kh, kw), (sh, sw), (ph, pw), (dh, dw) = mod.kernel_size, mod.stride, mod.padding, mod.dilation
+    return (b, n, conv_out_size(h, kh, sh, ph, dh), conv_out_size(w, kw, sw, pw, dw))
+
+
+def forward_codes(mod, a_codes, out_dtype, tail=None):
     """The switched layer on its input's codes (uint8, the input's shape: [..., K] for Linear, an NCHW view of
     channels-last [B, H, W, Cin] storage for Conv2d), in the encoding of the layer's state.  Call only when
-    `code_input_spec` (or `_code_state`) accepted the layer for this input."""
+    `code_input_spec` (or `_code_state`) accepted the layer for this input.
+    tail = (bn, relu, consumer, encoding, g): return instead the consumer's input codes of relu(bn(output)) (uint8, the
+    output's shape and memory format) from the same kernel - eval `bn` with running statistics, the consumer's
+    per-tensor AFFINE input quantizer with grad_scale factor g, codes in `encoding` (`code_input_spec`), byte-identical
+    to the output in out_dtype followed by the fused BatchNorm producer's codes (fuse.py)."""
     st = mod.__dict__['_code_gemm']
     mod.__dict__.pop('_wq', None)                        # a weight group's pre-hook may have staged its copy: unused here
     alpha, beta = st.epilogue(mod, mod.__dict__['_code_gemm_forms'], a_codes.numel())
+    t = None
+    if tail is not None:
+        bn, relu, consumer, encoding, g = tail
+        t = bnq_tail(bn.running_mean, bn.running_var, consumer.in_scale.detach().reshape(-1),
+                     consumer.in_offset.detach().reshape(-1), consumer.in_min_val, consumer.in_max_val, g,
+                     bn.weight, bn.bias, bn.eps, relu, out_dtype, encoding)
+    a_signed = mod.in_min_val < 0
     if st.conv:
-        out = qconv(a_codes.permute(0, 2, 3, 1), st.w_codes, alpha, beta, mod.stride, mod.padding, mod.dilation,
-                    out_dtype=out_dtype, a_signed=mod.in_min_val < 0, encoding=st.encoding)
+        a = a_codes.permute(0, 2, 3, 1)
+        if t is not None:
+            out = qconv_codes(a, st.w_codes, alpha, beta, t, mod.stride, mod.padding, mod.dilation, a_signed=a_signed,
+                              encoding=st.encoding)
+        else:
+            out = qconv(a, st.w_codes, alpha, beta, mod.stride, mod.padding, mod.dilation, out_dtype=out_dtype,
+                        a_signed=a_signed, encoding=st.encoding)
         return out.permute(0, 3, 1, 2)                           # NCHW view of channels-last storage
     n = mod.weight.shape[0]
     if isinstance(mod, nn.Conv2d):
         b, k, h, w = a_codes.shape
         # elementwise codes keep x's memory order: channels-last NCHW storage is the [B*H*W, C] matrix
-        out = qgemm(a_codes.permute(0, 2, 3, 1).reshape(b * h * w, k), st.w_codes, alpha, beta, out_dtype=out_dtype,
-                    a_signed=mod.in_min_val < 0, encoding=st.encoding)
+        a = a_codes.permute(0, 2, 3, 1).reshape(b * h * w, k)
+        if t is not None:
+            out = qgemm_codes(a, st.w_codes, alpha, beta, t, a_signed=a_signed, encoding=st.encoding)
+        else:
+            out = qgemm(a, st.w_codes, alpha, beta, out_dtype=out_dtype, a_signed=a_signed, encoding=st.encoding)
         return out.view(b, h, w, n).permute(0, 3, 1, 2)          # NCHW view of channels-last storage
     k = a_codes.shape[-1]
-    out = qgemm(a_codes.reshape(-1, k), st.w_codes, alpha, beta, out_dtype=out_dtype, a_signed=mod.in_min_val < 0,
-                encoding=st.encoding)
+    a = a_codes.reshape(-1, k)
+    if t is not None:
+        out = qgemm_codes(a, st.w_codes, alpha, beta, t, a_signed=a_signed, encoding=st.encoding)
+    else:
+        out = qgemm(a, st.w_codes, alpha, beta, out_dtype=out_dtype, a_signed=a_signed, encoding=st.encoding)
     return out.view(*a_codes.shape[:-1], n)
+
+
+def input_codes(mod, input):
+    """A switched layer's input codes for this call (`_code_state` accepted it): the codes a fused producer handed over
+    (`_dlmcq_codes`), else its own x -> codes pass; None when a fused producer handed over the fake-quantised tensor
+    instead (`_dlmcq_q`: the layer then runs its original forward on it)."""
+    pre = getattr(input, '_dlmcq_codes', None)           # (consumer, codes) from a fused producer (fuse.py)
+    if pre is not None and pre[0] is mod:
+        return pre[1]
+    pre = getattr(input, '_dlmcq_q', None)
+    if pre is not None and pre[0] is mod:
+        return None
+    st = mod.__dict__['_code_gemm']
+    a_form, _ = mod.__dict__['_code_gemm_forms']
+    if isinstance(mod, nn.Conv2d):
+        x = input if input.is_contiguous(memory_format=torch.channels_last) else \
+            input.contiguous(memory_format=torch.channels_last)
+    else:
+        x = input if input.is_contiguous() else input.contiguous()
+    st.epilogue(mod, mod.__dict__['_code_gemm_forms'], x.numel())
+    return codes_forward(x, mod.in_scale.detach().reshape(-1), mod.in_offset, mod.in_min_val, mod.in_max_val, a_form,
+                         st._g_a, encoding=st.encoding)
 
 
 def _code_forward(self, input):
     st = _code_state(self, input.dtype, input.dim()) if input.is_cuda else None
     if st is None:
         return self._code_gemm_orig_forward(input)
-    pre = getattr(input, '_dlmcq_codes', None)           # (consumer, codes) from a fused producer (fuse.py)
-    if pre is not None and pre[0] is self:
-        return forward_codes(self, pre[1], input.dtype)
-    pre = getattr(input, '_dlmcq_q', None)
-    if pre is not None and pre[0] is self:
+    a_codes = input_codes(self, input)
+    if a_codes is None:
         return self._code_gemm_orig_forward(input)      # a fused producer already handed over the fake-quantised tensor
-    a_form, _ = self.__dict__['_code_gemm_forms']
-    if isinstance(self, nn.Conv2d):
-        x = input if input.is_contiguous(memory_format=torch.channels_last) else \
-            input.contiguous(memory_format=torch.channels_last)
-    else:
-        x = input if input.is_contiguous() else input.contiguous()
-    st.epilogue(self, self.__dict__['_code_gemm_forms'], x.numel())
-    a_codes = codes_forward(x, self.in_scale.detach().reshape(-1), self.in_offset, self.in_min_val, self.in_max_val,
-                            a_form, st._g_a, encoding=st.encoding)
     return forward_codes(self, a_codes, input.dtype)
 
 

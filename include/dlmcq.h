@@ -582,6 +582,43 @@ int dlmcq_qconv_prepare(const void* w_codes, const dlmcq_conv_geom* geom, int en
 int dlmcq_qconv(const void* a_codes, const void* w_codes, const float* alpha, const float* beta, void* out,
                 const dlmcq_conv_geom* geom, int encoding, int a_signed, int relu, int out_dtype, void* stream);
 
+/* ---- layer in codes, layer out codes: the code GEMM / convolution followed by eval BatchNorm (+ ReLU) and the next
+ * layer's input quantizer, in one kernel (inference) ------------------------------------------------------------
+ * dlmcq_qgemm_codes / dlmcq_qconv_codes take the operands of dlmcq_qgemm / dlmcq_qconv and, instead of the layer
+ * output, write the CONSUMER layer's input codes: codes_out [m, n] bytes (channels-last rows; m = batch*Ho*Wo for the
+ * convolution).  The fp32 / bf16 layer output never reaches memory.  The result is byte-identical to the two calls it
+ * replaces:
+ *     y     = dlmcq_qgemm / dlmcq_qconv (same operands, alpha, beta, encoding, a_signed; relu = 0;
+ *                                        out_dtype = tail->inter_dtype)
+ *     codes = dlmcq_bnq_forward_codes(y, identity = NULL, gamma, beta, running_mean, running_var, eval,
+ *                                     DLMCQ_BNQ_RELU if tail->relu, tail->qp, tail->encoding)
+ * i.e. per element: v = RN(RN(acc * alpha[n]) + beta[(class)][n]) rounded to inter_dtype; z = fma(v - mean[n],
+ * RN(gamma[n] * invstd[n]), bn_beta[n]) with invstd = RN(1 / RN(sqrt(running_var[n] + eps))); ReLU (NaN propagates);
+ * rounded to inter_dtype; the AFFINE quantizer of qp (grad_scale value with qp->g); the code byte in tail->encoding,
+ * NaN -> 0.  BatchNorm is not folded into alpha / beta (that would change the roundings).
+ * dlmcq_bnq_tail: gamma / beta may be NULL (1 / 0, as dlmcq_bnq_forward); running_mean / running_var [n] fp32 are
+ * required; qp is the consumer's per-tensor FORM_AFFINE input quantizer (scale, offset: one float each).
+ * Refused before any CUDA call, besides everything dlmcq_qgemm / dlmcq_qconv refuse: tail NULL, running buffers NULL,
+ * qp NULL / not FORM_AFFINE / no scale, an unknown encoding or inter_dtype (DLMCQ_EINVAL); a code range
+ * tail->encoding cannot hold, n % 16 != 0 (DLMCQ_EUNSUPPORTED); codes_out not 16-byte aligned (DLMCQ_EALIGN). */
+typedef struct {
+  const float* gamma;
+  const float* beta;
+  const float* running_mean;
+  const float* running_var;
+  float eps;
+  int32_t relu;
+  int32_t inter_dtype;      /* dlmcq_dtype of the layer output the unchained model writes */
+  const dlmcq_qparams* qp;  /* consumer's per-tensor AFFINE input quantizer */
+  int32_t encoding;         /* DLMCQ_QGEMM_*: the consumer's operand encoding of codes_out */
+} dlmcq_bnq_tail;
+int dlmcq_qgemm_codes(const void* a_codes, const void* w_codes, const float* alpha, const float* beta, void* codes_out,
+                      int64_t m, int64_t n, int64_t k, int encoding, int a_signed, const dlmcq_bnq_tail* tail,
+                      void* stream);
+int dlmcq_qconv_codes(const void* a_codes, const void* w_codes, const float* alpha, const float* beta, void* codes_out,
+                      const dlmcq_conv_geom* geom, int encoding, int a_signed, const dlmcq_bnq_tail* tail,
+                      void* stream);
+
 #ifdef __cplusplus
 }
 #endif
