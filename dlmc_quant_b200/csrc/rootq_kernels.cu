@@ -5,7 +5,7 @@
 // saved N-sized tensors per layer); here forward is one pass (read w, write w_q) and backward
 // is one pass (read w, dy; write dw) that also block-reduces d(upper), d(lower), d(alpha)
 // (weights) or d(in_scale) (activations).  Closed forms: SURVEY.md A.5, re-derived and checked
-// against autograd in fp64 (tests/test_closed_forms.py).
+// against autograd in fp64 (tests/test_closed_forms.py, float64 terms in tests/rootq_terms.py).
 //
 // The scalar prologue (EMA of the running bounds, gradient mix, delta, clamped alpha) is a
 // one-thread "prepare" kernel writing a small state block: no host sync, and the in-place
@@ -85,7 +85,8 @@ __device__ __forceinline__ float rq_act_bwd(float x, float dy, float rs, float u
   const float I = round_pass(v);
   const bool clipped_hi = ov > 0.f;
   acc += dy * ((I - v) + (clipped_hi ? q : 0.f));
-  return ((nl > 0.f) || clipped_hi) ? 0.f : dy;
+  // relu's gradient passes wherever its input is not <= 0, NaN included: a NaN x gets dx = 0 like x -> +-inf
+  return ((nl <= 0.f) && (ov <= 0.f)) ? dy : 0.f;
 }
 
 // Fast path of the activation chain on vectors (same results; see fq_math.cuh for the argument):
@@ -133,7 +134,7 @@ __device__ __forceinline__ void rq_act_bwd_vec(const float (&x)[N], const float 
         const float I = rintf(v) + 0.f;
         const bool hi_clip = ov[e] > 0.f;
         acc = __fmaf_rn(dy[e], (I - v) + (hi_clip ? q : 0.f), acc);
-        dx[e] = ((nl[e] > 0.f) || hi_clip) ? 0.f : dy[e];
+        dx[e] = ((nl[e] <= 0.f) && (ov[e] <= 0.f)) ? dy[e] : 0.f;
       }
       return;
     }
@@ -159,8 +160,15 @@ __device__ __forceinline__ RqW load_rqw(const float* st) {
   p.fd = make_fastdiv(p.delta);
   return p;
 }
-// weight forward value: base.py:146-155.  sign(pow(b, alpha)*sg) == sign(z) because b >= 1e-5 > 0,
-// so the forward needs no pow; torch.sgn(NaN) is 0.
+// The level sign of function.py:31,58, sgn(pow(b, alpha) * sg) with b = k*|z| + 1e-5, as the reference evaluates it.
+// With delta > 0 (k > 0), b >= 1e-5 > 0 and the sign is sign(z), which the callers use without a pow.  With U < L
+// (delta < 0) b can be negative: pow gives NaN (sgn 0) for a fractional alpha and b itself for alpha == 1.
+__device__ __forceinline__ float rq_sgn(float v) { return (v > 0.f) ? 1.f : ((v < 0.f) ? -1.f : 0.f); }
+__device__ __forceinline__ float rq_level_sign_literal(float z, const RqW& p) {
+  const float az = fabsf(z);
+  return rq_sgn(powf(p.k * az + 1e-5f, p.alpha) * (z / (az + 1e-5f)));
+}
+// weight forward value: base.py:146-155; torch.sgn(NaN) is 0.
 __device__ __forceinline__ float rq_wt_fwd(float w, const RqW& p) {
   const float x1 = w + relu_ref(p.L - w);
   const float c = x1 - relu_ref(x1 - p.U);
@@ -169,7 +177,7 @@ __device__ __forceinline__ float rq_wt_fwd(float w, const RqW& p) {
   const float I = (fl - t) + t;                      // floor_pass value, utils.py:34-37
   const float mi = (I + 0.5f) * p.delta + p.L;       // base.py:149
   const float z = c - mi;
-  const float sig = (z > 0.f) ? 1.f : ((z < 0.f) ? -1.f : 0.f);
+  const float sig = (p.k > 0.f) ? rq_sgn(z) : rq_level_sign_literal(z, p);
   return ((sig + 1.f) / 2.f + I) * p.delta + p.L;    // function.py:63-67
 }
 // weight backward: returns dw, accumulates the three reduced gradients (un-chained).
@@ -192,13 +200,15 @@ __device__ __forceinline__ float rq_wt_bwd(float w, float dy, const RqW& p, floa
   const float sg = z / den;
   const float b = p.k * az + 1e-5f;
   const float lb = logf(b);
-  const float pw = expf(p.alpha * lb);               // b^alpha
-  const float sgnz = (z > 0.f) ? 1.f : ((z < 0.f) ? -1.f : 0.f);
+  const bool kpos = p.k > 0.f;
+  const float pw = kpos ? expf(p.alpha * lb) : powf(b, p.alpha);   // b^alpha (b may be negative when U < L)
+  const float sgnz = rq_sgn(z);
+  const float sig = kpos ? sgnz : rq_sgn(pw * sg);   // level sign, as in rq_wt_fwd
   const float pw_b = pw / b;                         // b^(alpha-1)
   const float dpdz = p.alpha * pw_b * p.k * sgnz * sg + pw * 1e-5f / (den * den);
   const float dpdd = -(p.alpha * pw_b * p.k * az * sg) / p.delta;
   const float dpda = pw * lb * sg;
-  const float lvl = (sgnz + 1.f) * 0.5f + I;
+  const float lvl = (sig + 1.f) * 0.5f + I;
   const float inv_q = 1.f / p.q;
   accA += dy * (p.half_delta * dpda);
   accU += dy * (p.half_delta * (dpdz * cu + dpdd * inv_q) + (cu - t * inv_q) + lvl * inv_q);

@@ -115,7 +115,7 @@ void orc_rootq_act(const float* x, const float* dy, float* y, float* dx, double*
     if (dy) {
       int hi_clip = ov > 0.f;
       acc += (double)dy[i] * (((double)I - (double)v) + (hi_clip ? (double)q : 0.0));
-      dx[i] = ((nl > 0.f) || hi_clip) ? 0.f : dy[i];
+      dx[i] = ((nl <= 0.f) && (ov <= 0.f)) ? dy[i] : 0.f;   /* relu' passes NaN: dx(NaN) = 0 */
     }
   }
   if (d_rs) *d_rs = acc;                  /* caller multiplies by m*g (base.py:95,97) */
@@ -144,8 +144,13 @@ void orc_rootq_wt(const float* w, const float* dy, float* y, float* dw, double* 
     float I = floor_pass(t);              /* base.py:148 */
     float mi = (I + 0.5f) * delta + L;    /* base.py:149 */
     float z = c - mi;
-    float sig = (z > 0.f) ? 1.f : ((z < 0.f) ? -1.f : 0.f);   /* sign(pow(b,a)*sg) == sign(z) */
-    y[i] = ((sig + 1.f) / 2.f + I) * delta + L;                /* function.py:63-67 */
+    float sig = (z > 0.f) ? 1.f : ((z < 0.f) ? -1.f : 0.f);
+    float lsig = sig;                     /* level sign sgn(pow(b,a)*sg): sign(z) when delta > 0 (b >= 1e-5) */
+    if (!(k > 0.f)) {                     /* U < L: b may be negative, pow NaN (sgn 0) or b itself (a == 1) */
+      float p = powf(k * fabsf(z) + 1e-5f, a2) * (z / (fabsf(z) + 1e-5f));
+      lsig = (p > 0.f) ? 1.f : ((p < 0.f) ? -1.f : 0.f);
+    }
+    y[i] = ((lsig + 1.f) / 2.f + I) * delta + L;               /* function.py:63-67 */
     if (dy) {
       int m_lo = lw > 0.f, m_hi = ov > 0.f;
       double dcw = (m_lo || m_hi) ? 0.0 : 1.0, cu = m_hi ? 1.0 : 0.0, cl = (m_lo && !m_hi) ? 1.0 : 0.0;
@@ -154,7 +159,7 @@ void orc_rootq_wt(const float* w, const float* dy, float* y, float* dw, double* 
       double dpdz = (double)a2 * pw / b * (double)k * (double)sig * sg + pw * 1e-5 / (den * den);
       double dpdd = -((double)a2 * pw / b * (double)k * az * sg) / (double)delta;
       double dpda = pw * lb * sg;
-      double lvl = ((double)sig + 1.0) * 0.5 + (double)I, hd = (double)delta * 0.5, iq = 1.0 / (double)q;
+      double lvl = ((double)lsig + 1.0) * 0.5 + (double)I, hd = (double)delta * 0.5, iq = 1.0 / (double)q;
       gA += (double)dy[i] * hd * dpda;
       gU += (double)dy[i] * (hd * (dpdz * cu + dpdd * iq) + (cu - (double)t * iq) + lvl * iq);
       gL += (double)dy[i] * (hd * (dpdz * cl - dpdd * iq) + (cl - 1.0 + (double)t * iq) - lvl * iq + 1.0);
