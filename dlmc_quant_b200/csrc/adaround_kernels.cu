@@ -63,7 +63,10 @@ adaround_bwd_kernel(const T* __restrict__ w, const T* __restrict__ alpha, const 
     const bool in_q = (q >= lo) && (q <= hi);                   // clamp backward, inclusive
     const bool in_h = (pre >= 0.f) && (pre <= 1.f);
     const float sg = sigmoid_ref(a);
-    const float d = (in_q && in_h) ? ((g * s) * kZetaMinusGamma) * ((1.f - sg) * sg) : 0.f;
+    // the masks zero the incoming gradient, not the result: sigmoid's backward still multiplies it by
+    // (1 - sg) * sg, so a NaN alpha gives a NaN d alpha, as autograd of the reference chain does
+    const float gm = (in_q && in_h) ? (g * s) * kZetaMinusGamma : 0.f;
+    const float d = gm * ((1.f - sg) * sg);
     dalpha[beg + j] = from_f32<T>(d);
   }
   acc = warp_sum(acc);
